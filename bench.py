@@ -16,6 +16,8 @@ A step is one pass of the hot path over the workload: assemble every affine part
     cpu_baseline   the CPU oracle (a port: the reference cannot be built here) on a bounded sample, rank 0, N = 1 only
 
 `--impl reference` times the CPU restatement of the reference path (oracle/, serial walk like the reference) instead.
+`--dump-outputs DIR` writes what the last timed step computed (solution, system matrix, rhs; see dump_outputs) as .npy
+files: the inputs are the same for the same arguments, so two builds can be compared output for output.
 N > 1: one rank per GPU (torchrun); the 8 x 8 subdomains of BlockSWIPDG are dealt to the ranks in contiguous slabs,
 NCCL carries the coupling-face halo of the CG direction and the dot-product all-reduces (strong scaling of one grid).
 """
@@ -279,6 +281,44 @@ def gather_concat(local, world, torch):
     return np.concatenate([p[:k].cpu().numpy() for p, k in zip(parts, sizes)])
 
 
+DUMP_SAMPLE = 1 << 21  # entries per dumped array: three arrays of float64 stay under 64 MB
+
+
+class _DeviceArray:
+    """a float64 device buffer of the library, for torch to view without a copy"""
+
+    def __init__(self, ptr, n):
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": "<f8", "data": (ptr, False), "version": 3,
+                                         "strides": None}
+
+
+def dump_outputs(dirname, d, torch, capi, rank, world):
+    """What the last timed step leaves its caller - the solution of the solve, the CSR values (over pattern()) of the
+    assembled system matrix and the assembled rhs - as <dirname>/{solution,system_matrix,rhs}.npy in float64.  A longer
+    array than DUMP_SAMPLE entries is sampled at the sorted global indices numpy.random.default_rng(0) draws without
+    replacement, so that runs with the same arguments write the same entries.  Collective on N > 1 ranks (rank order is
+    global order); rank 0 writes."""
+    import ctypes as C
+    x = C.c_void_p()
+    capi.check(capi.lib().hdd_solution_dev(d._h, C.byref(x)))
+    arrays = {"solution": (x.value, d.num_owned_dofs()), "system_matrix": d.system_matrix().device_pointer(-1),
+              "rhs": d.rhs().device_pointer(-1)}
+    if rank == 0:
+        os.makedirs(dirname, exist_ok=True)
+    for name, (ptr, n) in arrays.items():
+        counts = gather_concat(np.array([n], np.int64), world, torch)
+        total, offset = int(counts.sum()), int(counts[:rank].sum())
+        if total <= DUMP_SAMPLE:
+            idx = np.arange(total)
+        else:
+            idx = np.sort(np.random.default_rng(0).choice(total, DUMP_SAMPLE, replace=False))
+        mine = torch.from_numpy(idx[(idx >= offset) & (idx < offset + n)] - offset).cuda()
+        values = torch.as_tensor(_DeviceArray(ptr, n), device="cuda")[mine].cpu().numpy()
+        values = gather_concat(values, world, torch)
+        if rank == 0:
+            np.save(os.path.join(dirname, name + ".npy"), values.astype(np.float64))
+
+
 def small_grid_parity(hdd, torch, comm, rank, world, local_rank):
     """In-run parity of what this process group computes, against the CPU oracle (checker only, rank 0): a 256^2 Q1 grid
     (pattern bit-exact, entries and rhs 1e-12, cg.mg solution 1e-8) and 8192 triangles (block-Jacobi CG solution and every
@@ -458,8 +498,15 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the small-grid check against the CPU oracle")
     ap.add_argument("--solver", default="cg.mg", help="cg.mg | cg.blockdiagonal | cg.diagonal | cg.identity")
     ap.add_argument("--no-jacobi", action="store_true", help="skip the extra Jacobi-CG solve reported next to --solver")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed "
+                                                          "(solution, system matrix values, rhs; a fixed seeded sample of "
+                                                          "at most %d entries each) as DIR/<name>.npy" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the GPU path computed; the reference arm has no such outputs")
         if args.cpu_cg_iters <= 0:
             n_cpu = args.cpu_n if args.cpu_n > 0 else default_cpu_n(args.n)
             args.cpu_cg_iters = max(3, int(100 * (768.0 / n_cpu) ** 2))
@@ -527,6 +574,8 @@ def main():
     wall = time.perf_counter() - t0
     launches = capi.kernel_launches() - launches1
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, d, torch, capi, rank, world)
 
     t_asm = sum(r[0] for r in results)
     t_cg = sum(r[1]["seconds"] for r in results)

@@ -2,12 +2,12 @@
 """Transcribes the reference's committed test expectations (the golden vectors of this path) into
 tests/golden/reference_expectations.json.
 
-Run in the build container, where the reference tree is mounted read-only at /root/reference:
+Run against a checkout of the reference:
 
-    python tests/golden/extract_expectations.py [/root/reference]
+    python tests/golden/extract_expectations.py <dune-hdd checkout>
 
-The GPU box has no /root/reference; the tests only read the JSON.  Every vector keeps the file and line it came
-from.  Keys: "<file stem>" -> "<partitioning or '-'>" -> "<mu,mu_bar,mu_hat or '-'>" -> "<type>" -> {values, line}.
+The tests only read the JSON.  Every vector keeps the file and line it came from.  Keys: "<file stem>" ->
+"<partitioning or '-'>" -> "<mu,mu_bar,mu_hat or '-'>" -> "<type>" -> {values, line}.
 Only the four expectation files that are reproducible offline are transcribed (SURVEY.md 8c): the SPE10 ones need
 perm_case1.dat, which the reference does not ship.
 """
@@ -46,7 +46,9 @@ def parse(path):
 
 
 def main():
-    ref = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+    if len(sys.argv) != 2:
+        sys.exit("usage: %s <dune-hdd checkout>" % sys.argv[0])
+    ref = sys.argv[1]
     data = {"_source": "tobiasleibner/dune-hdd test/*.cxx, transcribed by tests/golden/extract_expectations.py"}
     for f in FILES:
         data[f[:-4]] = parse(os.path.join(ref, "test", f))

@@ -202,14 +202,6 @@ def test_golden_fixture_is_complete_and_cites_its_source():
     assert alu["eta_ESV2007"]["values"] == [4.49e-01, 2.07e-01, 9.91e-02, 4.85e-02] and alu["eta_ESV2007"]["line"] > 0
     blk = d["linearelliptic-block-swipdg-expectations_esv2007_2daluconform"]
     assert sorted(blk) == ["[1 1 1]", "[2 2 1]", "[4 4 1]", "[8 8 1]"]
-    # if the reference tree is mounted (build container), the fixture must equal a fresh transcription
-    if os.path.isdir("/root/reference/test"):
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("extract", os.path.join(os.path.dirname(path), "extract_expectations.py"))
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        for f in mod.FILES:
-            assert d[f[:-4]] == mod.parse(os.path.join("/root/reference/test", f)), f
 
 
 def test_father_search_finds_the_containing_coarse_cell():

@@ -1,5 +1,5 @@
-import sys, warnings
-sys.path.insert(0, '/root/repo')
+import os, sys, warnings
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, scipy.sparse as sp, scipy.sparse.linalg as spla
 from oracle import oracle as o
 from tests.test_mg_prototype import _hierarchy, _vcycle
