@@ -228,7 +228,7 @@ struct hdd_swipdg {
   bool p2p_ready = false, p2p_failed = false;
   hdd::PeerView peer_view{};
   std::vector<void*> ipc_opened;
-  int last_precond = 1;  // 0 identity, 1 diagonal, 2 cell-block diagonal, 3 two-level multigrid (cg.mg)
+  int last_precond = 1;  // 0 identity, 1 diagonal, 2 cell-block diagonal, 3 two-level multigrid (cg.mg), 4 cg.mg2
   hdd::MgState* mg = nullptr;
   // CUDA graph of two CG iterations, cached per solver type; valid while the operator / workspace pointers it was
   // captured with are the ones in use (cg_graph_key)
@@ -237,7 +237,7 @@ struct hdd_swipdg {
     const void* key[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     int64_t launches = 0;
   };
-  CgGraph cg_graph[4];
+  CgGraph cg_graph[5];
   hdd::DevBuf<hdd::CgScalars> sc;
   hdd::CgScalars* sc_host = nullptr;  // pinned
   bool have_solution = false;
@@ -263,10 +263,10 @@ void require_init(const hdd_swipdg* h);                                         
 void check_mu(const hdd_swipdg* h, const double* mu, int mu_size, const char* name);  // base.hh:333-334
 double eval_coef(const Program& p, const double* mu, int mu_size);
 void assemble_products(hdd_swipdg* h);
-// multigrid.cu ("cg.mg")
+// multigrid.cu ("cg.mg", "cg.mg2")
 void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_dev, int64_t v_begin, int64_t v_end,
                          const int32_t* cv_dev, int64_t n_verts);
-void mg_setup(hdd_swipdg* h, const double* frozen_values);
+void mg_setup(hdd_swipdg* h, const double* frozen_values, bool q2);
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc);
 void mg_release(MgState* st);
 int mg_num_levels(const hdd_swipdg* h);  // the product assemblers added to system_assembler (discretizations/swipdg.hh:359-479)

@@ -24,6 +24,14 @@
 // vertex levels are swept in row strips with one halo row exchanged per sweep (grouped ncclSend/ncclRecv with the rank
 // below / above), the level-2 right-hand side is summed over the ranks and levels >= 2 run replicated.  Otherwise the
 // whole V-cycle runs replicated on the all-reduced restricted residual.
+//
+// "cg.mg2": the same machinery for polOrder 2 on structured Q2 grids,
+//
+//   M^-1 r = D_9^-1 r  +  P V_P(P^T r)  +  H V_H(H^T r)
+//
+// with P the bilinear interpolation of the conforming Q1 space into Q2-DG and H the hourglass family of the Q2 volume
+// term (see k_vertex_galerkin_q2).  A_P and A_H are two independent 9-point vertex operators: the two hierarchies of
+// MgState (MgState::q2), each with a level-0 operator of its own.  On N GPUs the vertex levels always run replicated.
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -778,6 +786,174 @@ __global__ void __launch_bounds__(kMgThreads)
   grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
 }
 
+// ---- DG level for polOrder 2 on cubes ("cg.mg2"): two auxiliary vertex spaces with hierarchies of their own ----------
+// P: bilinear interpolation of the conforming Q1 vertex space at the 9 nodes (node a + 3 b of a cell gets
+//    q2_w(i, a) q2_w(j, b) of its vertex i + 2 j);
+// H: the hourglass family - cell c gets s[v0(c)] q2_g(a) q2_g(b) at node a + 3 b, v0(c) its lower-left vertex.  Under the
+//    2 x 2 Gauss rule of the Q2 volume term (x^2 - 1/3)(y^2 - 1/3) has a zero gradient at every quadrature point and is
+//    continuous across faces: with a smooth amplitude it is an energy-free family no Q1 space represents (DESIGN.md 6).
+// Hierarchy 0 holds A_P = P^T A P, hierarchy 1 A_H = H^T A H; both are 9-point vertex stencils.
+__device__ __forceinline__ double q2_w(int i, int a) { return i == 0 ? 1.0 - 0.5 * a : 0.5 * a; }
+__device__ __forceinline__ double q2_g(int a) { return a == 1 ? -1.0 / 3.0 : 2.0 / 3.0; }
+
+// Both level-0 stencils per vertex v, gathered from the 9 x 9 blocks of the <= 4 owned cells around v (rows of cells owned
+// elsewhere are added by the all-reduce).  A_P: the rows of the nodes v interpolates into, weighted towards the vertices of
+// the block's cell (entries at index distance 2 cancel analytically, as for Q1).  A_H: only the cell whose lower-left
+// vertex is v has hourglass rows at v; they couple to the face neighbours, whose lower-left vertices are lattice
+// neighbours of v.  S: hierarchy 0 in S[e nv + v], hierarchy 1 in S[(9 + e) nv + v].
+__global__ void __launch_bounds__(kMgThreads)
+    k_vertex_galerkin_q2(MeshView m, const double* __restrict__ vals, const int32_t* __restrict__ cell_v0,
+                         const int32_t* __restrict__ lex_cell, int nx, int ny, double* __restrict__ S) {
+  const int64_t nv = int64_t(nx + 1) * (ny + 1);
+  const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v >= nv) return;
+  const int nx1 = nx + 1;
+  const int ix = int(v % nx1), iy = int(v / nx1);
+  double ap[9], ah[9];
+#pragma unroll
+  for (int e = 0; e < 9; ++e) ap[e] = ah[e] = 0.0;
+#pragma unroll
+  for (int b = 0; b < 2; ++b)
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+      const int cx = ix - 1 + a, cy = iy - 1 + b;
+      if (cx < 0 || cy < 0 || cx >= nx || cy >= ny) continue;
+      const int c = __ldg(lex_cell + cx + nx * cy);
+      const int k = c - m.own0;
+      if (c < 0 || k < 0 || k >= m.n_own) continue;
+      const int vx = 1 - a, vy = 1 - b;   // v is vertex vx + 2 vy of cell c
+      const bool hg = a == 1 && b == 1;   // v is the lower-left vertex of c
+      int nb[4];
+      load_neigh4(m.neigh, k, nb);
+      const int nblk = block_count<4>(nb);
+      const double* blk = vals + __ldg(m.blk_start + k) * 81;
+#pragma unroll 1
+      for (int t = 0; t < 5; ++t) {
+        const int cell = t == 0 ? c : nb[t - 1];
+        if (cell < 0) continue;
+        const int slot = block_slot<4>(c, nb, cell);
+        const int v0 = __ldg(cell_v0 + cell);
+        const int jx = v0 % nx1 - ix, jy = v0 / nx1 - iy;
+        double sp[4] = {0.0, 0.0, 0.0, 0.0}, sh = 0.0;
+#pragma unroll
+        for (int n = 0; n < 9; ++n) {
+          const double wp = q2_w(vx, n % 3) * q2_w(vy, n / 3);
+          const double wh = hg ? q2_g(n % 3) * q2_g(n / 3) : 0.0;
+          if (wp == 0.0 && wh == 0.0) continue;
+          const double* row = blk + int64_t(n) * nblk * 9 + slot * 9;
+          double rp[4] = {0.0, 0.0, 0.0, 0.0}, rh = 0.0;
+#pragma unroll
+          for (int q = 0; q < 9; ++q) {
+            const double a_nq = __ldg(row + q);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const double w = q2_w(j & 1, q % 3) * q2_w(j >> 1, q / 3);
+              if (w != 0.0) rp[j] = fma(w, a_nq, rp[j]);
+            }
+            rh = fma(q2_g(q % 3) * q2_g(q / 3), a_nq, rh);
+          }
+#pragma unroll
+          for (int j = 0; j < 4; ++j) sp[j] = fma(wp, rp[j], sp[j]);
+          sh = fma(wh, rh, sh);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          const int dx = jx + (j & 1), dy = jy + (j >> 1);
+          if (dx < -1 || dx > 1 || dy < -1 || dy > 1) continue;
+          ap[(dy + 1) * 3 + dx + 1] += sp[j];
+        }
+        if (hg) ah[(jy + 1) * 3 + jx + 1] += sh;
+      }
+    }
+#pragma unroll
+  for (int e = 0; e < 9; ++e) {
+    S[e * nv + v] = ap[e];
+    S[(9 + e) * nv + v] = ah[e];
+  }
+}
+
+// No cell has its lower-left vertex in the top vertex row or the right vertex column: those rows of A_H are empty.  They
+// get the mean diagonal of the other rows, which keeps the Jacobi sweeps and the coarsest Cholesky defined (the rows stay
+// decoupled on level 0; H ignores their values).  One CTA, fixed summation order.
+__global__ void __launch_bounds__(1024) k_hourglass_fill(double* __restrict__ diag, int nx, int ny) {
+  __shared__ double smem[32];
+  const int nx1 = nx + 1;
+  const int64_t nv = int64_t(nx1) * (ny + 1);
+  double s[1] = {0.0};
+  for (int64_t v = threadIdx.x; v < nv; v += blockDim.x)
+    if (v % nx1 < nx && v / nx1 < ny) s[0] += diag[v];
+  block_sum<1>(s, smem);
+  __shared__ double mean;
+  if (threadIdx.x == 0) mean = s[0] / (double(nx) * ny);
+  __syncthreads();
+  for (int64_t v = threadIdx.x; v < nv; v += blockDim.x)
+    if (v % nx1 == nx || v / nx1 == ny) diag[v] = mean;
+}
+
+// b_P = P^T r and b_H = H^T r: per vertex the weighted residual entries of the owned cells around it
+__global__ void __launch_bounds__(kMgThreads)
+    k_dg_restrict_q2(const int* done, const double* __restrict__ r, const int32_t* __restrict__ lex_cell, int own0, int n_own,
+                     int nx, int ny, double* __restrict__ bp, double* __restrict__ bh) {
+  if (done && *done) return;
+  const int nx1 = nx + 1;
+  const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v >= int64_t(nx1) * (ny + 1)) return;
+  const int ix = int(v % nx1), iy = int(v / nx1);
+  double sp = 0.0, sh = 0.0;
+#pragma unroll
+  for (int b = 0; b < 2; ++b)
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+      const int cx = ix - 1 + a, cy = iy - 1 + b;
+      if (cx < 0 || cy < 0 || cx >= nx || cy >= ny) continue;
+      const int k = __ldg(lex_cell + cx + nx * cy) - own0;
+      if (k < 0 || k >= n_own) continue;
+      const double* rc = r + size_t(9) * k;
+      const int vx = 1 - a, vy = 1 - b;
+#pragma unroll
+      for (int n = 0; n < 9; ++n) {
+        const double wp = q2_w(vx, n % 3) * q2_w(vy, n / 3);
+        const bool hg = a == 1 && b == 1;
+        if (wp == 0.0 && !hg) continue;
+        const double rn = __ldg(rc + n);
+        if (wp != 0.0) sp = fma(wp, rn, sp);
+        if (hg) sh = fma(q2_g(n % 3) * q2_g(n / 3), rn, sh);
+      }
+    }
+  bp[v] = sp;
+  bh[v] = sh;
+}
+
+// z += P xp + H xh, r.z recomputed; optionally p = z (first direction).  One thread per owned cell.
+__global__ void __launch_bounds__(kMgThreads)
+    k_dg_prolong_dot_q2(const int* done, int32_t n_cells, const int32_t* __restrict__ cell_v0 /* of the owned cells */, int nx,
+                        const double* __restrict__ xp, const double* __restrict__ xh, const double* __restrict__ r,
+                        double* __restrict__ z, double* __restrict__ p_init, double* partial, CgScalars* sc) {
+  if (done && *done) return;
+  const int nx1 = nx + 1;
+  double v[1] = {0.0};
+  const int64_t stride = int64_t(gridDim.x) * blockDim.x;
+  for (int64_t c = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; c < n_cells; c += stride) {
+    const int v0 = __ldg(cell_v0 + c);
+    const double x[4] = {__ldg(xp + v0), __ldg(xp + v0 + 1), __ldg(xp + v0 + nx1), __ldg(xp + v0 + nx1 + 1)};
+    const double h = __ldg(xh + v0);
+#pragma unroll
+    for (int n = 0; n < 9; ++n) {
+      double o = z[9 * c + n];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const double w = q2_w(j & 1, n % 3) * q2_w(j >> 1, n / 3);
+        if (w != 0.0) o = fma(w, x[j], o);
+      }
+      o = fma(q2_g(n % 3) * q2_g(n / 3), h, o);
+      z[9 * c + n] = o;
+      if (p_init) p_init[9 * c + n] = o;
+      v[0] = fma(r[9 * c + n], o, v[0]);
+    }
+  }
+  grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
+}
+
 }  // namespace
 
 // ---- host side ------------------------------------------------------------------------------------------------
@@ -823,6 +999,9 @@ struct MgState {
   bool strips_known = false;
   int nx = 0, ny = 0;
   int n_hier = 2;  // Q1 on cubes: plain + checkerboard-twisted hierarchy; P1 on lattice-structured simplex grids: one
+  // Q2 on cubes ("cg.mg2"): hierarchy 0 for A_P, hierarchy 1 for A_H, each with a level-0 operator of its own (the
+  // twisted Q1 hierarchy instead reads its level-0 operator from the plain one's arrays)
+  bool q2 = false;
   MgDist dist;
 };
 
@@ -963,7 +1142,8 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
       HDD_CUDA(cudaMemsetAsync(c.S.p, 0, size_t(nh) * 9 * c.nv * sizeof(double), s));
       rc = row_range(c, d.own_lo, d.own_hi);
     }
-    k_rap<<<grid2(rc.cnt, nh), kMgThreads, 0, s>>>(f.S.p, l == 0 ? 0 : 9 * f.nv, f.nx, f.ny, (l == 0 && nh == 2) ? 1 : 0, rc, c.S.p,
+    const bool shared = l == 0 && !st.q2;  // level 0 of the twisted hierarchy is read from the plain one's arrays
+    k_rap<<<grid2(rc.cnt, nh), kMgThreads, 0, s>>>(f.S.p, shared ? 0 : 9 * f.nv, f.nx, f.ny, (shared && nh == 2) ? 1 : 0, rc, c.S.p,
                                                   9 * c.nv);
     count_launch();
     if (lc == nd && nd > 0) Nccl::get().all_reduce_sum(c.S.p, size_t(nh) * 9 * c.nv, m->comm, s);
@@ -971,16 +1151,17 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
   for (size_t l = 0; l < nl; ++l) {
     MgLevel& L = *st.levels[l];
     const Rows r = int(l) < nd ? row_range(L, d.b_lo[l], d.b_hi[l]) : Rows{0, L.nv};
-    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), l == 0 ? 1u : unsigned(st.n_hier)), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
+    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), (l == 0 && !st.q2) ? 1u : unsigned(st.n_hier)), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
     count_launch();
   }
   // dense inverses of the coarsest operators (s.p.d.): Gauss-Jordan on the device, one CTA per hierarchy
   MgLevel& C = *st.levels.back();
+  const char* type = st.q2 ? "cg.mg2" : "cg.mg";
   if (C.nv > kMaxCoarse)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "cg.mg: the " << st.nx << " x " << st.ny << " grid cannot be coarsened by halving down to at most "
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, type << ": the " << st.nx << " x " << st.ny << " grid cannot be coarsened by halving down to at most "
                                                            << kMaxCoarse << " vertices (stuck at " << C.nx << " x " << C.ny << ")");
   const int n = int(C.nv);
-  const bool coarsest_is_finest = nl == 1;
+  const bool shared = nl == 1 && !st.q2;  // coarsest = finest level, whose operator the twisted hierarchy shares
   const size_t need = size_t(st.n_hier) * n * n;
   if (st.coarse_inv.n < need) st.coarse_inv.alloc(need);
   if (st.coarse_work.n < need) st.coarse_work.alloc(need);
@@ -992,19 +1173,19 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
   const size_t band_bytes = size_t(n) * size_t(C.nx + 3) * sizeof(double);
   if (!gauss_jordan && band_bytes <= 200 * 1024 && n <= 512) {
     HDD_CUDA(cudaFuncSetAttribute(k_dense_inverse_banded, cudaFuncAttributeMaxDynamicSharedMemorySize, int(band_bytes)));
-    k_dense_inverse_banded<<<st.n_hier, 512, band_bytes, s>>>(C.S.p, coarsest_is_finest ? 0 : int64_t(9) * n, C.nx, C.ny,
-                                                              (coarsest_is_finest && st.n_hier == 2) ? 1 : 0, st.coarse_work.p,
+    k_dense_inverse_banded<<<st.n_hier, 512, band_bytes, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny,
+                                                              (shared && st.n_hier == 2) ? 1 : 0, st.coarse_work.p,
                                                               st.coarse_inv.p, st.coarse_flag.p);
   } else {
-    k_dense_inverse<<<st.n_hier, 1024, 0, s>>>(C.S.p, coarsest_is_finest ? 0 : int64_t(9) * n, C.nx, C.ny,
-                                               (coarsest_is_finest && st.n_hier == 2) ? 1 : 0, st.coarse_work.p, st.coarse_inv.p,
+    k_dense_inverse<<<st.n_hier, 1024, 0, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny,
+                                               (shared && st.n_hier == 2) ? 1 : 0, st.coarse_work.p, st.coarse_inv.p,
                                                st.coarse_flag.p);
   }
   count_launch();
   int bad = 0;
   HDD_CUDA(cudaMemcpyAsync(&bad, st.coarse_flag.p, sizeof(int), cudaMemcpyDeviceToHost, s));
   HDD_CUDA(cudaStreamSynchronize(s));
-  if (bad) HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "cg.mg: the coarsest operator is not positive definite");
+  if (bad) HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, type << ": the coarsest operator is not positive definite");
 }
 
 // levels with at most this many vertices prolongate and post-smooth in one kernel (launch bound there)
@@ -1023,7 +1204,7 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
     MgLevel& L = *st.levels[size_t(l)];
     MgLevel& Cn = *st.levels[size_t(l) + 1];
     const Rows rp = l < nd ? row_range(L, d.pre_lo[l], d.pre_hi[l]) : Rows{0, L.nv};
-    if (l == 0 && nh == 2)
+    if (l == 0 && nh == 2 && !st.q2)
       k_mg_pre2<<<blocks_for(rp.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
     else
       k_mg_pre<<<grid2(rp.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
@@ -1060,7 +1241,7 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
     } else {
       const Rows rq = l < nd ? row_range(L, d.pro_lo[l], d.pro_hi[l]) : Rows{0, L.nv};
       k_mg_prolong_add<<<grid2(rq.cnt, nh), kMgThreads, 0, s>>>(done, Cn.result, L.nx, L.ny, rq, L.x.p);
-      if (l == 0 && nh == 2)
+      if (l == 0 && nh == 2 && !st.q2)
         k_mg_post2<<<blocks_for(ru.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
       else
         k_mg_post<<<grid2(ru.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
@@ -1155,11 +1336,17 @@ static void detect_strips(hdd_swipdg* h, MgState& st) {
 
 void mg_release(MgState* st) { delete st; }
 
-// (re)builds both hierarchies for the frozen operator `vals`
-void mg_setup(hdd_swipdg* h, const double* vals) {
+// (re)builds both hierarchies for the frozen operator `vals`; q2: "cg.mg2", otherwise "cg.mg"
+void mg_setup(hdd_swipdg* h, const double* vals, bool q2) {
   hdd_mesh* m = h->mesh;
   const bool cube = m->kind == HDD_CUBE2D && m->sx > 0, lattice = m->kind == HDD_SIMPLEX2D && m->lx > 0;
-  if ((!cube && !lattice) || h->polorder != 1)
+  if (q2 && h->polorder == 1)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "solver type 'cg.mg2' is the multigrid preconditioner for polOrder 2; use 'cg.mg' for polOrder 1");
+  if (q2 && !cube)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2' needs Q2 on a logically structured HDD_CUBE2D grid with the vertices numbered x-fastest "
+              "(Stuff::Grid::Providers::Cube / hdd_grid_cube); use 'cg.blockdiagonal'");
+  if (!q2 && ((!cube && !lattice) || h->polorder != 1))
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
               "solver type 'cg.mg' needs polOrder 1 on a logically structured grid: HDD_CUBE2D with the vertices numbered x-fastest "
               "(Stuff::Grid::Providers::Cube / hdd_grid_cube) or a simplex grid whose vertices form such a lattice and whose "
@@ -1170,6 +1357,7 @@ void mg_setup(hdd_swipdg* h, const double* vals) {
   st.nx = cube ? m->sx : m->lx;
   st.ny = cube ? m->sy : m->ly;
   st.n_hier = cube ? 2 : 1;
+  st.q2 = q2;
   const int64_t nv = int64_t(st.nx + 1) * (st.ny + 1);
   if (!st.levels.empty() && (st.levels[0]->nx != st.nx || st.levels[0]->ny != st.ny)) {
     st.levels.clear();
@@ -1182,7 +1370,7 @@ void mg_setup(hdd_swipdg* h, const double* vals) {
       L->nx = lx;
       L->ny = ly;
       L->nv = int64_t(lx + 1) * (ly + 1);
-      const size_t ops = l == 0 ? 1 : 2;  // the twisted hierarchy shares the level-0 operator of the plain one
+      const size_t ops = (l == 0 && !q2) ? 1 : 2;  // the twisted hierarchy shares the level-0 operator of the plain one
       L->S.alloc(ops * 9 * size_t(L->nv));
       L->dinv.alloc(ops * size_t(L->nv));
       L->b.alloc(2 * size_t(L->nv));
@@ -1198,8 +1386,9 @@ void mg_setup(hdd_swipdg* h, const double* vals) {
   }
   phase_timer().mark("setup mg: allocation", s);
   // the strip layout depends on the mesh and the communicator only: decided at the first solve of this discretization
-  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated)
-  if (!st.strips_known) {
+  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated).  "cg.mg2" always runs
+  // its vertex levels replicated.
+  if (!st.strips_known && !q2) {
     detect_strips(h, st);
     st.strips_known = true;
   }
@@ -1241,6 +1430,13 @@ void mg_setup(hdd_swipdg* h, const double* vals) {
         f0.S.p, nv, d.lower >= 0 ? lo.p : nullptr, d.upper >= 0 ? up.p : nullptr, st.nx, d.c0, d.c1, g, lo_row, hi_row);
     count_launch();
     HDD_CUDA(cudaStreamSynchronize(s));  // lo / up are freed at the end of this scope
+  } else if (q2) {
+    // every rank writes every vertex (zeros where it owns no cell): the all-reduce makes both operators global
+    k_vertex_galerkin_q2<<<blocks_for(nv), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, f0.S.p);
+    count_launch();
+    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(18) * nv, m->comm, s);
+    k_hourglass_fill<<<1, 1024, 0, s>>>(f0.S.p + 13 * nv, st.nx, st.ny);  // diagonal of hierarchy 1: array 9 + 4
+    count_launch();
   } else if (lattice) {
     if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
     k_vertex_galerkin_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
@@ -1259,7 +1455,8 @@ void mg_setup(hdd_swipdg* h, const double* vals) {
   HDD_CUDA(cudaGetLastError());
 }
 
-// z += P V(P^T r) + P C V_C(C P^T r), red[1] = r.z; p_init != nullptr also stores z as the first direction
+// z += P V(P^T r) + P C V_C(C P^T r) ("cg.mg2": z += P V_P(P^T r) + H V_H(H^T r)), red[1] = r.z; p_init != nullptr also
+// stores z as the first direction
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc) {
   hdd_mesh* m = h->mesh;
   MgState& st = *h->mg;
@@ -1298,6 +1495,11 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
     k_ghost_unpack_twist<<<blocks_for(int64_t(hi_row - lo_row + 1) * nx1), kMgThreads, 0, s>>>(
         done, b0, b1, d.lower >= 0 ? d.tmp_lo.p : nullptr, d.upper >= 0 ? d.tmp_up.p : nullptr, st.nx, d.c0, d.c1, g, lo_row, hi_row);
     count_launch();
+  } else if (st.q2) {
+    // Q2: b0 = P^T r, b1 = H^T r; every rank writes every vertex (zeros where it owns no cell), one all-reduce of both
+    k_dg_restrict_q2<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, b0, b1);
+    count_launch();
+    if (multi) Nccl::get().all_reduce_sum(b0, size_t(2) * a.nv, m->comm, s);
   } else if (st.n_hier == 1) {
     // lattice-structured simplex grid: conforming P1 auxiliary space, one hierarchy
     if (multi) HDD_CUDA(cudaMemsetAsync(b0, 0, size_t(a.nv) * sizeof(double), s));
@@ -1325,7 +1527,10 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
     vcycle(m, st, done, s);
   }
   const int grid = int(std::min<int64_t>((m->n_own + kMgThreads - 1) / kMgThreads, kMaxBlocks));
-  if (st.n_hier == 1)
+  if (st.q2)
+    k_dg_prolong_dot_q2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z,
+                                                    p_init, partial, sc);
+  else if (st.n_hier == 1)
     k_dg_prolong_dot_p1<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
   else
     k_dg_prolong_dot<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z, p_init,

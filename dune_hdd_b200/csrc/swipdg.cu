@@ -370,6 +370,7 @@ int parse_solver_type(const char* type) {
   if (t == "cg.identity" || t == "cg.identity.lower" || t == "cg.identity.upper") return 0;
   if (t == "cg.blockdiagonal" || t == "cg.blockjacobi") return 2;
   if (t == "cg.mg" || t == "cg.multigrid") return 3;
+  if (t == "cg.mg2" || t == "cg.multigrid2") return 4;
   HDD_THROW(HDD_ERR_WRONG_INPUT, "solver type '" << t << "' is not one of solver_types()");
 }
 
@@ -494,7 +495,7 @@ double total(const std::vector<double>& v) {
 const char* const kEstimatorTypes[] = {"eta_NC_ESV2007", "eta_R_ESV2007",  "eta_R_ESV2007_*", "eta_DF_ESV2007", "eta_ESV2007",
                                        "eta_ESV2007_alt", "eta_NC_OS2014", "eta_R_OS2014",    "eta_R_OS2014_*", "eta_DF_OS2014",
                                        "eta_DF_OS2014_*", "eta_OS2014",    "eta_OS2014_*"};
-const char* const kSolverTypes[] = {"cg.diagonal", "cg.blockdiagonal", "cg.identity", "cg.mg"};
+const char* const kSolverTypes[] = {"cg.diagonal", "cg.blockdiagonal", "cg.identity", "cg.mg", "cg.mg2"};
 
 }  // namespace
 
@@ -837,7 +838,7 @@ int hdd_residual(hdd_swipdg* h, const double* mu, int mu_size, double* relative_
 int hdd_solver_types(const char* const** types, int* n_types) {
   return guarded([&] {
     if (types) *types = kSolverTypes;
-    if (n_types) *n_types = 4;
+    if (n_types) *n_types = int(sizeof(kSolverTypes) / sizeof(kSolverTypes[0]));
   });
 }
 
@@ -884,7 +885,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       pt.mark("setup: block inverses", s);
       c.dinv_block = h->dinv_block.p;
       c.z = h->z.p;
-      if (use_diag == 3) mg_setup(h, vals);
+      if (use_diag >= 3) mg_setup(h, vals, use_diag == 4);
     } else {
       launch_extract_dinv(v, vals, use_diag, h->dinv.p, s);
     }
@@ -920,11 +921,11 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       peer = &h->peer_view;
     }
     launch_cg_init(v, c, precision, max_iter, s);
-    if (use_diag == 3) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
+    if (use_diag >= 3) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
     if (multi) nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s);
     launch_cg_init_finish(v, c, s);
     pt.mark("setup: cg init", s);
-    // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg).  The first batch is
+    // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg / cg.mg2).  The first batch is
     // launched directly (one-time attribute / buffer set-up happens there); after that two iterations (parity 0 and 1)
     // are captured into a CUDA graph and replayed, so a launch-bound iteration costs one graph launch instead of up to
     // a hundred kernel launches and does not stall the GPU when the host thread is delayed.  HDD_CG_GRAPH=0 disables it.
@@ -935,7 +936,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       if (multi) { nc.all_reduce_sum(&c.sc->red[0], 1, m->comm, s); pt.mark("all-reduce p.q", s); }
       launch_cg_update(v, c, parity, s);
       pt.mark("update", s);
-      if (use_diag == 3) mg_apply(h, &c.sc->done[parity], c.r, c.z, nullptr, c.partial, c.sc);
+      if (use_diag >= 3) mg_apply(h, &c.sc->done[parity], c.r, c.z, nullptr, c.partial, c.sc);
       if (multi) { nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s); pt.mark("all-reduce r.z", s); }
       launch_cg_direction(v, c, parity, s);
       pt.mark("direction", s);
@@ -952,7 +953,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     }
     bool capture_failed = false;
     double rr_prev = 1e300;
-    int par = 0, launched = 0, batch = use_diag == 3 ? 8 : 16;
+    int par = 0, launched = 0, batch = use_diag >= 3 ? 8 : 16;
     bool first_batch = !cached.exec;  // a cached graph means every one-time set-up has already happened
     for (;;) {
       if (!first_batch && graphs_wanted && !cached.exec && !capture_failed) {

@@ -210,10 +210,13 @@ typedef struct hdd_solve_info {
 
 /* solver_types() / solver_options(type) (discretizations/base.hh:314-322). Types: "cg.diagonal" (default,
  * Jacobi), "cg.blockdiagonal" (block Jacobi with the n_loc x n_loc cell blocks), "cg.identity", and "cg.mg": CG with
- * a two-level preconditioner (block Jacobi + conforming-Q1 coarse space solved by geometric multigrid V-cycles, the
- * counterpart of the AMG-preconditioned default of the reference's Stuff::LA::Solver) - polOrder 1 on logically
- * structured HDD_CUBE2D grids only, HDD_ERR_REQUIREMENTS_NOT_MET otherwise.  Aliases "cg", "cg.jacobi",
- * "cg.diagonal.lower", "cg.identity.lower", "cg.blockjacobi", "cg.multigrid". */
+ * a two-level preconditioner (block Jacobi + conforming-Q1 / P1 coarse space solved by geometric multigrid V-cycles,
+ * the counterpart of the AMG-preconditioned default of the reference's Stuff::LA::Solver) - polOrder 1 on logically
+ * structured grids: HDD_CUBE2D with the vertices numbered x-fastest, or a simplex grid whose vertices form such a
+ * lattice and whose triangles join lattice neighbours; and "cg.mg2": the same for polOrder 2 (block Jacobi with the
+ * 9 x 9 cell blocks + conforming Q1 + the Q2 hourglass family, one V-cycle each) - Q2 on logically structured
+ * HDD_CUBE2D grids only.  Elsewhere both give HDD_ERR_REQUIREMENTS_NOT_MET.  Aliases "cg", "cg.jacobi",
+ * "cg.diagonal.lower", "cg.identity.lower", "cg.blockjacobi", "cg.multigrid", "cg.multigrid2". */
 int hdd_solver_types(const char* const** types, int* n_types);
 /* uncached_solve(options, vector, mu) (discretizations/base.hh:327-367): freeze lhs and rhs at mu, CG.
  * precision / max_iter mirror Stuff::LA::Solver's option keys.  x_host[n_owned] receives the solution
