@@ -11,7 +11,7 @@ SOURCES = ["mesh.cu", "swipdg.cu", "products.cu", "kernels_assembly.cu", "kernel
            "grids.cpp", "partition.cpp"]
 HEADERS = ["common.hpp", "expr.hpp", "quadrature.hpp", "device.cuh", "reduce.cuh", "kernels.hpp", "handles.hpp",
            "partition.hpp",
-           os.path.join("..", "..", "include", "hdd_b200.h")]
+           os.path.join("..", "..", "include", "hdd_b200.h"), os.path.join("..", "..", "include", "hdd_b200_testing.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
          "-Xcompiler", "-fPIC,-Wall,-Wno-unknown-pragmas", "-x", "cu"]

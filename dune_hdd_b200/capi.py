@@ -51,7 +51,7 @@ class hdd_parameters(C.Structure):
                 ("mu_size", C.c_int)]
 
 
-# every symbol include/hdd_b200.h declares (checked by tests/test_capi_symbols.py)
+# every symbol include/hdd_b200.h declares (checked by tests/test_host_logic.py)
 SYMBOLS = [
     "hdd_last_error", "hdd_version", "hdd_mesh_create", "hdd_mesh_destroy", "hdd_mesh_num_cells",
     "hdd_grid_cube_sizes", "hdd_grid_cube", "hdd_grid_simplex_sizes", "hdd_grid_simplex", "hdd_swipdg_create",
@@ -64,8 +64,11 @@ SYMBOLS = [
     "hdd_kernel_bytes", "hdd_expression_evaluate", "hdd_partition_plan", "hdd_free",
     "hdd_swipdg_only_these_products", "hdd_products_available", "hdd_product_num_components", "hdd_product_values",
     "hdd_product_coefficient", "hdd_pattern_volume", "hdd_product_apply2", "hdd_error_norms",
-    "hdd_host_alloc", "hdd_host_free", "hdd_grid_fathers", "hdd_prolong", "hdd_residual", "hdd_mg_strip_plan", "hdd_fast_cos", "hdd_trig_product", "hdd_partition_plan_local", "hdd_mesh_create_cube", "hdd_h2d_bytes",
+    "hdd_host_alloc", "hdd_host_free", "hdd_grid_fathers", "hdd_prolong", "hdd_residual", "hdd_partition_plan_local", "hdd_mesh_create_cube", "hdd_h2d_bytes",
 ]
+
+# every symbol include/hdd_b200_testing.h declares: the entry points of the tests
+TESTING_SYMBOLS = ["hdd_mg_strip_plan", "hdd_fast_cos", "hdd_trig_product", "hdd_precondition", "hdd_mg_level_operator"]
 
 _lib = None
 

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "../../include/hdd_b200.h"
+#include "../../include/hdd_b200_testing.h"
 
 namespace hdd {
 

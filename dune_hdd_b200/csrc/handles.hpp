@@ -269,6 +269,8 @@ void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_de
 void mg_setup(hdd_swipdg* h, const double* frozen_values, bool q2);
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc);
 void mg_release(MgState* st);
+// copies the finest level's V-cycle results of the last mg_apply, n_hier (nx+1)(ny+1) doubles, on the handle's stream
+void mg_vertex_result(const hdd_swipdg* h, double* host);
 int mg_num_levels(const hdd_swipdg* h);  // the product assemblers added to system_assembler (discretizations/swipdg.hh:359-479)
 DevCombo make_combo(const hdd_swipdg* h, const AffineFn& f, const double* mu, int mu_size);  // f frozen at mu
 }  // namespace hdd

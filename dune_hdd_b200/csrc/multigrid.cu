@@ -1542,7 +1542,36 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
 
 int mg_num_levels(const hdd_swipdg* h) { return h->mg ? int(h->mg->levels.size()) : 0; }
 
+void mg_vertex_result(const hdd_swipdg* h, double* host) {
+  const MgLevel& a = *h->mg->levels[0];
+  HDD_CUDA(cudaMemcpyAsync(host, a.result, size_t(h->mg->n_hier) * a.nv * sizeof(double), cudaMemcpyDeviceToHost,
+                           h->mesh->stream));
+}
+
 }  // namespace hdd
+
+extern "C" int hdd_mg_level_operator(const hdd_swipdg* h, int level, int hier, int* nx, int* ny, double* S_host) {
+  return hdd::guarded([&] {
+    if (!h) HDD_THROW(HDD_ERR_WRONG_INPUT, "discretization handle is NULL");
+    const hdd::MgState* st = h->mg;
+    if (!st) HDD_THROW(HDD_ERR_USING_THIS_WRONG, "no multigrid hierarchy: solve with 'cg.mg' or 'cg.mg2' first");
+    if (level < 0 || level >= int(st->levels.size()))
+      HDD_THROW(HDD_ERR_WRONG_INPUT, "level " << level << " of " << st->levels.size());
+    if (hier < 0 || hier >= st->n_hier) HDD_THROW(HDD_ERR_WRONG_INPUT, "hierarchy " << hier << " of " << st->n_hier);
+    if (level == 0 && hier == 1 && !st->q2)
+      HDD_THROW(HDD_ERR_WRONG_INPUT, "level 0 of the twisted hierarchy is C A_c C, read from the plain one's arrays");
+    const hdd::MgLevel& L = *st->levels[size_t(level)];
+    if (nx) *nx = L.nx;
+    if (ny) *ny = L.ny;
+    if (S_host) {
+      h->mesh->set_device();
+      cudaStream_t s = h->mesh->stream;
+      HDD_CUDA(cudaMemcpyAsync(S_host, L.S.p + size_t(hier) * 9 * L.nv, size_t(9) * L.nv * sizeof(double),
+                               cudaMemcpyDeviceToHost, s));
+      HDD_CUDA(cudaStreamSynchronize(s));
+    }
+  });
+}
 
 // host-only view of the strip plan for the CPU tests: out[8 * l + {0..7}] = pre_lo, pre_hi, b_lo, b_hi, up_lo, up_hi,
 // pro_lo, pro_hi of level l; out[8 * n_dist + {0, 1, 2}] = own_lo, own_hi, ghost

@@ -842,6 +842,83 @@ int hdd_solver_types(const char* const** types, int* n_types) {
   });
 }
 
+namespace {
+
+struct CgStart {
+  const double* vals = nullptr;  // the frozen operator the iteration reads
+  bool p2p = false;
+  const PeerView* peer = nullptr;
+};
+
+// The start of a CG solve, shared by hdd_solve and hdd_precondition: A(mu) frozen (and b(mu) into c.b if freeze_b), the
+// pure-Neumann fix, the preconditioner's set-up, the peer-memory decision, then x = 0, r = b, p = z = M^-1 b and
+// rz[0] = r.z.  The caller provides c.b, c.x, c.r, c.z (block Jacobi and multigrid), c.p, c.q, c.partial and c.sc.
+CgStart start_cg(hdd_swipdg* h, int use_diag, const double* mu, int mu_size, bool freeze_b, double precision, int max_iter,
+                 CgBuffers& c) {
+  hdd_mesh* m = h->mesh;
+  cudaStream_t s = m->stream;
+  SolvePhases& pt = phase_timer();
+  CgStart st;
+  const double* vals = freeze_lhs(h, mu, mu_size);
+  if (freeze_b) freeze_rhs(h, mu, mu_size);
+  pt.mark("setup: freeze", s);
+  const MeshView v = h->view();
+  if (m->purely_neumann) {
+    // discretizations/base.hh:337-345: unit_row(0), rhs[0] = 0, solve, subtract the mean
+    if (m->world > 1) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "pure Neumann problems on more than one GPU");
+    if (!h->frozen.p) h->frozen.alloc(size_t(h->nnz));
+    if (vals != h->frozen.p)
+      HDD_CUDA(cudaMemcpyAsync(h->frozen.p, vals, size_t(h->nnz) * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    launch_unit_row_col0(v, h->frozen.p, h->b.p, s);  // c.b is h->b here: hdd_precondition refuses this case
+    vals = h->frozen.p;
+  }
+  c.values = vals;
+  c.dinv = h->dinv.p;
+  if (use_diag >= 2) {
+    if (!h->dinv_block.p) h->dinv_block.alloc(size_t(m->n_own) * h->nl * h->nl);
+    launch_invert_diag_blocks(v, vals, h->dinv_block.p, s);
+    pt.mark("setup: block inverses", s);
+    c.dinv_block = h->dinv_block.p;
+    if (use_diag >= 3) mg_setup(h, vals, use_diag == 4);
+  } else {
+    c.z = nullptr;
+    launch_extract_dinv(v, vals, use_diag, h->dinv.p, s);
+  }
+  Nccl& nc = Nccl::get();
+  const bool multi = m->world > 1;
+  // multi GPU, Q1, Jacobi / identity: fused SpMV + halo read over peer memory instead of pack + send/recv
+  bool p2p = multi && p2p_wanted() && use_diag < 2 && cg_spmv_uses_tma(v);
+  if (multi && use_diag < 2) {  // the decision must be collective: a rank without owned cells large enough would disagree
+    DevBuf<double> vote;
+    double want = p2p ? 0.0 : 1.0;
+    vote.upload(&want, 1, s);
+    nc.all_reduce_sum(vote.p, 1, m->comm, s);
+    HDD_CUDA(cudaMemcpyAsync(&want, vote.p, sizeof(double), cudaMemcpyDeviceToHost, s));
+    HDD_CUDA(cudaStreamSynchronize(s));
+    p2p = (want == 0.0);
+  }
+  if (p2p) p2p = setup_p2p(h);
+  pt.mark("setup: solver vote", s);
+  if (p2p) {
+    // Jacobi diagonal including the halo (static during the solve): owned part computed here, halo exchanged once
+    double* dl = h->dinv_local.p;
+    HDD_CUDA(cudaMemcpyAsync(dl + size_t(m->own0) * h->nl, h->dinv.p, size_t(h->n_rows) * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    m->halo_exchange(dl, h->nl);
+    c.p_alt = h->p_alt.p;
+    st.peer = &h->peer_view;
+  }
+  launch_cg_init(v, c, precision, max_iter, s);
+  if (use_diag >= 3) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
+  if (multi) nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s);
+  launch_cg_init_finish(v, c, s);
+  pt.mark("setup: cg init", s);
+  st.vals = vals;
+  st.p2p = p2p;
+  return st;
+}
+
+}  // namespace
+
 int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, const double* mu, int mu_size,
               double* x_host, hdd_solve_info* info) {
   return guarded([&] {
@@ -853,78 +930,34 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     m->set_device();
     cudaStream_t s = m->stream;
     ensure_solve_workspace(h);
+    if (use_diag >= 2 && !h->z.p) h->z.alloc(size_t(h->n_rows));
     cudaEvent_t e0, e1;
     HDD_CUDA(cudaEventCreate(&e0));
     HDD_CUDA(cudaEventCreate(&e1));
     HDD_CUDA(cudaEventRecord(e0, s));
     SolvePhases& pt = phase_timer();
     pt.begin(s);
-    const double* vals = freeze_lhs(h, mu, mu_size);
-    freeze_rhs(h, mu, mu_size);
-    pt.mark("setup: freeze", s);
-    const MeshView v = h->view();
-    if (m->purely_neumann) {
-      // discretizations/base.hh:337-345: unit_row(0), rhs[0] = 0, solve, subtract the mean
-      if (m->world > 1) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "pure Neumann problems on more than one GPU");
-      if (!h->frozen.p) h->frozen.alloc(size_t(h->nnz));
-      if (vals != h->frozen.p)
-        HDD_CUDA(cudaMemcpyAsync(h->frozen.p, vals, size_t(h->nnz) * sizeof(double), cudaMemcpyDeviceToDevice, s));
-      launch_unit_row_col0(v, h->frozen.p, h->b.p, s);
-      vals = h->frozen.p;
-    }
-    CgBuffers c{};
-    c.values = vals;
-    c.dinv = h->dinv.p;
     h->last_precond = use_diag;
-    if (use_diag >= 2) {
-      if (!h->dinv_block.p) {
-        h->dinv_block.alloc(size_t(m->n_own) * h->nl * h->nl);
-        h->z.alloc(size_t(h->n_rows));
-      }
-      launch_invert_diag_blocks(v, vals, h->dinv_block.p, s);
-      pt.mark("setup: block inverses", s);
-      c.dinv_block = h->dinv_block.p;
-      c.z = h->z.p;
-      if (use_diag >= 3) mg_setup(h, vals, use_diag == 4);
-    } else {
-      launch_extract_dinv(v, vals, use_diag, h->dinv.p, s);
-    }
+    CgBuffers c{};
     c.b = h->b.p;
     c.x = h->x.p;
     c.r = h->r.p;
+    c.z = h->z.p;
     c.p = h->p.p;
     c.q = h->q.p;
     c.partial = h->partial.p;
     c.sc = h->sc.p;
+    if (!c.b) {  // freeze_rhs allocates b at the first solve
+      h->b.alloc(size_t(h->n_rows));
+      c.b = h->b.p;
+    }
+    const CgStart st = start_cg(h, use_diag, mu, mu_size, true, precision, max_iter, c);
+    const double* vals = st.vals;
+    const bool p2p = st.p2p;
+    const PeerView* peer = st.peer;
+    const MeshView v = h->view();
     Nccl& nc = Nccl::get();
     const bool multi = m->world > 1;
-    // multi GPU, Q1, Jacobi / identity: fused SpMV + halo read over peer memory instead of pack + send/recv
-    bool p2p = multi && p2p_wanted() && use_diag < 2 && cg_spmv_uses_tma(v);
-    if (multi && use_diag < 2) {  // the decision must be collective: a rank without owned cells large enough would disagree
-      DevBuf<double> vote;
-      double want = p2p ? 0.0 : 1.0;
-      vote.upload(&want, 1, s);
-      nc.all_reduce_sum(vote.p, 1, m->comm, s);
-      HDD_CUDA(cudaMemcpyAsync(&want, vote.p, sizeof(double), cudaMemcpyDeviceToHost, s));
-      HDD_CUDA(cudaStreamSynchronize(s));
-      p2p = (want == 0.0);
-    }
-    if (p2p) p2p = setup_p2p(h);
-    pt.mark("setup: solver vote", s);
-    const PeerView* peer = nullptr;
-    if (p2p) {
-      // Jacobi diagonal including the halo (static during the solve): owned part computed here, halo exchanged once
-      double* dl = h->dinv_local.p;
-      HDD_CUDA(cudaMemcpyAsync(dl + size_t(m->own0) * h->nl, h->dinv.p, size_t(h->n_rows) * sizeof(double), cudaMemcpyDeviceToDevice, s));
-      m->halo_exchange(dl, h->nl);
-      c.p_alt = h->p_alt.p;
-      peer = &h->peer_view;
-    }
-    launch_cg_init(v, c, precision, max_iter, s);
-    if (use_diag >= 3) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
-    if (multi) nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s);
-    launch_cg_init_finish(v, c, s);
-    pt.mark("setup: cg init", s);
     // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg / cg.mg2).  The first batch is
     // launched directly (one-time attribute / buffer set-up happens there); after that two iterations (parity 0 and 1)
     // are captured into a CUDA graph and replayed, so a launch-bound iteration costs one graph launch instead of up to
@@ -1039,6 +1072,50 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     if (!converged)
       HDD_THROW(HDD_ERR_NOT_CONVERGED, "CG did not reach precision " << precision << " in " << sc.it[par]
                                                                      << " iterations (relative residual " << relres << ")");
+  });
+}
+
+int hdd_precondition(hdd_swipdg* h, const char* type, const double* mu, int mu_size, const double* r_host,
+                     double* z_host, double* rz, double* vertex_host) {
+  return guarded([&] {
+    require_init(h);
+    check_mu(h, mu, mu_size, "mu");
+    const int use_diag = parse_solver_type(type);
+    if (!r_host || !z_host) HDD_THROW(HDD_ERR_WRONG_INPUT, "r_host and z_host must not be NULL");
+    if (vertex_host && use_diag < 3) HDD_THROW(HDD_ERR_WRONG_INPUT, "vertex_host needs a multigrid solver type");
+    hdd_mesh* m = h->mesh;
+    if (m->world > 1) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "hdd_precondition on more than one GPU");
+    if (m->purely_neumann) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "hdd_precondition for the modified pure-Neumann system");
+    m->set_device();
+    cudaStream_t s = m->stream;
+    ensure_solve_workspace(h);
+    const size_t rows = size_t(h->n_rows);
+    // scratch copies of everything the set-up writes besides the preconditioner's own state
+    DevBuf<double> b, x, r, z, p, q, partial;
+    DevBuf<CgScalars> sc;
+    b.alloc(rows);
+    x.alloc(rows);
+    r.alloc(rows);
+    z.alloc(rows);
+    p.alloc(size_t(m->n_loc) * h->nl);
+    q.alloc(rows);
+    partial.alloc(size_t(cg_partial_capacity()));
+    sc.alloc(1);
+    HDD_CUDA(h2d_async(b.p, r_host, rows * sizeof(double), s));
+    CgBuffers c{};
+    c.b = b.p;
+    c.x = x.p;
+    c.r = r.p;
+    c.z = z.p;
+    c.p = p.p;
+    c.q = q.p;
+    c.partial = partial.p;
+    c.sc = sc.p;
+    start_cg(h, use_diag, mu, mu_size, false, 1.0, 1, c);
+    HDD_CUDA(cudaMemcpyAsync(z_host, p.p + size_t(m->own0) * h->nl, rows * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (rz) HDD_CUDA(cudaMemcpyAsync(rz, &sc.p->rz[0], sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (vertex_host) mg_vertex_result(h, vertex_host);
+    HDD_CUDA(cudaStreamSynchronize(s));
   });
 }
 

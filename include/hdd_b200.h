@@ -332,21 +332,7 @@ int hdd_partition_plan_local(int kind, int64_t n_cells, const int32_t* cell_vert
                              const int64_t* rank_cell_offsets, int rank, int32_t** halo_cells, int64_t* n_halo,
                              int32_t** send_cells, int64_t* send_offsets);
 int hdd_free(void* p);
-/* Host arithmetic of the strip-distributed multigrid preconditioner ("cg.mg" on N GPUs, DESIGN.md 7), exported for the CPU
- * tests: the inclusive vertex-row ranges the sweeps of the n_dist finest vertex levels run on for the rank owning the cell
- * rows [c0, c1) of an ny-row structured grid.  out[8 l + k], k = 0..7: pre_lo, pre_hi (pre-smoothing), b_lo, b_hi
- * (right-hand side), up_lo, up_hi (post-smoothing), pro_lo, pro_hi (prolongation) of level l; out[8 n_dist + {0,1,2}]:
- * first and last own row of the first replicated level, and the number of level-0 rows received from each neighbour.
- * No device needed. */
-int hdd_mg_strip_plan(int ny, int c0, int c1, int n_dist, int* out);
-/* The branch-free cosine the estimator kernel evaluates trigonometric data functions with (csrc/expr.hpp: fast_cos, valid
- * for |x| <= 1e5), run on the host for the CPU tests: out[i] = fast_cos(x[i]).  No device needed. */
-int hdd_fast_cos(const double* x, int64_t n, double* out);
-/* Whether the kernels would evaluate the Expression `expression` (variable "x") as a product of at most two cosines of
- * affine arguments (csrc/expr.hpp: TrigProduct), and with which numbers: out[7] = c, a0, b0, d0, a1, b1, d1 of
- * c cos(a0 x[0] + b0 x[1] + d0) cos(a1 x[0] + b1 x[1] + d1); *valid = 0 if the expression has another shape (it is then
- * evaluated by the general path).  For the CPU tests; no device needed. */
-int hdd_trig_product(const char* expression, double* out, int* valid);
+/* Entry points for tests (host arithmetic, the preconditioners' intermediate results) are in hdd_b200_testing.h. */
 
 /* ---- measurement ------------------------------------------------------------------------------------------------ */
 /* Times `reps` back-to-back launches of one hot kernel on the handle's stream with CUDA events (after 3 warm-up

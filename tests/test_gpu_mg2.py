@@ -137,3 +137,8 @@ def test_cg_mg2_requirements(gpu):
     # the same discretization still solves with block Jacobi
     u, info = dp.solve({"type": "cg.blockdiagonal", "precision": 1e-10, "max_iter": 5000}, return_info=True)
     assert info["converged"]
+    # 42 x 42: halving stops at 21 x 21 vertex cells (484 vertices > 400, odd)
+    d42 = hdd.SWIPDG(grids.cube(42), problems.ESV2007(), polorder=2)
+    d42.init()
+    with pytest.raises(hdd.discretizations.requirements_not_met, match="21 x 21"):
+        d42.solve({"type": "cg.mg2", "precision": 1e-10, "max_iter": 100})

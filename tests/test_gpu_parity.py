@@ -354,9 +354,10 @@ def test_neumann_faces_and_pure_neumann_fix(gpu):
         b2[0] = 0.0
         x = spla.spsolve(S.tocsc(), b2)
         x -= x.mean()
-        u = d.solve({"type": "cg.diagonal", "precision": 1e-13, "max_iter": 50000})
-        assert abs(u.mean()) <= 1e-12 * np.abs(u).max()
-        assert rel(u, x) <= 1e-7
+        for typ in ("cg.diagonal", "cg.mg"):  # the multigrid hierarchy is built from the unit-row operator
+            u = d.solve({"type": typ, "precision": 1e-13, "max_iter": 50000})
+            assert abs(u.mean()) <= 1e-12 * np.abs(u).max(), typ
+            assert rel(u, x) <= 1e-7, typ
 
 
 # ---- polOrder 2 (BASELINE config 5: "SWIPDG p1 and p2"): P2 / Q2, GPU vs oracle -----------------------------------
@@ -634,6 +635,11 @@ def test_cg_mg_spe10_shape_parametric_and_requirements(gpu):
     dq.init()
     with pytest.raises(hdd.discretizations.requirements_not_met):
         dq.solve({"type": "cg.mg", "precision": 1e-10, "max_iter": 100})
+    # 42 x 42: halving stops at 21 x 21 vertex cells (484 vertices > 400, odd)
+    d42 = hdd.SWIPDG(grids.cube(42), problems.ESV2007())
+    d42.init()
+    with pytest.raises(hdd.discretizations.requirements_not_met, match="21 x 21"):
+        d42.solve({"type": "cg.mg", "precision": 1e-10, "max_iter": 100})
 
 
 @pytest.mark.parametrize("kind,n,polorder", [("alu", 16, 1), ("alu", 32, 1), ("alu", 16, 2), ("sgrid", 32, 2), ("sgrid", 40, 1)])

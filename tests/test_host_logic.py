@@ -14,26 +14,32 @@ from oracle import oracle as o
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+HEADERS = {"hdd_b200.h": capi.SYMBOLS, "hdd_b200_testing.h": capi.TESTING_SYMBOLS}
+
+
 def test_library_exports_every_symbol_the_header_declares():
     L = capi.lib()
-    header = open(os.path.join(ROOT, "include", "hdd_b200.h")).read()
-    declared = set(re.findall(r"\b(hdd_[a-z0-9_]+)\s*\(", header))
-    declared -= {"hdd_status"}
-    assert declared == set(capi.SYMBOLS), declared ^ set(capi.SYMBOLS)
-    for name in capi.SYMBOLS:
-        assert hasattr(L, name), name
+    for name, symbols in HEADERS.items():
+        header = open(os.path.join(ROOT, "include", name)).read()
+        declared = set(re.findall(r"\b(hdd_[a-z0-9_]+)\s*\(", header))
+        declared -= {"hdd_status"}
+        assert declared == set(symbols), (name, declared ^ set(symbols))
+        for sym in symbols:
+            assert hasattr(L, sym), sym
     assert b"sm_100a" in L.hdd_version()
 
 
 def test_header_is_plain_c_and_matches_the_definitions(tmp_path):
     """include/hdd_b200.h is the drop-in boundary: it has to compile as C99 (cgo / JNI / ctypes generators read it) and
     as C++ against the definitions - the csrc files include it, so a drifted prototype would already fail the build;
-    here the C side is checked"""
+    here the C side is checked.  The same for include/hdd_b200_testing.h, the entry points of the tests."""
     import subprocess
-    header = os.path.join(ROOT, "include", "hdd_b200.h")
-    subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Wextra", "-Werror", "-pedantic", "-fsyntax-only", "-x", "c", header])
+    for name in HEADERS:
+        header = os.path.join(ROOT, "include", name)
+        subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Wextra", "-Werror", "-pedantic", "-fsyntax-only", "-x", "c", header])
     src = tmp_path / "use.c"
-    src.write_text('#include "hdd_b200.h"\nint main(void) { return hdd_version() == 0; }\n')
+    src.write_text('#include "hdd_b200_testing.h"\n'
+                   'int main(void) { double c; return hdd_version() == 0 || hdd_fast_cos(&c, 0, &c) != HDD_OK; }\n')
     libdir = os.path.join(ROOT, "dune_hdd_b200")
     capi.lib()
     subprocess.check_call(["gcc", "-std=c99", "-Wall", "-Werror", "-I" + os.path.join(ROOT, "include"), str(src), "-L" + libdir,

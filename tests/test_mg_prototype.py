@@ -6,7 +6,8 @@ restatement of the preconditioner on oracle-assembled matrices.
 With the reference's midpoint-rule volume term the conforming auxiliary operator A_c = P^T A P has a second family of
 low-energy modes (checkerboard x smooth).  A plain multigrid hierarchy does not see it - the CG iteration count grows
 with 1/h - while the additional checkerboard-twisted hierarchy brings it back to the count of an exact coarse solve.
-The CUDA path is compared with direct solves in tests/test_gpu_parity.py; this file pins the algorithm itself on CPU."""
+The CUDA path is compared with direct solves in tests/test_gpu_parity.py and operator by operator with the restatement
+in tests/mg_reference.py in tests/test_gpu_preconditioners.py; this file pins the algorithm itself on CPU."""
 import warnings
 
 import numpy as np
@@ -14,41 +15,9 @@ import scipy.sparse as sp
 import scipy.sparse.linalg as spla
 
 from oracle import oracle as o
+from tests.mg_reference import hierarchy, vcycle
 
 warnings.filterwarnings("ignore")
-
-
-def _interp1d(nc):
-    rows, cols, vals = [], [], []
-    for i in range(2 * nc + 1):
-        if i % 2 == 0:
-            rows.append(i); cols.append(i // 2); vals.append(1.0)
-        else:
-            rows += [i, i]; cols += [i // 2, i // 2 + 1]; vals += [0.5, 0.5]
-    return sp.csr_matrix((vals, (rows, cols)), shape=(2 * nc + 1, nc + 1))
-
-
-def _hierarchy(Ac, n):
-    levels = [{"A": Ac.tocsr(), "n": n}]
-    while n > 2 and n % 2 == 0:
-        I = _interp1d(n // 2)
-        Pm = sp.kron(I, I).tocsr()
-        levels[-1]["P"] = Pm
-        levels.append({"A": (Pm.T @ levels[-1]["A"] @ Pm).tocsr(), "n": n // 2})
-        n //= 2
-    levels[-1]["lu"] = spla.splu(levels[-1]["A"].tocsc())
-    for L in levels:
-        L["dinv"] = 0.8 / L["A"].diagonal()  # damped Jacobi, omega = 0.8
-    return levels
-
-
-def _vcycle(levels, l, b):
-    L = levels[l]
-    if "lu" in L:
-        return L["lu"].solve(b)
-    x = L["dinv"] * b
-    x = x + L["P"] @ _vcycle(levels, l + 1, L["P"].T @ (b - L["A"] @ x))
-    return x + L["dinv"] * (b - L["A"] @ x)
 
 
 def _iterations(n, variant):
@@ -65,7 +34,8 @@ def _iterations(n, variant):
     far = (np.abs(ix[coo.row] - ix[coo.col]) > 1) | (np.abs(iy[coo.row] - iy[coo.col]) > 1)
     assert np.abs(coo.data[far]).max(initial=0.0) <= 1e-12 * np.abs(coo.data).max()
     C = sp.diags((-1.0) ** (ix + iy))
-    lv, lvC = _hierarchy(Ac, n), _hierarchy((C @ Ac @ C).tocsr(), n)
+    # the prototype coarsens down to 3 x 3 vertices (the device stops at 400)
+    lv, lvC = hierarchy(Ac, n, n, max_coarse=9), hierarchy((C @ Ac @ C).tocsr(), n, n, max_coarse=9)
     lu = spla.splu(Ac.tocsc())
     D = sp.block_diag([sp.csr_matrix(np.linalg.inv(A[4 * c:4 * c + 4, 4 * c:4 * c + 4].toarray())) for c in range(m.nc)], format="csr")
 
@@ -73,9 +43,9 @@ def _iterations(n, variant):
         z, rc = D @ r, P.T @ r
         if variant == "exact":
             return z + P @ lu.solve(rc)
-        z = z + P @ _vcycle(lv, 0, rc)
+        z = z + P @ vcycle(lv, rc)
         if variant == "twisted":
-            z = z + P @ (C @ _vcycle(lvC, 0, C @ rc))
+            z = z + P @ (C @ vcycle(lvC, C @ rc))
         return z
 
     it = [0]

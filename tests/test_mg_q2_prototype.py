@@ -9,8 +9,8 @@ gets s[v0(c)] g with v0(c) the cell's lower-left vertex and g = (2/3, -1/3, 2/3)
 a constant factor is integrated with the 2 x 2 Gauss rule, under which the cell function (x^2 - 1/3)(y^2 - 1/3) has a zero
 gradient at every quadrature point; it is continuous across faces, so a field of that shape with a smoothly varying
 amplitude has almost no energy, and neither the conforming Q1 space nor the cell blocks represent it.  Without H the CG
-iteration count grows with 1/h; with H it stays flat.  V_P and V_H are one geometric V(1,1)-cycle each (the helpers of
-tests/test_mg_prototype.py).  The CUDA path is compared with direct solves in tests/test_gpu_mg2.py."""
+iteration count grows with 1/h; with H it stays flat.  V_P and V_H are one geometric V(1,1)-cycle each
+(tests/mg_reference.py).  The CUDA path is compared with direct solves in tests/test_gpu_mg2.py."""
 import warnings
 
 import numpy as np
@@ -18,46 +18,9 @@ import scipy.sparse as sp
 import scipy.sparse.linalg as spla
 
 from oracle import oracle as o
-from tests.test_mg_prototype import _hierarchy, _vcycle
+from tests.mg_reference import from_stencil, hierarchy, hourglass_fill, to_stencil, transfers, vcycle
 
 warnings.filterwarnings("ignore")
-
-G1 = np.array([2.0 / 3.0, -1.0 / 3.0, 2.0 / 3.0])
-HOURGLASS = np.outer(G1, G1).ravel()  # node a + 3 b
-
-
-def _w(i, a):
-    return 1.0 - a / 2.0 if i == 0 else a / 2.0
-
-
-def _operators(m):
-    """P (conforming Q1 -> Q2-DG) and H (hourglass family indexed by the lower-left vertex) as sparse matrices"""
-    N, nv, nc = m.n_dofs, m.nv, m.nc
-    cv = m.cv.reshape(-1, 4)
-    rows, cols, vals = [], [], []
-    for c in range(nc):
-        for b in range(3):
-            for a in range(3):
-                for j in range(2):
-                    for i in range(2):
-                        w = _w(i, a) * _w(j, b)
-                        if w:
-                            rows.append(9 * c + a + 3 * b); cols.append(cv[c, i + 2 * j]); vals.append(w)
-    P = sp.csr_matrix((vals, (rows, cols)), shape=(N, nv))
-    H = sp.csr_matrix((np.tile(HOURGLASS, nc), (np.arange(N), np.repeat(cv[:, 0], 9))), shape=(N, nv))
-    return P, H
-
-
-def _hourglass_operator(A, H):
-    """H^T A H; the rows of the top vertex row and the right vertex column are empty (no cell has its lower-left vertex
-    there) and get the mean diagonal"""
-    Ah = (H.T @ A @ H).tolil()
-    d = Ah.diagonal()
-    mean = d[d > 0].mean()
-    for v in np.flatnonzero(d == 0):
-        Ah[v, v] = mean
-    return Ah.tocsr()
-
 
 def _iterations(n, variant, tensor=None):
     m = o.mesh_cube(n, n, -1.0, 1.0, -1.0, 1.0).with_polorder(2)
@@ -65,23 +28,21 @@ def _iterations(n, variant, tensor=None):
     A = o.to_scipy(rp, col, o.assemble_lhs(m, o.const(1.0), tensor, rp, col)).tocsr()
     b = o.assemble_rhs(m, o.esv2007_force())
     N, nv = m.n_dofs, m.nv
-    P, H = _operators(m)
-    Ap, Ah = (P.T @ A @ P).tocsr(), _hourglass_operator(A, H)
-    # both auxiliary operators are 9-point vertex stencils: nothing at index distance 2 (A_P: jumps of continuous
-    # functions cancel; A_H: only cells sharing a face couple, and their lower-left vertices are lattice neighbours)
-    ix, iy = np.arange(nv) % (n + 1), np.arange(nv) // (n + 1)
-    for S in (Ap, Ah):
-        coo = S.tocoo()
-        far = (np.abs(ix[coo.row] - ix[coo.col]) > 1) | (np.abs(iy[coo.row] - iy[coo.col]) > 1)
-        assert np.abs(coo.data[far]).max(initial=0.0) <= 1e-12 * np.abs(coo.data).max()
-    lvp, lvh = _hierarchy(Ap, n), _hierarchy(Ah, n)
+    P, H = transfers("q2", m.cv.reshape(-1, 4), nv)
+    # both auxiliary operators are 9-point vertex stencils (to_stencil asserts that nothing is at index distance 2: A_P:
+    # jumps of continuous functions cancel; A_H: only cells sharing a face couple, and their lower-left vertices are
+    # lattice neighbours); the rows of A_H that no cell reaches get the mean diagonal
+    Ap = from_stencil(to_stencil(P.T @ A @ P, n, n), n, n)
+    Ah = from_stencil(hourglass_fill(to_stencil(H.T @ A @ H, n, n), n, n), n, n)
+    # the prototype coarsens down to 3 x 3 vertices (the device stops at 400)
+    lvp, lvh = hierarchy(Ap, n, n, max_coarse=9), hierarchy(Ah, n, n, max_coarse=9)
     D = sp.block_diag([sp.csr_matrix(np.linalg.inv(A[9 * c:9 * c + 9, 9 * c:9 * c + 9].toarray())) for c in range(m.nc)],
                       format="csr")
 
     def prec(r):
-        z = D @ r + P @ _vcycle(lvp, 0, P.T @ r)
+        z = D @ r + P @ vcycle(lvp, P.T @ r)
         if variant == "hourglass":
-            z = z + H @ _vcycle(lvh, 0, H.T @ r)
+            z = z + H @ vcycle(lvh, H.T @ r)
         return z
 
     it = [0]
