@@ -155,6 +155,9 @@ struct AffineFn {
 };
 
 struct MgState;  // multigrid.cu
+// the multigrid preconditioners of multigrid.cu: "cg.mg" (Q1 on cubes, P1 on lattice simplices), "cg.mg2" (Q2 on cubes),
+// "cg.mg2.simplex" (P2 on lattice simplices)
+enum class MgKind { mg, mg2, mg2_simplex };
 
 struct RhsTerm {  // one local functional added into a rhs vector
   int kind;       // 0 L2Volume(f), 1 DirichletBoundarySWIPDG(factor f, g), 2 L2Face(f) on the Neumann faces
@@ -228,7 +231,8 @@ struct hdd_swipdg {
   bool p2p_ready = false, p2p_failed = false;
   hdd::PeerView peer_view{};
   std::vector<void*> ipc_opened;
-  int last_precond = 1;  // 0 identity, 1 diagonal, 2 cell-block diagonal, 3 two-level multigrid (cg.mg), 4 cg.mg2
+  int last_precond = 1;  // 0 identity, 1 diagonal, 2 cell-block diagonal, 3 two-level multigrid (cg.mg), 4 cg.mg2,
+                         // 5 cg.mg2.simplex
   hdd::MgState* mg = nullptr;
   // CUDA graph of two CG iterations, cached per solver type; valid while the operator / workspace pointers it was
   // captured with are the ones in use (cg_graph_key)
@@ -237,7 +241,7 @@ struct hdd_swipdg {
     const void* key[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     int64_t launches = 0;
   };
-  CgGraph cg_graph[5];
+  CgGraph cg_graph[6];
   hdd::DevBuf<hdd::CgScalars> sc;
   hdd::CgScalars* sc_host = nullptr;  // pinned
   bool have_solution = false;
@@ -266,7 +270,7 @@ void assemble_products(hdd_swipdg* h);
 // multigrid.cu ("cg.mg", "cg.mg2")
 void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_dev, int64_t v_begin, int64_t v_end,
                          const int32_t* cv_dev, int64_t n_verts);
-void mg_setup(hdd_swipdg* h, const double* frozen_values, bool q2);
+void mg_setup(hdd_swipdg* h, const double* frozen_values, MgKind kind);
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc);
 void mg_release(MgState* st);
 // copies the finest level's V-cycle results of the last mg_apply, n_hier (nx+1)(ny+1) doubles, on the handle's stream

@@ -31,7 +31,15 @@
 //
 // with P the bilinear interpolation of the conforming Q1 space into Q2-DG and H the hourglass family of the Q2 volume
 // term (see k_vertex_galerkin_q2).  A_P and A_H are two independent 9-point vertex operators: the two hierarchies of
-// MgState (MgState::q2), each with a level-0 operator of its own.  On N GPUs the vertex levels always run replicated.
+// MgState (MgKind::mg2), each with a level-0 operator of its own.  On N GPUs the vertex levels always run replicated.
+//
+// "cg.mg2.simplex": polOrder 2 on lattice-structured triangle grids,
+//
+//   M^-1 r = D_6^-1 r  +  P V(P^T r)
+//
+// with P the interpolation of the conforming P1 space on the vertex lattice into P2-DG (see k_vertex_galerkin_p2).  The P2
+// volume rule is exact, so there is no hourglass family: one hierarchy, the vertex levels of the P1 lattice path of
+// "cg.mg", and only the DG level is new.  On N GPUs the vertex levels run replicated, as for "cg.mg2".
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -743,6 +751,118 @@ __global__ void __launch_bounds__(kMgThreads)
   grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
 }
 
+// ---- DG level for polOrder 2 on lattice-structured simplex grids ("cg.mg2.simplex"): P = interpolation of the conforming
+// P1 space into P2-DG, one hierarchy (the P2 volume rule is exact: no hourglass family).  P2 nodes in the DoF order of
+// Elem<SIMPLEX, 2>: (0,0), (1/2,0), (1,0), (0,1/2), (1/2,1/2), (0,1) - corner i of the cell is node p2_corner(i), the edge
+// midpoints next to it are p2_mid1(i) and p2_mid2(i), each with weight 1/2 for either of its two corners.
+__device__ __forceinline__ int p2_corner(int i) { return i == 0 ? 0 : i == 1 ? 2 : 5; }
+__device__ __forceinline__ int p2_mid1(int i) { return i == 2 ? 3 : 1; }
+__device__ __forceinline__ int p2_mid2(int i) { return i == 0 ? 3 : 4; }
+
+// A_c = P^T A P per local vertex v: for every owned (cell, corner) at v the three rows of the nodes v interpolates into
+// (its corner node with weight 1, the two adjacent edge midpoints with weight 1/2); each 6-wide block of such a row is
+// folded onto the three vertices of the block's cell.  Entries at lattice distance 2 cancel analytically (jumps of
+// continuous functions) and are dropped.  Writes only the rows of vertices with an owned triangle: the rows of cells owned
+// elsewhere are added by the all-reduce.
+__global__ void __launch_bounds__(kMgThreads)
+    k_vertex_galerkin_p2(MeshView m, const double* __restrict__ vals, const int64_t* __restrict__ vptr,
+                         const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid,
+                         const int32_t* __restrict__ cell_gv, int32_t n_verts_loc, int nx, int ny, double* __restrict__ S) {
+  const int lv = blockIdx.x * blockDim.x + threadIdx.x;
+  if (lv >= n_verts_loc) return;
+  const int nx1 = nx + 1;
+  const int64_t nv = int64_t(nx1) * (ny + 1);
+  const int v = __ldg(lvert_gid + lv);
+  const int ix = v % nx1, iy = v / nx1;
+  double acc[9];
+#pragma unroll
+  for (int e = 0; e < 9; ++e) acc[e] = 0.0;
+  bool any = false;
+  for (int64_t q = __ldg(vptr + lv); q < __ldg(vptr + lv + 1); ++q) {
+    const int dof = __ldg(vdof + q);
+    const int c = dof / 3, i = dof - 3 * c, k = c - m.own0;
+    if (k < 0 || k >= m.n_own) continue;
+    any = true;
+    int nb[3];
+    nb[0] = __ldg(m.neigh + size_t(3) * k);
+    nb[1] = __ldg(m.neigh + size_t(3) * k + 1);
+    nb[2] = __ldg(m.neigh + size_t(3) * k + 2);
+    const int nblk = block_count<3>(nb);
+    const double* blk = vals + __ldg(m.blk_start + k) * 36;
+    const int rows[3] = {p2_corner(i), p2_mid1(i), p2_mid2(i)};
+    const double wr[3] = {1.0, 0.5, 0.5};
+#pragma unroll 1
+    for (int t = 0; t < 4; ++t) {
+      const int cell = t == 0 ? c : nb[t - 1];
+      if (cell < 0) continue;
+      const int slot = block_slot<3>(c, nb, cell);
+      double f[3] = {0.0, 0.0, 0.0};  // the weighted rows folded onto vertex j of `cell`
+#pragma unroll
+      for (int rr = 0; rr < 3; ++rr) {
+        const double* row = blk + int64_t(rows[rr]) * nblk * 6 + slot * 6;
+        double a[6];
+#pragma unroll
+        for (int n = 0; n < 6; ++n) a[n] = __ldg(row + n);
+        f[0] = fma(wr[rr], a[0] + 0.5 * (a[1] + a[3]), f[0]);
+        f[1] = fma(wr[rr], a[2] + 0.5 * (a[1] + a[4]), f[1]);
+        f[2] = fma(wr[rr], a[5] + 0.5 * (a[3] + a[4]), f[2]);
+      }
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+        const int w = __ldg(cell_gv + size_t(3) * cell + j);
+        const int dx = w % nx1 - ix, dy = w / nx1 - iy;
+        if (dx < -1 || dx > 1 || dy < -1 || dy > 1) continue;  // cancels analytically
+        acc[(dy + 1) * 3 + dx + 1] += f[j];
+      }
+    }
+  }
+  if (!any) return;  // no owned cell at this vertex: its row comes from the owners
+#pragma unroll
+  for (int e = 0; e < 9; ++e) S[e * nv + v] = acc[e];
+}
+
+// b0 = P^T r: per local vertex, over the owned (cell, corner) pairs at it, r[corner node] + (r[mid 1] + r[mid 2]) / 2
+__global__ void __launch_bounds__(kMgThreads)
+    k_dg_restrict_p2(const int* done, const double* __restrict__ r, const int64_t* __restrict__ vptr,
+                     const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid, int32_t n_verts_loc, int own0,
+                     int n_own, double* __restrict__ b0) {
+  if (done && *done) return;
+  const int lv = blockIdx.x * blockDim.x + threadIdx.x;
+  if (lv >= n_verts_loc) return;
+  double s = 0.0;
+  for (int64_t q = __ldg(vptr + lv); q < __ldg(vptr + lv + 1); ++q) {
+    const int dof = __ldg(vdof + q);
+    const int c = dof / 3, i = dof - 3 * c, k = c - own0;
+    if (k < 0 || k >= n_own) continue;
+    const double* rc = r + size_t(6) * k;
+    s += __ldg(rc + p2_corner(i)) + 0.5 * (__ldg(rc + p2_mid1(i)) + __ldg(rc + p2_mid2(i)));
+  }
+  b0[__ldg(lvert_gid + lv)] = s;
+}
+
+// z += P x, r.z recomputed; optionally p = z (first direction).  One thread per owned triangle, grid-stride.
+__global__ void __launch_bounds__(kMgThreads)
+    k_dg_prolong_dot_p2(const int* done, int32_t n_cells, const int32_t* __restrict__ cell_gv /* of the owned cells */,
+                        const double* __restrict__ x0, const double* __restrict__ r, double* __restrict__ z,
+                        double* __restrict__ p_init, double* partial, CgScalars* sc) {
+  if (done && *done) return;
+  double v[1] = {0.0};
+  const int64_t stride = int64_t(gridDim.x) * blockDim.x;
+  for (int64_t c = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; c < n_cells; c += stride) {
+    const double x[3] = {__ldg(x0 + __ldg(cell_gv + 3 * c)), __ldg(x0 + __ldg(cell_gv + 3 * c + 1)),
+                         __ldg(x0 + __ldg(cell_gv + 3 * c + 2))};
+    const double px[6] = {x[0], 0.5 * (x[0] + x[1]), x[1], 0.5 * (x[0] + x[2]), 0.5 * (x[1] + x[2]), x[2]};
+#pragma unroll
+    for (int n = 0; n < 6; ++n) {
+      const double o = z[6 * c + n] + px[n];
+      z[6 * c + n] = o;
+      if (p_init) p_init[6 * c + n] = o;
+      v[0] = fma(r[6 * c + n], o, v[0]);
+    }
+  }
+  grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
+}
+
 // lattice rows touched by the owned triangles: min / max of (vertex id / nx1) over their vertices
 __global__ void k_vertex_row_range(const int32_t* __restrict__ gv_owned, int64_t n_entries, int nx1, int* __restrict__ minmax) {
   const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -1001,9 +1121,15 @@ struct MgState {
   int n_hier = 2;  // Q1 on cubes: plain + checkerboard-twisted hierarchy; P1 on lattice-structured simplex grids: one
   // Q2 on cubes ("cg.mg2"): hierarchy 0 for A_P, hierarchy 1 for A_H, each with a level-0 operator of its own (the
   // twisted Q1 hierarchy instead reads its level-0 operator from the plain one's arrays)
-  bool q2 = false;
+  // P2 on lattice-structured simplex grids ("cg.mg2.simplex"): one hierarchy, as for P1
+  MgKind kind = MgKind::mg;
+  bool q2() const { return kind == MgKind::mg2; }
   MgDist dist;
 };
+
+static const char* mg_type_name(MgKind k) {
+  return k == MgKind::mg2 ? "cg.mg2" : k == MgKind::mg2_simplex ? "cg.mg2.simplex" : "cg.mg";
+}
 
 static inline dim3 grid2(int64_t cnt, int n_hier = 2) { return dim3(unsigned(blocks_for(cnt)), unsigned(n_hier)); }
 
@@ -1142,7 +1268,7 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
       HDD_CUDA(cudaMemsetAsync(c.S.p, 0, size_t(nh) * 9 * c.nv * sizeof(double), s));
       rc = row_range(c, d.own_lo, d.own_hi);
     }
-    const bool shared = l == 0 && !st.q2;  // level 0 of the twisted hierarchy is read from the plain one's arrays
+    const bool shared = l == 0 && !st.q2();  // level 0 of the twisted hierarchy is read from the plain one's arrays
     k_rap<<<grid2(rc.cnt, nh), kMgThreads, 0, s>>>(f.S.p, shared ? 0 : 9 * f.nv, f.nx, f.ny, (shared && nh == 2) ? 1 : 0, rc, c.S.p,
                                                   9 * c.nv);
     count_launch();
@@ -1151,17 +1277,17 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
   for (size_t l = 0; l < nl; ++l) {
     MgLevel& L = *st.levels[l];
     const Rows r = int(l) < nd ? row_range(L, d.b_lo[l], d.b_hi[l]) : Rows{0, L.nv};
-    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), (l == 0 && !st.q2) ? 1u : unsigned(st.n_hier)), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
+    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), (l == 0 && !st.q2()) ? 1u : unsigned(st.n_hier)), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
     count_launch();
   }
   // dense inverses of the coarsest operators (s.p.d.): Gauss-Jordan on the device, one CTA per hierarchy
   MgLevel& C = *st.levels.back();
-  const char* type = st.q2 ? "cg.mg2" : "cg.mg";
+  const char* type = mg_type_name(st.kind);
   if (C.nv > kMaxCoarse)
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, type << ": the " << st.nx << " x " << st.ny << " grid cannot be coarsened by halving down to at most "
                                                            << kMaxCoarse << " vertices (stuck at " << C.nx << " x " << C.ny << ")");
   const int n = int(C.nv);
-  const bool shared = nl == 1 && !st.q2;  // coarsest = finest level, whose operator the twisted hierarchy shares
+  const bool shared = nl == 1 && !st.q2();  // coarsest = finest level, whose operator the twisted hierarchy shares
   const size_t need = size_t(st.n_hier) * n * n;
   if (st.coarse_inv.n < need) st.coarse_inv.alloc(need);
   if (st.coarse_work.n < need) st.coarse_work.alloc(need);
@@ -1204,7 +1330,7 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
     MgLevel& L = *st.levels[size_t(l)];
     MgLevel& Cn = *st.levels[size_t(l) + 1];
     const Rows rp = l < nd ? row_range(L, d.pre_lo[l], d.pre_hi[l]) : Rows{0, L.nv};
-    if (l == 0 && nh == 2 && !st.q2)
+    if (l == 0 && nh == 2 && !st.q2())
       k_mg_pre2<<<blocks_for(rp.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
     else
       k_mg_pre<<<grid2(rp.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
@@ -1241,7 +1367,7 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
     } else {
       const Rows rq = l < nd ? row_range(L, d.pro_lo[l], d.pro_hi[l]) : Rows{0, L.nv};
       k_mg_prolong_add<<<grid2(rq.cnt, nh), kMgThreads, 0, s>>>(done, Cn.result, L.nx, L.ny, rq, L.x.p);
-      if (l == 0 && nh == 2 && !st.q2)
+      if (l == 0 && nh == 2 && !st.q2())
         k_mg_post2<<<blocks_for(ru.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
       else
         k_mg_post<<<grid2(ru.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
@@ -1336,28 +1462,42 @@ static void detect_strips(hdd_swipdg* h, MgState& st) {
 
 void mg_release(MgState* st) { delete st; }
 
-// (re)builds both hierarchies for the frozen operator `vals`; q2: "cg.mg2", otherwise "cg.mg"
-void mg_setup(hdd_swipdg* h, const double* vals, bool q2) {
+// (re)builds the hierarchies for the frozen operator `vals`
+void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
   hdd_mesh* m = h->mesh;
   const bool cube = m->kind == HDD_CUBE2D && m->sx > 0, lattice = m->kind == HDD_SIMPLEX2D && m->lx > 0;
+  const bool q2 = kind == MgKind::mg2, p2s = kind == MgKind::mg2_simplex;
+  const bool p2_lattice = lattice && h->polorder == 2;  // what "cg.mg2.simplex" is for
   if (q2 && h->polorder == 1)
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "solver type 'cg.mg2' is the multigrid preconditioner for polOrder 2; use 'cg.mg' for polOrder 1");
   if (q2 && !cube)
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
               "solver type 'cg.mg2' needs Q2 on a logically structured HDD_CUBE2D grid with the vertices numbered x-fastest "
-              "(Stuff::Grid::Providers::Cube / hdd_grid_cube); use 'cg.blockdiagonal'");
-  if (!q2 && ((!cube && !lattice) || h->polorder != 1))
+              "(Stuff::Grid::Providers::Cube / hdd_grid_cube); use 'cg.blockdiagonal'"
+                  << (p2_lattice ? " or 'cg.mg2.simplex'" : ""));
+  if (p2s && m->kind != HDD_SIMPLEX2D)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' needs a simplex grid; on HDD_CUBE2D grids use 'cg.mg' (polOrder 1) or 'cg.mg2' (polOrder 2)");
+  if (p2s && h->polorder == 1)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' is the multigrid preconditioner for polOrder 2 on triangles; use 'cg.mg' for polOrder 1");
+  if (p2s && !lattice)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' needs a simplex grid whose vertices form a lattice numbered x-fastest and whose "
+              "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.blockdiagonal'");
+  if (kind == MgKind::mg && ((!cube && !lattice) || h->polorder != 1))
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
               "solver type 'cg.mg' needs polOrder 1 on a logically structured grid: HDD_CUBE2D with the vertices numbered x-fastest "
               "(Stuff::Grid::Providers::Cube / hdd_grid_cube) or a simplex grid whose vertices form such a lattice and whose "
-              "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.diagonal' or 'cg.blockdiagonal'");
+              "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.diagonal' or 'cg.blockdiagonal'"
+                  << (p2_lattice ? " or 'cg.mg2.simplex'" : ""));
   cudaStream_t s = m->stream;
   if (!h->mg) h->mg = new MgState;
   MgState& st = *h->mg;
   st.nx = cube ? m->sx : m->lx;
   st.ny = cube ? m->sy : m->ly;
   st.n_hier = cube ? 2 : 1;
-  st.q2 = q2;
+  st.kind = kind;
   const int64_t nv = int64_t(st.nx + 1) * (st.ny + 1);
   if (!st.levels.empty() && (st.levels[0]->nx != st.nx || st.levels[0]->ny != st.ny)) {
     st.levels.clear();
@@ -1386,9 +1526,9 @@ void mg_setup(hdd_swipdg* h, const double* vals, bool q2) {
   }
   phase_timer().mark("setup mg: allocation", s);
   // the strip layout depends on the mesh and the communicator only: decided at the first solve of this discretization
-  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated).  "cg.mg2" always runs
-  // its vertex levels replicated.
-  if (!st.strips_known && !q2) {
+  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated).  "cg.mg2" and
+  // "cg.mg2.simplex" always run their vertex levels replicated.
+  if (!st.strips_known && kind == MgKind::mg) {
     detect_strips(h, st);
     st.strips_known = true;
   }
@@ -1437,6 +1577,12 @@ void mg_setup(hdd_swipdg* h, const double* vals, bool q2) {
     if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(18) * nv, m->comm, s);
     k_hourglass_fill<<<1, 1024, 0, s>>>(f0.S.p + 13 * nv, st.nx, st.ny);  // diagonal of hierarchy 1: array 9 + 4
     count_launch();
+  } else if (p2s) {
+    if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
+    k_vertex_galerkin_p2<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
+                                                                          m->cell_gv.p, m->n_verts_loc, st.nx, st.ny, f0.S.p);
+    count_launch();
+    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
   } else if (lattice) {
     if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
     k_vertex_galerkin_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
@@ -1455,8 +1601,8 @@ void mg_setup(hdd_swipdg* h, const double* vals, bool q2) {
   HDD_CUDA(cudaGetLastError());
 }
 
-// z += P V(P^T r) + P C V_C(C P^T r) ("cg.mg2": z += P V_P(P^T r) + H V_H(H^T r)), red[1] = r.z; p_init != nullptr also
-// stores z as the first direction
+// z += P V(P^T r) + P C V_C(C P^T r) ("cg.mg2": z += P V_P(P^T r) + H V_H(H^T r); P1 on lattice simplices and
+// "cg.mg2.simplex": z += P V(P^T r)), red[1] = r.z; p_init != nullptr also stores z as the first direction
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc) {
   hdd_mesh* m = h->mesh;
   MgState& st = *h->mg;
@@ -1495,7 +1641,14 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
     k_ghost_unpack_twist<<<blocks_for(int64_t(hi_row - lo_row + 1) * nx1), kMgThreads, 0, s>>>(
         done, b0, b1, d.lower >= 0 ? d.tmp_lo.p : nullptr, d.upper >= 0 ? d.tmp_up.p : nullptr, st.nx, d.c0, d.c1, g, lo_row, hi_row);
     count_launch();
-  } else if (st.q2) {
+  } else if (st.kind == MgKind::mg2_simplex) {
+    // P2 on a lattice-structured simplex grid: conforming P1 auxiliary space, one hierarchy, run replicated
+    if (multi) HDD_CUDA(cudaMemsetAsync(b0, 0, size_t(a.nv) * sizeof(double), s));
+    k_dg_restrict_p2<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->n_verts_loc,
+                                                                      m->own0, m->n_own, b0);
+    count_launch();
+    if (multi) Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
+  } else if (st.q2()) {
     // Q2: b0 = P^T r, b1 = H^T r; every rank writes every vertex (zeros where it owns no cell), one all-reduce of both
     k_dg_restrict_q2<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, b0, b1);
     count_launch();
@@ -1527,9 +1680,11 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
     vcycle(m, st, done, s);
   }
   const int grid = int(std::min<int64_t>((m->n_own + kMgThreads - 1) / kMgThreads, kMaxBlocks));
-  if (st.q2)
+  if (st.q2())
     k_dg_prolong_dot_q2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z,
                                                     p_init, partial, sc);
+  else if (st.kind == MgKind::mg2_simplex)
+    k_dg_prolong_dot_p2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
   else if (st.n_hier == 1)
     k_dg_prolong_dot_p1<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
   else
@@ -1554,11 +1709,11 @@ extern "C" int hdd_mg_level_operator(const hdd_swipdg* h, int level, int hier, i
   return hdd::guarded([&] {
     if (!h) HDD_THROW(HDD_ERR_WRONG_INPUT, "discretization handle is NULL");
     const hdd::MgState* st = h->mg;
-    if (!st) HDD_THROW(HDD_ERR_USING_THIS_WRONG, "no multigrid hierarchy: solve with 'cg.mg' or 'cg.mg2' first");
+    if (!st) HDD_THROW(HDD_ERR_USING_THIS_WRONG, "no multigrid hierarchy: solve with 'cg.mg', 'cg.mg2' or 'cg.mg2.simplex' first");
     if (level < 0 || level >= int(st->levels.size()))
       HDD_THROW(HDD_ERR_WRONG_INPUT, "level " << level << " of " << st->levels.size());
     if (hier < 0 || hier >= st->n_hier) HDD_THROW(HDD_ERR_WRONG_INPUT, "hierarchy " << hier << " of " << st->n_hier);
-    if (level == 0 && hier == 1 && !st->q2)
+    if (level == 0 && hier == 1 && !st->q2())
       HDD_THROW(HDD_ERR_WRONG_INPUT, "level 0 of the twisted hierarchy is C A_c C, read from the plain one's arrays");
     const hdd::MgLevel& L = *st->levels[size_t(level)];
     if (nx) *nx = L.nx;

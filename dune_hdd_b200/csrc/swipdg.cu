@@ -371,6 +371,7 @@ int parse_solver_type(const char* type) {
   if (t == "cg.blockdiagonal" || t == "cg.blockjacobi") return 2;
   if (t == "cg.mg" || t == "cg.multigrid") return 3;
   if (t == "cg.mg2" || t == "cg.multigrid2") return 4;
+  if (t == "cg.mg2.simplex" || t == "cg.multigrid2.simplex") return 5;
   HDD_THROW(HDD_ERR_WRONG_INPUT, "solver type '" << t << "' is not one of solver_types()");
 }
 
@@ -495,7 +496,7 @@ double total(const std::vector<double>& v) {
 const char* const kEstimatorTypes[] = {"eta_NC_ESV2007", "eta_R_ESV2007",  "eta_R_ESV2007_*", "eta_DF_ESV2007", "eta_ESV2007",
                                        "eta_ESV2007_alt", "eta_NC_OS2014", "eta_R_OS2014",    "eta_R_OS2014_*", "eta_DF_OS2014",
                                        "eta_DF_OS2014_*", "eta_OS2014",    "eta_OS2014_*"};
-const char* const kSolverTypes[] = {"cg.diagonal", "cg.blockdiagonal", "cg.identity", "cg.mg", "cg.mg2"};
+const char* const kSolverTypes[] = {"cg.diagonal", "cg.blockdiagonal", "cg.identity", "cg.mg", "cg.mg2", "cg.mg2.simplex"};
 
 }  // namespace
 
@@ -879,7 +880,7 @@ CgStart start_cg(hdd_swipdg* h, int use_diag, const double* mu, int mu_size, boo
     launch_invert_diag_blocks(v, vals, h->dinv_block.p, s);
     pt.mark("setup: block inverses", s);
     c.dinv_block = h->dinv_block.p;
-    if (use_diag >= 3) mg_setup(h, vals, use_diag == 4);
+    if (use_diag >= 3) mg_setup(h, vals, use_diag == 5 ? MgKind::mg2_simplex : use_diag == 4 ? MgKind::mg2 : MgKind::mg);
   } else {
     c.z = nullptr;
     launch_extract_dinv(v, vals, use_diag, h->dinv.p, s);
@@ -958,7 +959,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     const MeshView v = h->view();
     Nccl& nc = Nccl::get();
     const bool multi = m->world > 1;
-    // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg / cg.mg2).  The first batch is
+    // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg / cg.mg2 / cg.mg2.simplex).  The first batch is
     // launched directly (one-time attribute / buffer set-up happens there); after that two iterations (parity 0 and 1)
     // are captured into a CUDA graph and replayed, so a launch-bound iteration costs one graph launch instead of up to
     // a hundred kernel launches and does not stall the GPU when the host thread is delayed.  HDD_CG_GRAPH=0 disables it.

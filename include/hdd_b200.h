@@ -215,8 +215,10 @@ typedef struct hdd_solve_info {
  * structured grids: HDD_CUBE2D with the vertices numbered x-fastest, or a simplex grid whose vertices form such a
  * lattice and whose triangles join lattice neighbours; and "cg.mg2": the same for polOrder 2 (block Jacobi with the
  * 9 x 9 cell blocks + conforming Q1 + the Q2 hourglass family, one V-cycle each) - Q2 on logically structured
- * HDD_CUBE2D grids only.  Elsewhere both give HDD_ERR_REQUIREMENTS_NOT_MET.  Aliases "cg", "cg.jacobi",
- * "cg.diagonal.lower", "cg.identity.lower", "cg.blockjacobi", "cg.multigrid", "cg.multigrid2". */
+ * HDD_CUBE2D grids only; and "cg.mg2.simplex": polOrder 2 on the lattice-structured simplex grids of "cg.mg" (block
+ * Jacobi with the 6 x 6 cell blocks + the conforming P1 space on the vertex lattice, one V-cycle).  Elsewhere each gives
+ * HDD_ERR_REQUIREMENTS_NOT_MET.  Aliases "cg", "cg.jacobi", "cg.diagonal.lower", "cg.identity.lower",
+ * "cg.blockjacobi", "cg.multigrid", "cg.multigrid2", "cg.multigrid2.simplex". */
 int hdd_solver_types(const char* const** types, int* n_types);
 /* uncached_solve(options, vector, mu) (discretizations/base.hh:327-367): freeze lhs and rhs at mu, CG.
  * precision / max_iter mirror Stuff::LA::Solver's option keys.  x_host[n_owned] receives the solution

@@ -1,7 +1,7 @@
 /*
  * hdd_b200_testing.h - entry points of libhdd_b200 that exist for tests: host arithmetic the CPU tests check without a
  * device, and views into the solvers' intermediate results that the GPU tests compare with a plain float64 restatement
- * (tests/mg_reference.py).  A drop-in host of the reference needs none of them; conventions as in hdd_b200.h.
+ * (tests/mg_reference.py, tests/mg_reference_p2.py).  A drop-in host of the reference needs none of them; conventions as in hdd_b200.h.
  */
 #ifndef HDD_B200_TESTING_H
 #define HDD_B200_TESTING_H
@@ -30,14 +30,15 @@ int hdd_trig_product(const char* expression, double* out, int* valid);
 /* z = M^-1 r: one application of the preconditioner of solver type `type` (names and aliases as hdd_solve) for the
  * operator frozen at mu, through hdd_solve's own set-up and CG initialisation (z is the first search direction of a
  * solve whose right-hand side is r).  r_host, z_host: n_owned.  rz (nullable): r.z as the solver's fused reduction
- * computed it.  vertex_host (nullable; cg.mg / cg.mg2 only): the V-cycle results on the finest vertex level,
- * n_hier (nx+1)(ny+1) doubles - cg.mg on cubes: V(P^T r), V_C(C P^T r); on lattice simplices: V(P^T r);
- * cg.mg2: V_P(P^T r), V_H(H^T r).  Leaves the solution, the rhs and hdd_solve's cached CUDA graphs untouched.
+ * computed it.  vertex_host (nullable; cg.mg / cg.mg2 / cg.mg2.simplex only): the V-cycle results on the finest
+ * vertex level, n_hier (nx+1)(ny+1) doubles - cg.mg on cubes: V(P^T r), V_C(C P^T r); on lattice simplices: V(P^T r);
+ * cg.mg2: V_P(P^T r), V_H(H^T r); cg.mg2.simplex: V(P^T r), one hierarchy.  Leaves the solution, the rhs and hdd_solve's cached CUDA graphs untouched.
  * One GPU only; HDD_ERR_NOT_IMPLEMENTED on N GPUs and for purely Neumann problems. */
 int hdd_precondition(hdd_swipdg* h, const char* type, const double* mu, int mu_size, const double* r_host,
                      double* z_host, double* rz, double* vertex_host);
 
-/* The 9-point operator of multigrid level `level`, hierarchy `hier`, as the last cg.mg / cg.mg2 set-up left it:
+/* The 9-point operator of multigrid level `level`, hierarchy `hier`, as the last cg.mg / cg.mg2 / cg.mg2.simplex set-up
+ * left it (cg.mg2.simplex has hierarchy 0 only):
  * nx, ny of the level's vertex grid; S_host (nullable) 9 (nx+1)(ny+1) doubles, S[e nv + v] = coupling of
  * v = (ix, iy) to (ix+dx, iy+dy), e = 3 (dy+1) + dx + 1.  HDD_ERR_WRONG_INPUT past the coarsest level, for a
  * hierarchy that does not exist, and for level 0 of cg.mg's twisted hierarchy (C A_c C is not stored). */
