@@ -155,9 +155,14 @@ struct AffineFn {
 };
 
 struct MgState;  // multigrid.cu
-// the multigrid preconditioners of multigrid.cu: "cg.mg" (Q1 on cubes, P1 on lattice simplices), "cg.mg2" (Q2 on cubes),
+// the preconditioners of the CG solver; the numeric order indexes hdd_swipdg::cg_graph.  mg, mg2 and mg2_simplex are the
+// multigrid preconditioners of multigrid.cu: "cg.mg" (Q1 on cubes, P1 on lattice simplices), "cg.mg2" (Q2 on cubes),
 // "cg.mg2.simplex" (P2 on lattice simplices)
-enum class MgKind { mg, mg2, mg2_simplex };
+enum class SolverType { identity, diagonal, blockdiagonal, mg, mg2, mg2_simplex };
+constexpr int kNumSolverTypes = int(SolverType::mg2_simplex) + 1;
+// block Jacobi and the multigrid types (whose DG-level smoother it is) use the inverses of the cell blocks
+inline bool uses_block_inverses(SolverType t) { return t >= SolverType::blockdiagonal; }
+inline bool is_multigrid(SolverType t) { return t >= SolverType::mg; }
 
 struct RhsTerm {  // one local functional added into a rhs vector
   int kind;       // 0 L2Volume(f), 1 DirichletBoundarySWIPDG(factor f, g), 2 L2Face(f) on the Neumann faces
@@ -231,8 +236,7 @@ struct hdd_swipdg {
   bool p2p_ready = false, p2p_failed = false;
   hdd::PeerView peer_view{};
   std::vector<void*> ipc_opened;
-  int last_precond = 1;  // 0 identity, 1 diagonal, 2 cell-block diagonal, 3 two-level multigrid (cg.mg), 4 cg.mg2,
-                         // 5 cg.mg2.simplex
+  hdd::SolverType last_type = hdd::SolverType::diagonal;  // of the last hdd_solve
   hdd::MgState* mg = nullptr;
   // CUDA graph of two CG iterations, cached per solver type; valid while the operator / workspace pointers it was
   // captured with are the ones in use (cg_graph_key)
@@ -241,7 +245,7 @@ struct hdd_swipdg {
     const void* key[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
     int64_t launches = 0;
   };
-  CgGraph cg_graph[6];
+  CgGraph cg_graph[hdd::kNumSolverTypes];
   hdd::DevBuf<hdd::CgScalars> sc;
   hdd::CgScalars* sc_host = nullptr;  // pinned
   bool have_solution = false;
@@ -267,10 +271,10 @@ void require_init(const hdd_swipdg* h);                                         
 void check_mu(const hdd_swipdg* h, const double* mu, int mu_size, const char* name);  // base.hh:333-334
 double eval_coef(const Program& p, const double* mu, int mu_size);
 void assemble_products(hdd_swipdg* h);
-// multigrid.cu ("cg.mg", "cg.mg2")
+// multigrid.cu ("cg.mg", "cg.mg2", "cg.mg2.simplex")
 void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_dev, int64_t v_begin, int64_t v_end,
                          const int32_t* cv_dev, int64_t n_verts);
-void mg_setup(hdd_swipdg* h, const double* frozen_values, MgKind kind);
+void mg_setup(hdd_swipdg* h, const double* frozen_values, SolverType type);
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc);
 void mg_release(MgState* st);
 // copies the finest level's V-cycle results of the last mg_apply, n_hier (nx+1)(ny+1) doubles, on the handle's stream

@@ -83,7 +83,7 @@ struct FreezeArgs {
 };
 void launch_freeze(const FreezeArgs& a, double* out, int64_t count, cudaStream_t s);
 // dinv[row] = 1 / A[row,row] (Jacobi) or 1 (identity)
-void launch_extract_dinv(const MeshView& m, const double* values, int use_diagonal, double* dinv, cudaStream_t s);
+void launch_extract_dinv(const MeshView& m, const double* values, int jacobi, double* dinv, cudaStream_t s);
 void launch_invert_diag_blocks(const MeshView& m, const double* values, double* dinv_block, cudaStream_t s);
 
 // ---- K5/K6: CG ---------------------------------------------------------------------------------------------------

@@ -1587,11 +1587,11 @@ __global__ void __launch_bounds__(256) k_freeze(FreezeArgs a, double* __restrict
 }
 
 template <int NF, int NL>
-__global__ void k_extract_dinv(MeshView m, const double* __restrict__ values, int use_diagonal,
+__global__ void k_extract_dinv(MeshView m, const double* __restrict__ values, int jacobi,
                                double* __restrict__ dinv) {
   const int64_t t = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (t >= int64_t(m.n_own) * NL) return;
-  if (!use_diagonal) { dinv[t] = 1.0; return; }
+  if (!jacobi) { dinv[t] = 1.0; return; }
   const int k = int(t / NL), i = int(t % NL);
   int nb[NF];
   load_neigh<NF>(m.neigh, k, nb);
@@ -1924,11 +1924,11 @@ void launch_freeze(const FreezeArgs& a, double* out, int64_t count, cudaStream_t
   HDD_CUDA(cudaGetLastError());
 }
 
-void launch_extract_dinv(const MeshView& m, const double* values, int use_diagonal, double* dinv, cudaStream_t s) {
+void launch_extract_dinv(const MeshView& m, const double* values, int jacobi, double* dinv, cudaStream_t s) {
   if (m.n_own == 0) return;
   const int64_t rows = int64_t(m.n_own) * m.nl;
   dispatch_block(m, [&](auto nf, auto nl) {
-    k_extract_dinv<decltype(nf)::value, decltype(nl)::value><<<grid_for(rows, 256), 256, 0, s>>>(m, values, use_diagonal, dinv);
+    k_extract_dinv<decltype(nf)::value, decltype(nl)::value><<<grid_for(rows, 256), 256, 0, s>>>(m, values, jacobi, dinv);
   });
   count_launch();
   HDD_CUDA(cudaGetLastError());

@@ -31,15 +31,18 @@
 //
 // with P the bilinear interpolation of the conforming Q1 space into Q2-DG and H the hourglass family of the Q2 volume
 // term (see k_vertex_galerkin_q2).  A_P and A_H are two independent 9-point vertex operators: the two hierarchies of
-// MgState (MgKind::mg2), each with a level-0 operator of its own.  On N GPUs the vertex levels always run replicated.
+// MgState (MgSpace::q2_cube), each with a level-0 operator of its own.  On N GPUs the vertex levels always run replicated.
 //
-// "cg.mg2.simplex": polOrder 2 on lattice-structured triangle grids,
+// Lattice-structured triangle grids, "cg.mg" at polOrder 1 and "cg.mg2.simplex" at polOrder 2,
 //
-//   M^-1 r = D_6^-1 r  +  P V(P^T r)
+//   M^-1 r = D_blk^-1 r  +  P V(P^T r)
 //
-// with P the interpolation of the conforming P1 space on the vertex lattice into P2-DG (see k_vertex_galerkin_p2).  The P2
-// volume rule is exact, so there is no hourglass family: one hierarchy, the vertex levels of the P1 lattice path of
-// "cg.mg", and only the DG level is new.  On N GPUs the vertex levels run replicated, as for "cg.mg2".
+// with P the interpolation of the conforming P1 space on the vertex lattice into P1-DG or P2-DG (one kernel set for both,
+// see k_vertex_galerkin_lattice).  The P1 and P2 volume rules are exact, so there is no hourglass family: one hierarchy.
+// On N GPUs the vertex levels of P1 run in row strips like those of Q1; those of P2 run replicated, as for "cg.mg2".
+//
+// mg_space maps (solver type, grid, polOrder) to one of these four variants (MgSpace) once per set-up; everything below
+// follows from it.
 #include <algorithm>
 #include <climits>
 #include <cmath>
@@ -665,109 +668,69 @@ __global__ void __launch_bounds__(kMgThreads)
   else if (up && iy == c1) Se[v] += up[e * chunk + ix];
 }
 
-// ---- DG level on lattice-structured simplex grids: P = injection of the conforming P1 space (one hierarchy: the P1
-// volume term is integrated exactly, there is no hourglass family) --------------------------------------------------------
-// A_c = P^T A P per local vertex through the vertex -> DoF incidence of the Oswald pass; rows of cells owned elsewhere
-// are added by the all-reduce
-__global__ void __launch_bounds__(kMgThreads)
-    k_vertex_galerkin_p1(MeshView m, const double* __restrict__ vals, const int64_t* __restrict__ vptr,
-                         const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid,
-                         const int32_t* __restrict__ cell_gv, int32_t n_verts_loc, int nx, int ny, double* __restrict__ S) {
-  const int lv = blockIdx.x * blockDim.x + threadIdx.x;
-  if (lv >= n_verts_loc) return;
-  const int nx1 = nx + 1;
-  const int64_t nv = int64_t(nx1) * (ny + 1);
-  const int v = __ldg(lvert_gid + lv);
-  const int ix = v % nx1, iy = v / nx1;
-  double acc[9];
-#pragma unroll
-  for (int e = 0; e < 9; ++e) acc[e] = 0.0;
-  bool any = false;
-  for (int64_t q = __ldg(vptr + lv); q < __ldg(vptr + lv + 1); ++q) {
-    const int dof = __ldg(vdof + q);
-    const int c = dof / 3, i = dof - 3 * c, k = c - m.own0;
-    if (k < 0 || k >= m.n_own) continue;
-    any = true;
-    int nb[3];
-    nb[0] = __ldg(m.neigh + size_t(3) * k);
-    nb[1] = __ldg(m.neigh + size_t(3) * k + 1);
-    nb[2] = __ldg(m.neigh + size_t(3) * k + 2);
-    const int nblk = block_count<3>(nb);
-    const double* row = vals + __ldg(m.blk_start + k) * 9 + int64_t(i) * nblk * 3;
-#pragma unroll
-    for (int t = 0; t < 4; ++t) {
-      const int cell = t == 0 ? c : nb[t - 1];
-      if (cell < 0) continue;
-      const int slot = block_slot<3>(c, nb, cell);
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        const int w = __ldg(cell_gv + size_t(3) * cell + j);
-        const int dx = w % nx1 - ix, dy = w / nx1 - iy;
-        if (dx < -1 || dx > 1 || dy < -1 || dy > 1) continue;  // cancels analytically (jumps of continuous functions)
-        acc[(dy + 1) * 3 + dx + 1] += __ldg(row + slot * 3 + j);
-      }
-    }
-  }
-  if (!any) return;  // no owned cell at this vertex: its row comes from the owners
-#pragma unroll
-  for (int e = 0; e < 9; ++e) S[e * nv + v] = acc[e];
-}
-
-// b0 = P^T r: per local vertex the sum of the owned DG residual entries sitting on it
-__global__ void __launch_bounds__(kMgThreads)
-    k_dg_restrict_p1(const int* done, const double* __restrict__ r, const int64_t* __restrict__ vptr,
-                     const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid, int32_t n_verts_loc, int own0,
-                     int n_own, double* __restrict__ b0) {
-  if (done && *done) return;
-  const int lv = blockIdx.x * blockDim.x + threadIdx.x;
-  if (lv >= n_verts_loc) return;
-  double s = 0.0;
-  for (int64_t q = __ldg(vptr + lv); q < __ldg(vptr + lv + 1); ++q) {
-    const int dof = __ldg(vdof + q);
-    const int k = dof / 3 - own0;
-    if (k < 0 || k >= n_own) continue;
-    s += __ldg(r + size_t(dof) - size_t(3) * own0);
-  }
-  b0[__ldg(lvert_gid + lv)] = s;
-}
-
-// z += P x, r.z recomputed; optionally p = z (first direction).  One thread per owned triangle.
-__global__ void __launch_bounds__(kMgThreads)
-    k_dg_prolong_dot_p1(const int* done, int32_t n_cells, const int32_t* __restrict__ cell_gv /* of the owned cells */,
-                        const double* __restrict__ x0, const double* __restrict__ r, double* __restrict__ z,
-                        double* __restrict__ p_init, double* partial, CgScalars* sc) {
-  if (done && *done) return;
-  double v[1] = {0.0};
-  const int64_t stride = int64_t(gridDim.x) * blockDim.x;
-  for (int64_t c = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; c < n_cells; c += stride) {
-#pragma unroll
-    for (int i = 0; i < 3; ++i) {
-      const double o = z[3 * c + i] + __ldg(x0 + __ldg(cell_gv + 3 * c + i));
-      z[3 * c + i] = o;
-      if (p_init) p_init[3 * c + i] = o;
-      v[0] = fma(r[3 * c + i], o, v[0]);
-    }
-  }
-  grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
-}
-
-// ---- DG level for polOrder 2 on lattice-structured simplex grids ("cg.mg2.simplex"): P = interpolation of the conforming
-// P1 space into P2-DG, one hierarchy (the P2 volume rule is exact: no hourglass family).  P2 nodes in the DoF order of
-// Elem<SIMPLEX, 2>: (0,0), (1/2,0), (1,0), (0,1/2), (1/2,1/2), (0,1) - corner i of the cell is node p2_corner(i), the edge
-// midpoints next to it are p2_mid1(i) and p2_mid2(i), each with weight 1/2 for either of its two corners.
+// ---- DG level on lattice-structured simplex grids: P = interpolation of the conforming P1 space on the vertex lattice into
+// P_P-DG, P = 1 ("cg.mg") or 2 ("cg.mg2.simplex").  One hierarchy: the P1 and P2 volume rules are exact, there is no
+// hourglass family.  P1 nodes are the corners.  P2 nodes in the DoF order of Elem<SIMPLEX, 2>: (0,0), (1/2,0), (1,0),
+// (0,1/2), (1/2,1/2), (0,1) - corner i of the cell is node p2_corner(i), the edge midpoints next to it are p2_mid1(i) and
+// p2_mid2(i), each with weight 1/2 for either of its two corners.
 __device__ __forceinline__ int p2_corner(int i) { return i == 0 ? 0 : i == 1 ? 2 : 5; }
 __device__ __forceinline__ int p2_mid1(int i) { return i == 2 ? 3 : 1; }
 __device__ __forceinline__ int p2_mid2(int i) { return i == 0 ? 3 : 4; }
 
-// A_c = P^T A P per local vertex v: for every owned (cell, corner) at v the three rows of the nodes v interpolates into
-// (its corner node with weight 1, the two adjacent edge midpoints with weight 1/2); each 6-wide block of such a row is
-// folded onto the three vertices of the block's cell.  Entries at lattice distance 2 cancel analytically (jumps of
-// continuous functions) and are dropped.  Writes only the rows of vertices with an owned triangle: the rows of cells owned
-// elsewhere are added by the all-reduce.
+// The DG nodes corner i interpolates into: rr < corner_rows(P), node corner_node<P>(i, rr) with weight corner_weight(rr)
+// (the corner itself with weight 1; for P2 also the two adjacent edge midpoints with weight 1/2)
+constexpr int corner_rows(int P) { return P == 1 ? 1 : 3; }
+template <int P>
+__device__ __forceinline__ int corner_node(int i, int rr) {
+  return P == 1 ? i : rr == 0 ? p2_corner(i) : rr == 1 ? p2_mid1(i) : p2_mid2(i);
+}
+__device__ __forceinline__ double corner_weight(int rr) { return rr == 0 ? 1.0 : 0.5; }
+
+// f[j] += w (row block `row` of a cell, applied to the P interpolant of vertex j of that cell).  P1: the one row has
+// weight 1 and f starts at 0, so f is the row itself.
+template <int P>
+__device__ __forceinline__ void fold_row(const double* __restrict__ row, double w, double (&f)[3]) {
+  if constexpr (P == 1) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) f[j] = __ldg(row + j);
+  } else {
+    double a[6];
+#pragma unroll
+    for (int n = 0; n < 6; ++n) a[n] = __ldg(row + n);
+    f[0] = fma(w, a[0] + 0.5 * (a[1] + a[3]), f[0]);
+    f[1] = fma(w, a[2] + 0.5 * (a[1] + a[4]), f[1]);
+    f[2] = fma(w, a[5] + 0.5 * (a[3] + a[4]), f[2]);
+  }
+}
+
+// (P^T r) at corner i of a cell whose residual block is rc
+template <int P>
+__device__ __forceinline__ double corner_sum(const double* __restrict__ rc, int i) {
+  if constexpr (P == 1) return __ldg(rc + i);
+  else return __ldg(rc + p2_corner(i)) + 0.5 * (__ldg(rc + p2_mid1(i)) + __ldg(rc + p2_mid2(i)));
+}
+
+// (P x) at the nodes of a cell whose vertex values are x
+template <int P>
+__device__ __forceinline__ void node_values(const double (&x)[3], double (&px)[(P + 1) * (P + 2) / 2]) {
+  if constexpr (P == 1) {
+    px[0] = x[0]; px[1] = x[1]; px[2] = x[2];
+  } else {
+    px[0] = x[0]; px[1] = 0.5 * (x[0] + x[1]); px[2] = x[1]; px[3] = 0.5 * (x[0] + x[2]); px[4] = 0.5 * (x[1] + x[2]);
+    px[5] = x[2];
+  }
+}
+
+// A_c = P^T A P per local vertex v, through the vertex -> DoF incidence of the Oswald pass: for every owned (cell, corner)
+// at v the rows of the nodes v interpolates into; each block of such a row is folded onto the three vertices of the
+// block's cell.  Entries at lattice distance 2 cancel analytically (jumps of continuous functions) and are dropped.  Writes
+// only the rows of vertices with an owned triangle: the rows of cells owned elsewhere are added by the all-reduce.
+template <int P>
 __global__ void __launch_bounds__(kMgThreads)
-    k_vertex_galerkin_p2(MeshView m, const double* __restrict__ vals, const int64_t* __restrict__ vptr,
-                         const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid,
-                         const int32_t* __restrict__ cell_gv, int32_t n_verts_loc, int nx, int ny, double* __restrict__ S) {
+    k_vertex_galerkin_lattice(MeshView m, const double* __restrict__ vals, const int64_t* __restrict__ vptr,
+                              const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid,
+                              const int32_t* __restrict__ cell_gv, int32_t n_verts_loc, int nx, int ny, double* __restrict__ S) {
+  constexpr int NL = (P + 1) * (P + 2) / 2;
   const int lv = blockIdx.x * blockDim.x + threadIdx.x;
   if (lv >= n_verts_loc) return;
   const int nx1 = nx + 1;
@@ -788,25 +751,16 @@ __global__ void __launch_bounds__(kMgThreads)
     nb[1] = __ldg(m.neigh + size_t(3) * k + 1);
     nb[2] = __ldg(m.neigh + size_t(3) * k + 2);
     const int nblk = block_count<3>(nb);
-    const double* blk = vals + __ldg(m.blk_start + k) * 36;
-    const int rows[3] = {p2_corner(i), p2_mid1(i), p2_mid2(i)};
-    const double wr[3] = {1.0, 0.5, 0.5};
-#pragma unroll 1
+    const double* blk = vals + __ldg(m.blk_start + k) * (NL * NL);
+#pragma unroll(P == 1 ? 4 : 1)
     for (int t = 0; t < 4; ++t) {
       const int cell = t == 0 ? c : nb[t - 1];
       if (cell < 0) continue;
       const int slot = block_slot<3>(c, nb, cell);
       double f[3] = {0.0, 0.0, 0.0};  // the weighted rows folded onto vertex j of `cell`
 #pragma unroll
-      for (int rr = 0; rr < 3; ++rr) {
-        const double* row = blk + int64_t(rows[rr]) * nblk * 6 + slot * 6;
-        double a[6];
-#pragma unroll
-        for (int n = 0; n < 6; ++n) a[n] = __ldg(row + n);
-        f[0] = fma(wr[rr], a[0] + 0.5 * (a[1] + a[3]), f[0]);
-        f[1] = fma(wr[rr], a[2] + 0.5 * (a[1] + a[4]), f[1]);
-        f[2] = fma(wr[rr], a[5] + 0.5 * (a[3] + a[4]), f[2]);
-      }
+      for (int rr = 0; rr < corner_rows(P); ++rr)
+        fold_row<P>(blk + int64_t(corner_node<P>(i, rr)) * nblk * NL + slot * NL, corner_weight(rr), f);
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
         const int w = __ldg(cell_gv + size_t(3) * cell + j);
@@ -821,11 +775,13 @@ __global__ void __launch_bounds__(kMgThreads)
   for (int e = 0; e < 9; ++e) S[e * nv + v] = acc[e];
 }
 
-// b0 = P^T r: per local vertex, over the owned (cell, corner) pairs at it, r[corner node] + (r[mid 1] + r[mid 2]) / 2
+// b0 = P^T r: per local vertex, the sum over the owned (cell, corner) pairs at it
+template <int P>
 __global__ void __launch_bounds__(kMgThreads)
-    k_dg_restrict_p2(const int* done, const double* __restrict__ r, const int64_t* __restrict__ vptr,
-                     const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid, int32_t n_verts_loc, int own0,
-                     int n_own, double* __restrict__ b0) {
+    k_dg_restrict_lattice(const int* done, const double* __restrict__ r, const int64_t* __restrict__ vptr,
+                          const int32_t* __restrict__ vdof, const int32_t* __restrict__ lvert_gid, int32_t n_verts_loc,
+                          int own0, int n_own, double* __restrict__ b0) {
+  constexpr int NL = (P + 1) * (P + 2) / 2;
   if (done && *done) return;
   const int lv = blockIdx.x * blockDim.x + threadIdx.x;
   if (lv >= n_verts_loc) return;
@@ -834,30 +790,32 @@ __global__ void __launch_bounds__(kMgThreads)
     const int dof = __ldg(vdof + q);
     const int c = dof / 3, i = dof - 3 * c, k = c - own0;
     if (k < 0 || k >= n_own) continue;
-    const double* rc = r + size_t(6) * k;
-    s += __ldg(rc + p2_corner(i)) + 0.5 * (__ldg(rc + p2_mid1(i)) + __ldg(rc + p2_mid2(i)));
+    s += corner_sum<P>(r + size_t(NL) * k, i);
   }
   b0[__ldg(lvert_gid + lv)] = s;
 }
 
 // z += P x, r.z recomputed; optionally p = z (first direction).  One thread per owned triangle, grid-stride.
+template <int P>
 __global__ void __launch_bounds__(kMgThreads)
-    k_dg_prolong_dot_p2(const int* done, int32_t n_cells, const int32_t* __restrict__ cell_gv /* of the owned cells */,
-                        const double* __restrict__ x0, const double* __restrict__ r, double* __restrict__ z,
-                        double* __restrict__ p_init, double* partial, CgScalars* sc) {
+    k_dg_prolong_dot_lattice(const int* done, int32_t n_cells, const int32_t* __restrict__ cell_gv /* of the owned cells */,
+                             const double* __restrict__ x0, const double* __restrict__ r, double* __restrict__ z,
+                             double* __restrict__ p_init, double* partial, CgScalars* sc) {
+  constexpr int NL = (P + 1) * (P + 2) / 2;
   if (done && *done) return;
   double v[1] = {0.0};
   const int64_t stride = int64_t(gridDim.x) * blockDim.x;
   for (int64_t c = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; c < n_cells; c += stride) {
     const double x[3] = {__ldg(x0 + __ldg(cell_gv + 3 * c)), __ldg(x0 + __ldg(cell_gv + 3 * c + 1)),
                          __ldg(x0 + __ldg(cell_gv + 3 * c + 2))};
-    const double px[6] = {x[0], 0.5 * (x[0] + x[1]), x[1], 0.5 * (x[0] + x[2]), 0.5 * (x[1] + x[2]), x[2]};
+    double px[NL];
+    node_values<P>(x, px);
 #pragma unroll
-    for (int n = 0; n < 6; ++n) {
-      const double o = z[6 * c + n] + px[n];
-      z[6 * c + n] = o;
-      if (p_init) p_init[6 * c + n] = o;
-      v[0] = fma(r[6 * c + n], o, v[0]);
+    for (int n = 0; n < NL; ++n) {
+      const double o = z[NL * c + n] + px[n];
+      z[NL * c + n] = o;
+      if (p_init) p_init[NL * c + n] = o;
+      v[0] = fma(r[NL * c + n], o, v[0]);
     }
   }
   grid_sum<1>(v, partial, &sc->ticket_a, [sc](const double(&w)[1]) { sc->red[1] = w[0]; });
@@ -1102,8 +1060,7 @@ struct MgDist {
   int n_dist = 0;              // distributed levels 0 .. n_dist-1
   int lower = -1, upper = -1;  // ranks owning the strips below / above (-1: none)
   int c0 = 0, c1 = 0;          // owned cell rows [c0, c1) of level 0
-  bool last = false;           // the top strip
-  int ghost = 0;               // level-0 rows of b received from each neighbour
+  int ghost = 0;              // level-0 rows of b received from each neighbour
   // inclusive vertex-row ranges per distributed level: pre-smoothing (x, r), right-hand side b, post-smoothing (y),
   // prolongation (x += P x_H)
   int pre_lo[kMaxDist], pre_hi[kMaxDist], b_lo[kMaxDist], b_hi[kMaxDist], up_lo[kMaxDist], up_hi[kMaxDist],
@@ -1112,24 +1069,26 @@ struct MgDist {
   DevBuf<double> tmp_lo, tmp_up;
 };
 
+// the multigrid variants, chosen by mg_space: which DG space the conforming vertex space(s) interpolate into
+enum class MgSpace { q1_cube, p1_lattice, q2_cube, p2_lattice };
+
 struct MgState {
   std::vector<std::unique_ptr<MgLevel>> levels;
   DevBuf<double> coarse_inv, coarse_work;  // [n_hier][n * n]: inverse of the coarsest operators, scratch of its computation
   DevBuf<int> coarse_flag;
   bool strips_known = false;
   int nx = 0, ny = 0;
-  int n_hier = 2;  // Q1 on cubes: plain + checkerboard-twisted hierarchy; P1 on lattice-structured simplex grids: one
-  // Q2 on cubes ("cg.mg2"): hierarchy 0 for A_P, hierarchy 1 for A_H, each with a level-0 operator of its own (the
-  // twisted Q1 hierarchy instead reads its level-0 operator from the plain one's arrays)
-  // P2 on lattice-structured simplex grids ("cg.mg2.simplex"): one hierarchy, as for P1
-  MgKind kind = MgKind::mg;
-  bool q2() const { return kind == MgKind::mg2; }
+  MgSpace space = MgSpace::q1_cube;
+  // Q1 on cubes: plain + checkerboard-twisted hierarchy; Q2 on cubes: hierarchy 0 for A_P, hierarchy 1 for A_H; the
+  // lattices: one
+  int n_hier() const { return space == MgSpace::q1_cube || space == MgSpace::q2_cube ? 2 : 1; }
+  // level 0 of hierarchy 1 is C A_c C, read sign-twisted from hierarchy 0's arrays (it has no level-0 arrays of its own)
+  bool twisted0() const { return space == MgSpace::q1_cube; }
+  const char* type_name() const {
+    return space == MgSpace::q2_cube ? "cg.mg2" : space == MgSpace::p2_lattice ? "cg.mg2.simplex" : "cg.mg";
+  }
   MgDist dist;
 };
-
-static const char* mg_type_name(MgKind k) {
-  return k == MgKind::mg2 ? "cg.mg2" : k == MgKind::mg2_simplex ? "cg.mg2.simplex" : "cg.mg";
-}
 
 static inline dim3 grid2(int64_t cnt, int n_hier = 2) { return dim3(unsigned(blocks_for(cnt)), unsigned(n_hier)); }
 
@@ -1182,55 +1141,33 @@ void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_de
   while (nx1 < n_verts && xy_host[2 * nx1 + 1] == xy_host[1]) ++nx1;
   if (nx1 < 2 || n_verts % nx1 != 0) return;
   const int64_t nx = nx1 - 1, ny = n_verts / nx1 - 1;
+  // simplices: a lattice-structured triangulation (two triangles per lattice cell, e.g. the ALU ladder) whose vertex
+  // coordinates are a tensor product and whose triangles join lattice neighbours
+  const bool simplex = m->kind == HDD_SIMPLEX2D;
+  if (ny < 1 || (simplex ? 2 : 1) * nx * ny != m->n_global) return;
   cudaStream_t s = m->stream;
-  if (m->kind == HDD_SIMPLEX2D) {
-    // lattice-structured triangulation (two triangles per lattice cell, e.g. the ALU ladder): vertex coordinates are a
-    // tensor product, every triangle joins lattice neighbours
-    if (ny < 1 || 2 * nx * ny != m->n_global) return;
-    std::vector<double> xs, ys;
-    xs.resize(size_t(nx1));
-    ys.resize(size_t(ny) + 1);
-    for (int64_t i = 0; i < nx1; ++i) xs[size_t(i)] = xy_host[2 * i];
-    for (int64_t j = 0; j <= ny; ++j) ys[size_t(j)] = xy_host[2 * j * nx1 + 1];
-    DevBuf<double> d_xs, d_ys;
-    d_xs.upload(xs.data(), xs.size(), s);
-    d_ys.upload(ys.data(), ys.size(), s);
-    DevBuf<int32_t> flag;
-    flag.alloc(1);
-    flag.zero(s);
-    k_struct_triangles<<<blocks_for(m->n_loc), kMgThreads, 0, s>>>(cv_dev, m->n_loc, int(nx1), n_verts, flag.p);
-    k_struct_verts<<<blocks_for(v_end - v_begin), kMgThreads, 0, s>>>(xy_dev, v_begin, v_end - v_begin, int(nx), d_xs.p, d_ys.p, flag.p);
-    count_launch(2);
-    int32_t f = 0;
-    HDD_CUDA(cudaMemcpyAsync(&f, flag.p, sizeof(f), cudaMemcpyDeviceToHost, s));
-    HDD_CUDA(cudaStreamSynchronize(s));
-    if (f == 0) {
-      m->lx = int(nx);
-      m->ly = int(ny);
-    }
-    return;
-  }
-  if (ny < 1 || nx * ny != m->n_global) return;
   // column / row coordinates from the first grid row and the first grid column of the caller's array
-  std::vector<double> xs, ys;
-  xs.resize(size_t(nx1));
-  ys.resize(size_t(ny) + 1);
+  std::vector<double> xs(static_cast<size_t>(nx1)), ys(static_cast<size_t>(ny + 1));
   for (int64_t i = 0; i < nx1; ++i) xs[size_t(i)] = xy_host[2 * i];
   for (int64_t j = 0; j <= ny; ++j) ys[size_t(j)] = xy_host[2 * j * nx1 + 1];
   DevBuf<double> d_xs, d_ys;
   d_xs.upload(xs.data(), xs.size(), s);
   d_ys.upload(ys.data(), ys.size(), s);
-  m->cell_v0.alloc(size_t(m->n_loc));
-  m->lex_cell.alloc(size_t(m->n_global));
-  HDD_CUDA(cudaMemsetAsync(m->lex_cell.p, 0xFF, size_t(m->n_global) * sizeof(int32_t), s));  // -1: not on this rank
   DevBuf<int32_t> flag;
   flag.alloc(1);
   flag.zero(s);
-  k_struct_cells<<<blocks_for(m->n_loc), kMgThreads, 0, s>>>(cv_dev, m->n_loc, int(nx), int(ny), m->cell_v0.p, m->lex_cell.p, flag.p);
+  if (simplex) {
+    k_struct_triangles<<<blocks_for(m->n_loc), kMgThreads, 0, s>>>(cv_dev, m->n_loc, int(nx1), n_verts, flag.p);
+  } else {
+    m->cell_v0.alloc(size_t(m->n_loc));
+    m->lex_cell.alloc(size_t(m->n_global));
+    HDD_CUDA(cudaMemsetAsync(m->lex_cell.p, 0xFF, size_t(m->n_global) * sizeof(int32_t), s));  // -1: not on this rank
+    k_struct_cells<<<blocks_for(m->n_loc), kMgThreads, 0, s>>>(cv_dev, m->n_loc, int(nx), int(ny), m->cell_v0.p, m->lex_cell.p, flag.p);
+    m->tgeo.alloc(4 * size_t(nx + ny));
+    k_struct_geo<<<blocks_for(nx + ny), kMgThreads, 0, s>>>(d_xs.p, d_ys.p, int(nx), int(ny), m->tgeo.p);
+  }
   k_struct_verts<<<blocks_for(v_end - v_begin), kMgThreads, 0, s>>>(xy_dev, v_begin, v_end - v_begin, int(nx), d_xs.p, d_ys.p, flag.p);
-  m->tgeo.alloc(4 * size_t(nx + ny));
-  k_struct_geo<<<blocks_for(nx + ny), kMgThreads, 0, s>>>(d_xs.p, d_ys.p, int(nx), int(ny), m->tgeo.p);
-  count_launch(3);
+  count_launch(simplex ? 2 : 3);
   int32_t f = 0;
   HDD_CUDA(cudaMemcpyAsync(&f, flag.p, sizeof(f), cudaMemcpyDeviceToHost, s));
   HDD_CUDA(cudaStreamSynchronize(s));
@@ -1238,10 +1175,13 @@ void mg_detect_structure(hdd_mesh* m, const double* xy_host, const double* xy_de
     m->cell_v0.release();
     m->lex_cell.release();
     m->tgeo.release();
-    return;
+  } else if (simplex) {
+    m->lx = int(nx);
+    m->ly = int(ny);
+  } else {
+    m->sx = int(nx);
+    m->sy = int(ny);
   }
-  m->sx = int(nx);
-  m->sy = int(ny);
 }
 
 // recomputes the Galerkin operators below the finest level and the dense coarsest inverses; the level buffers are
@@ -1261,34 +1201,33 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
     MgLevel& c = *st.levels[l + 1];
     Rows rc{0, c.nv};
     const int lc = int(l) + 1;
-    const int nh = st.n_hier;
+    const int nh = st.n_hier();
     if (lc < nd) {
       rc = row_range(c, d.b_lo[lc], d.b_hi[lc]);
     } else if (lc == nd && nd > 0) {
       HDD_CUDA(cudaMemsetAsync(c.S.p, 0, size_t(nh) * 9 * c.nv * sizeof(double), s));
       rc = row_range(c, d.own_lo, d.own_hi);
     }
-    const bool shared = l == 0 && !st.q2();  // level 0 of the twisted hierarchy is read from the plain one's arrays
-    k_rap<<<grid2(rc.cnt, nh), kMgThreads, 0, s>>>(f.S.p, shared ? 0 : 9 * f.nv, f.nx, f.ny, (shared && nh == 2) ? 1 : 0, rc, c.S.p,
-                                                  9 * c.nv);
+    const bool shared = l == 0 && st.twisted0();  // level 0 of the twisted hierarchy is read from the plain one's arrays
+    k_rap<<<grid2(rc.cnt, nh), kMgThreads, 0, s>>>(f.S.p, shared ? 0 : 9 * f.nv, f.nx, f.ny, shared ? 1 : 0, rc, c.S.p, 9 * c.nv);
     count_launch();
     if (lc == nd && nd > 0) Nccl::get().all_reduce_sum(c.S.p, size_t(nh) * 9 * c.nv, m->comm, s);
   }
   for (size_t l = 0; l < nl; ++l) {
     MgLevel& L = *st.levels[l];
     const Rows r = int(l) < nd ? row_range(L, d.b_lo[l], d.b_hi[l]) : Rows{0, L.nv};
-    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), (l == 0 && !st.q2()) ? 1u : unsigned(st.n_hier)), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
+    k_mg_dinv<<<dim3(unsigned(blocks_for(r.cnt)), (l == 0 && st.twisted0()) ? 1u : unsigned(st.n_hier())), kMgThreads, 0, s>>>(L.S.p, L.nv, r, L.dinv.p);
     count_launch();
   }
   // dense inverses of the coarsest operators (s.p.d.): Gauss-Jordan on the device, one CTA per hierarchy
   MgLevel& C = *st.levels.back();
-  const char* type = mg_type_name(st.kind);
+  const char* type = st.type_name();
   if (C.nv > kMaxCoarse)
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, type << ": the " << st.nx << " x " << st.ny << " grid cannot be coarsened by halving down to at most "
                                                            << kMaxCoarse << " vertices (stuck at " << C.nx << " x " << C.ny << ")");
   const int n = int(C.nv);
-  const bool shared = nl == 1 && !st.q2();  // coarsest = finest level, whose operator the twisted hierarchy shares
-  const size_t need = size_t(st.n_hier) * n * n;
+  const bool shared = nl == 1 && st.twisted0();  // coarsest = finest level, whose operator the twisted hierarchy shares
+  const size_t need = size_t(st.n_hier()) * n * n;
   if (st.coarse_inv.n < need) st.coarse_inv.alloc(need);
   if (st.coarse_work.n < need) st.coarse_work.alloc(need);
   if (!st.coarse_flag.p) st.coarse_flag.alloc(1);
@@ -1299,13 +1238,11 @@ static void build_hierarchies(hdd_swipdg* h, MgState& st) {
   const size_t band_bytes = size_t(n) * size_t(C.nx + 3) * sizeof(double);
   if (!gauss_jordan && band_bytes <= 200 * 1024 && n <= 512) {
     HDD_CUDA(cudaFuncSetAttribute(k_dense_inverse_banded, cudaFuncAttributeMaxDynamicSharedMemorySize, int(band_bytes)));
-    k_dense_inverse_banded<<<st.n_hier, 512, band_bytes, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny,
-                                                              (shared && st.n_hier == 2) ? 1 : 0, st.coarse_work.p,
-                                                              st.coarse_inv.p, st.coarse_flag.p);
+    k_dense_inverse_banded<<<st.n_hier(), 512, band_bytes, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny, shared ? 1 : 0,
+                                                                st.coarse_work.p, st.coarse_inv.p, st.coarse_flag.p);
   } else {
-    k_dense_inverse<<<st.n_hier, 1024, 0, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny,
-                                               (shared && st.n_hier == 2) ? 1 : 0, st.coarse_work.p, st.coarse_inv.p,
-                                               st.coarse_flag.p);
+    k_dense_inverse<<<st.n_hier(), 1024, 0, s>>>(C.S.p, shared ? 0 : int64_t(9) * n, C.nx, C.ny, shared ? 1 : 0, st.coarse_work.p,
+                                                 st.coarse_inv.p, st.coarse_flag.p);
   }
   count_launch();
   int bad = 0;
@@ -1323,14 +1260,14 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
   const int nl = int(st.levels.size());
   const MgDist& d = st.dist;
   const int nd = d.on ? d.n_dist : 0;
-  const int nh = st.n_hier;
+  const int nh = st.n_hier();
   SolvePhases& pt = phase_timer();
   // ---- down: pre-smoothing + restriction ---------------------------------------------------------------------------
   for (int l = 0; l + 1 < nl; ++l) {
     MgLevel& L = *st.levels[size_t(l)];
     MgLevel& Cn = *st.levels[size_t(l) + 1];
     const Rows rp = l < nd ? row_range(L, d.pre_lo[l], d.pre_hi[l]) : Rows{0, L.nv};
-    if (l == 0 && nh == 2 && !st.q2())
+    if (l == 0 && st.twisted0())
       k_mg_pre2<<<blocks_for(rp.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
     else
       k_mg_pre<<<grid2(rp.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, rp, L.b.p, L.x.p, L.r.p);
@@ -1367,7 +1304,7 @@ static void vcycle(hdd_mesh* m, MgState& st, const int* done, cudaStream_t s) {
     } else {
       const Rows rq = l < nd ? row_range(L, d.pro_lo[l], d.pro_hi[l]) : Rows{0, L.nv};
       k_mg_prolong_add<<<grid2(rq.cnt, nh), kMgThreads, 0, s>>>(done, Cn.result, L.nx, L.ny, rq, L.x.p);
-      if (l == 0 && nh == 2 && !st.q2())
+      if (l == 0 && st.twisted0())
         k_mg_post2<<<blocks_for(ru.cnt), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
       else
         k_mg_post<<<grid2(ru.cnt, nh), kMgThreads, 0, s>>>(done, L.S.p, L.dinv.p, L.nx, L.ny, ru, L.b.p, L.x.p, L.y.p);
@@ -1447,12 +1384,7 @@ static void detect_strips(hdd_swipdg* h, MgState& st) {
   d.c1 = c1;
   d.lower = m->rank > 0 ? m->rank - 1 : -1;
   d.upper = m->rank + 1 < m->world ? m->rank + 1 : -1;
-  d.last = d.upper < 0;
   mg_strip_plan(st.ny, c0, c1, n_dist, d);
-  // the message size is the same on every rank: the ghost width of an interior strip
-  MgDist interior;
-  mg_strip_plan(st.ny, 1 << 20, (1 << 20) + (1 << 10), n_dist, interior);
-  (void)interior;
   const size_t rows = size_t(d.ghost) + 1;
   if (d.tmp_lo.n < rows * (size_t(st.nx) + 1)) {
     d.tmp_lo.alloc(rows * (size_t(st.nx) + 1));
@@ -1462,42 +1394,55 @@ static void detect_strips(hdd_swipdg* h, MgState& st) {
 
 void mg_release(MgState* st) { delete st; }
 
-// (re)builds the hierarchies for the frozen operator `vals`
-void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
-  hdd_mesh* m = h->mesh;
+// The multigrid variant `type` runs on this discretization; refuses the combinations no variant covers
+static MgSpace mg_space(const hdd_swipdg* h, SolverType type) {
+  const hdd_mesh* m = h->mesh;
   const bool cube = m->kind == HDD_CUBE2D && m->sx > 0, lattice = m->kind == HDD_SIMPLEX2D && m->lx > 0;
-  const bool q2 = kind == MgKind::mg2, p2s = kind == MgKind::mg2_simplex;
   const bool p2_lattice = lattice && h->polorder == 2;  // what "cg.mg2.simplex" is for
-  if (q2 && h->polorder == 1)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "solver type 'cg.mg2' is the multigrid preconditioner for polOrder 2; use 'cg.mg' for polOrder 1");
-  if (q2 && !cube)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
-              "solver type 'cg.mg2' needs Q2 on a logically structured HDD_CUBE2D grid with the vertices numbered x-fastest "
-              "(Stuff::Grid::Providers::Cube / hdd_grid_cube); use 'cg.blockdiagonal'"
-                  << (p2_lattice ? " or 'cg.mg2.simplex'" : ""));
-  if (p2s && m->kind != HDD_SIMPLEX2D)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
-              "solver type 'cg.mg2.simplex' needs a simplex grid; on HDD_CUBE2D grids use 'cg.mg' (polOrder 1) or 'cg.mg2' (polOrder 2)");
-  if (p2s && h->polorder == 1)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
-              "solver type 'cg.mg2.simplex' is the multigrid preconditioner for polOrder 2 on triangles; use 'cg.mg' for polOrder 1");
-  if (p2s && !lattice)
-    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
-              "solver type 'cg.mg2.simplex' needs a simplex grid whose vertices form a lattice numbered x-fastest and whose "
-              "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.blockdiagonal'");
-  if (kind == MgKind::mg && ((!cube && !lattice) || h->polorder != 1))
+  if (type == SolverType::mg) {
+    if (h->polorder == 1 && cube) return MgSpace::q1_cube;
+    if (h->polorder == 1 && lattice) return MgSpace::p1_lattice;
     HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
               "solver type 'cg.mg' needs polOrder 1 on a logically structured grid: HDD_CUBE2D with the vertices numbered x-fastest "
               "(Stuff::Grid::Providers::Cube / hdd_grid_cube) or a simplex grid whose vertices form such a lattice and whose "
               "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.diagonal' or 'cg.blockdiagonal'"
                   << (p2_lattice ? " or 'cg.mg2.simplex'" : ""));
+  }
+  if (type == SolverType::mg2) {
+    if (h->polorder == 1)
+      HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET, "solver type 'cg.mg2' is the multigrid preconditioner for polOrder 2; use 'cg.mg' for polOrder 1");
+    if (!cube)
+      HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+                "solver type 'cg.mg2' needs Q2 on a logically structured HDD_CUBE2D grid with the vertices numbered x-fastest "
+                "(Stuff::Grid::Providers::Cube / hdd_grid_cube); use 'cg.blockdiagonal'"
+                    << (p2_lattice ? " or 'cg.mg2.simplex'" : ""));
+    return MgSpace::q2_cube;
+  }
+  // SolverType::mg2_simplex
+  if (m->kind != HDD_SIMPLEX2D)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' needs a simplex grid; on HDD_CUBE2D grids use 'cg.mg' (polOrder 1) or 'cg.mg2' (polOrder 2)");
+  if (h->polorder == 1)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' is the multigrid preconditioner for polOrder 2 on triangles; use 'cg.mg' for polOrder 1");
+  if (!lattice)
+    HDD_THROW(HDD_ERR_REQUIREMENTS_NOT_MET,
+              "solver type 'cg.mg2.simplex' needs a simplex grid whose vertices form a lattice numbered x-fastest and whose "
+              "triangles join lattice neighbours (the ALU ladder, hdd_grid_simplex); use 'cg.blockdiagonal'");
+  return MgSpace::p2_lattice;
+}
+
+// (re)builds the hierarchies for the frozen operator `vals`
+void mg_setup(hdd_swipdg* h, const double* vals, SolverType type) {
+  const MgSpace space = mg_space(h, type);
+  hdd_mesh* m = h->mesh;
   cudaStream_t s = m->stream;
   if (!h->mg) h->mg = new MgState;
   MgState& st = *h->mg;
+  const bool cube = space == MgSpace::q1_cube || space == MgSpace::q2_cube;
   st.nx = cube ? m->sx : m->lx;
   st.ny = cube ? m->sy : m->ly;
-  st.n_hier = cube ? 2 : 1;
-  st.kind = kind;
+  st.space = space;
   const int64_t nv = int64_t(st.nx + 1) * (st.ny + 1);
   if (!st.levels.empty() && (st.levels[0]->nx != st.nx || st.levels[0]->ny != st.ny)) {
     st.levels.clear();
@@ -1510,7 +1455,7 @@ void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
       L->nx = lx;
       L->ny = ly;
       L->nv = int64_t(lx + 1) * (ly + 1);
-      const size_t ops = (l == 0 && !q2) ? 1 : 2;  // the twisted hierarchy shares the level-0 operator of the plain one
+      const size_t ops = (l == 0 && space != MgSpace::q2_cube) ? 1 : 2;  // only Q2 has a second level-0 operator of its own
       L->S.alloc(ops * 9 * size_t(L->nv));
       L->dinv.alloc(ops * size_t(L->nv));
       L->b.alloc(2 * size_t(L->nv));
@@ -1526,9 +1471,9 @@ void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
   }
   phase_timer().mark("setup mg: allocation", s);
   // the strip layout depends on the mesh and the communicator only: decided at the first solve of this discretization
-  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated).  "cg.mg2" and
-  // "cg.mg2.simplex" always run their vertex levels replicated.
-  if (!st.strips_known && kind == MgKind::mg) {
+  // (two stream synchronisations and a collective - 3 ms per solve at 2 and 8 ranks when repeated).  Q2 and P2 always run
+  // their vertex levels replicated.
+  if (!st.strips_known && (space == MgSpace::q1_cube || space == MgSpace::p1_lattice)) {
     detect_strips(h, st);
     st.strips_known = true;
   }
@@ -1540,9 +1485,9 @@ void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
     // g rows next to the strip from the neighbours - instead of an all-reduce of the whole operator
     const int nx1 = st.nx + 1;
     const Rows mine{int64_t(d.c0) * nx1, int64_t(d.c1 - d.c0 + 1) * nx1};
-    if (lattice)  // writes the rows of the vertices with an owned triangle: c0 .. c1
-      k_vertex_galerkin_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
-                                                                            m->cell_gv.p, m->n_verts_loc, st.nx, st.ny, f0.S.p);
+    if (space == MgSpace::p1_lattice)  // writes the rows of the vertices with an owned triangle: c0 .. c1
+      k_vertex_galerkin_lattice<1><<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
+                                                                                    m->cell_gv.p, m->n_verts_loc, st.nx, st.ny, f0.S.p);
     else
       k_vertex_galerkin<<<blocks_for(mine.cnt), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, mine, f0.S.p);
     count_launch();
@@ -1570,29 +1515,33 @@ void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
         f0.S.p, nv, d.lower >= 0 ? lo.p : nullptr, d.upper >= 0 ? up.p : nullptr, st.nx, d.c0, d.c1, g, lo_row, hi_row);
     count_launch();
     HDD_CUDA(cudaStreamSynchronize(s));  // lo / up are freed at the end of this scope
-  } else if (q2) {
-    // every rank writes every vertex (zeros where it owns no cell): the all-reduce makes both operators global
-    k_vertex_galerkin_q2<<<blocks_for(nv), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, f0.S.p);
-    count_launch();
-    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(18) * nv, m->comm, s);
-    k_hourglass_fill<<<1, 1024, 0, s>>>(f0.S.p + 13 * nv, st.nx, st.ny);  // diagonal of hierarchy 1: array 9 + 4
-    count_launch();
-  } else if (p2s) {
-    if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
-    k_vertex_galerkin_p2<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
-                                                                          m->cell_gv.p, m->n_verts_loc, st.nx, st.ny, f0.S.p);
-    count_launch();
-    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
-  } else if (lattice) {
-    if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
-    k_vertex_galerkin_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p,
-                                                                          m->cell_gv.p, m->n_verts_loc, st.nx, st.ny, f0.S.p);
-    count_launch();
-    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
   } else {
-    k_vertex_galerkin<<<blocks_for(nv), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, Rows{0, nv}, f0.S.p);
-    count_launch();
-    if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
+    switch (space) {
+      case MgSpace::q1_cube:
+        k_vertex_galerkin<<<blocks_for(nv), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, Rows{0, nv},
+                                                                f0.S.p);
+        count_launch();
+        if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
+        break;
+      case MgSpace::q2_cube:
+        // every rank writes every vertex (zeros where it owns no cell): the all-reduce makes both operators global
+        k_vertex_galerkin_q2<<<blocks_for(nv), kMgThreads, 0, s>>>(h->view(), vals, m->cell_v0.p, m->lex_cell.p, m->sx, m->sy, f0.S.p);
+        count_launch();
+        if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(18) * nv, m->comm, s);
+        k_hourglass_fill<<<1, 1024, 0, s>>>(f0.S.p + 13 * nv, st.nx, st.ny);  // diagonal of hierarchy 1: array 9 + 4
+        count_launch();
+        break;
+      case MgSpace::p1_lattice:
+      case MgSpace::p2_lattice: {
+        const auto kernel = space == MgSpace::p1_lattice ? k_vertex_galerkin_lattice<1> : k_vertex_galerkin_lattice<2>;
+        if (m->world > 1) HDD_CUDA(cudaMemsetAsync(f0.S.p, 0, size_t(9) * nv * sizeof(double), s));
+        kernel<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(h->view(), vals, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->cell_gv.p,
+                                                                 m->n_verts_loc, st.nx, st.ny, f0.S.p);
+        count_launch();
+        if (m->world > 1) Nccl::get().all_reduce_sum(f0.S.p, size_t(9) * nv, m->comm, s);
+        break;
+      }
+    }
   }
   HDD_CUDA(cudaGetLastError());
   phase_timer().mark("setup mg: level-0 operator", s);
@@ -1601,8 +1550,8 @@ void mg_setup(hdd_swipdg* h, const double* vals, MgKind kind) {
   HDD_CUDA(cudaGetLastError());
 }
 
-// z += P V(P^T r) + P C V_C(C P^T r) ("cg.mg2": z += P V_P(P^T r) + H V_H(H^T r); P1 on lattice simplices and
-// "cg.mg2.simplex": z += P V(P^T r)), red[1] = r.z; p_init != nullptr also stores z as the first direction
+// z += P V(P^T r) + P C V_C(C P^T r) (Q2 on cubes: z += P V_P(P^T r) + H V_H(H^T r); the lattices: z += P V(P^T r)),
+// red[1] = r.z; p_init != nullptr also stores z as the first direction
 void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double* p_init, double* partial, CgScalars* sc) {
   hdd_mesh* m = h->mesh;
   MgState& st = *h->mg;
@@ -1616,9 +1565,9 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
   if (d.on) {
     // vertex rows c0 .. c1 of my cells; rows c0 and c1 are shared with the ranks below / above
     const Rows mine{int64_t(d.c0) * nx1, int64_t(d.c1 - d.c0 + 1) * nx1};
-    if (st.n_hier == 1)  // triangles: every local vertex (rows c0 - 1 .. c1 + 1; the outer two receive zeros and are ghost rows)
-      k_dg_restrict_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->n_verts_loc,
-                                                                        m->own0, m->n_own, b0);
+    if (st.space == MgSpace::p1_lattice)  // every local vertex (rows c0 - 1 .. c1 + 1; the outer two receive zeros and are ghost rows)
+      k_dg_restrict_lattice<1><<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p,
+                                                                                m->n_verts_loc, m->own0, m->n_own, b0);
     else
       k_dg_restrict<<<blocks_for(mine.cnt), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, mine, b0, nullptr);
     count_launch();
@@ -1641,55 +1590,62 @@ void mg_apply(hdd_swipdg* h, const int* done, const double* r, double* z, double
     k_ghost_unpack_twist<<<blocks_for(int64_t(hi_row - lo_row + 1) * nx1), kMgThreads, 0, s>>>(
         done, b0, b1, d.lower >= 0 ? d.tmp_lo.p : nullptr, d.upper >= 0 ? d.tmp_up.p : nullptr, st.nx, d.c0, d.c1, g, lo_row, hi_row);
     count_launch();
-  } else if (st.kind == MgKind::mg2_simplex) {
-    // P2 on a lattice-structured simplex grid: conforming P1 auxiliary space, one hierarchy, run replicated
-    if (multi) HDD_CUDA(cudaMemsetAsync(b0, 0, size_t(a.nv) * sizeof(double), s));
-    k_dg_restrict_p2<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->n_verts_loc,
-                                                                      m->own0, m->n_own, b0);
-    count_launch();
-    if (multi) Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
-  } else if (st.q2()) {
-    // Q2: b0 = P^T r, b1 = H^T r; every rank writes every vertex (zeros where it owns no cell), one all-reduce of both
-    k_dg_restrict_q2<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, b0, b1);
-    count_launch();
-    if (multi) Nccl::get().all_reduce_sum(b0, size_t(2) * a.nv, m->comm, s);
-  } else if (st.n_hier == 1) {
-    // lattice-structured simplex grid: conforming P1 auxiliary space, one hierarchy
-    if (multi) HDD_CUDA(cudaMemsetAsync(b0, 0, size_t(a.nv) * sizeof(double), s));
-    k_dg_restrict_p1<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->n_verts_loc,
-                                                                      m->own0, m->n_own, b0);
-    count_launch();
-    if (multi) Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
   } else {
-    k_dg_restrict<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, Rows{0, a.nv}, b0,
-                                                           multi ? nullptr : b1);
-    count_launch();
-    if (multi) {
-      Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
-      k_twist_vector<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, b0, st.nx, Rows{0, a.nv}, b1);
-      count_launch();
+    switch (st.space) {
+      case MgSpace::q1_cube:
+        k_dg_restrict<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, Rows{0, a.nv}, b0,
+                                                               multi ? nullptr : b1);
+        count_launch();
+        if (multi) {
+          Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
+          k_twist_vector<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, b0, st.nx, Rows{0, a.nv}, b1);
+          count_launch();
+        }
+        break;
+      case MgSpace::q2_cube:
+        // b0 = P^T r, b1 = H^T r; every rank writes every vertex (zeros where it owns no cell), one all-reduce of both
+        k_dg_restrict_q2<<<blocks_for(a.nv), kMgThreads, 0, s>>>(done, r, m->lex_cell.p, m->own0, m->n_own, st.nx, st.ny, b0, b1);
+        count_launch();
+        if (multi) Nccl::get().all_reduce_sum(b0, size_t(2) * a.nv, m->comm, s);
+        break;
+      case MgSpace::p1_lattice:
+      case MgSpace::p2_lattice: {
+        const auto kernel = st.space == MgSpace::p1_lattice ? k_dg_restrict_lattice<1> : k_dg_restrict_lattice<2>;
+        if (multi) HDD_CUDA(cudaMemsetAsync(b0, 0, size_t(a.nv) * sizeof(double), s));
+        kernel<<<blocks_for(m->n_verts_loc), kMgThreads, 0, s>>>(done, r, m->vptr.p, m->vdof.p, m->lvert_gid.p, m->n_verts_loc, m->own0,
+                                                                 m->n_own, b0);
+        count_launch();
+        if (multi) Nccl::get().all_reduce_sum(b0, size_t(a.nv), m->comm, s);
+        break;
+      }
     }
   }
   phase_timer().mark(d.on ? "mg ghost unpack" : "mg dg-restrict", s);
   if (st.levels.size() == 1) {
     // the fine vertex grid is already small enough for the dense solve
-    k_mg_dense<<<dim3(unsigned(int(a.nv) + 3) / 4, unsigned(st.n_hier)), 128, 0, s>>>(done, st.coarse_inv.p, int(a.nv), a.b.p, a.x.p);
+    k_mg_dense<<<dim3(unsigned(int(a.nv) + 3) / 4, unsigned(st.n_hier())), 128, 0, s>>>(done, st.coarse_inv.p, int(a.nv), a.b.p, a.x.p);
     count_launch();
     a.result = a.x.p;
   } else {
     vcycle(m, st, done, s);
   }
   const int grid = int(std::min<int64_t>((m->n_own + kMgThreads - 1) / kMgThreads, kMaxBlocks));
-  if (st.q2())
-    k_dg_prolong_dot_q2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z,
-                                                    p_init, partial, sc);
-  else if (st.kind == MgKind::mg2_simplex)
-    k_dg_prolong_dot_p2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
-  else if (st.n_hier == 1)
-    k_dg_prolong_dot_p1<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
-  else
-    k_dg_prolong_dot<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z, p_init,
-                                                 partial, sc);
+  switch (st.space) {
+    case MgSpace::q1_cube:
+      k_dg_prolong_dot<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z, p_init,
+                                                   partial, sc);
+      break;
+    case MgSpace::q2_cube:
+      k_dg_prolong_dot_q2<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_v0.p + m->own0, st.nx, a.result, a.result + a.nv, r, z,
+                                                      p_init, partial, sc);
+      break;
+    case MgSpace::p1_lattice:
+    case MgSpace::p2_lattice: {
+      const auto kernel = st.space == MgSpace::p1_lattice ? k_dg_prolong_dot_lattice<1> : k_dg_prolong_dot_lattice<2>;
+      kernel<<<grid, kMgThreads, 0, s>>>(done, m->n_own, m->cell_gv.p + size_t(3) * m->own0, a.result, r, z, p_init, partial, sc);
+      break;
+    }
+  }
   count_launch();
   phase_timer().mark("mg dg-prolong + r.z", s);
   HDD_CUDA(cudaGetLastError());
@@ -1699,7 +1655,7 @@ int mg_num_levels(const hdd_swipdg* h) { return h->mg ? int(h->mg->levels.size()
 
 void mg_vertex_result(const hdd_swipdg* h, double* host) {
   const MgLevel& a = *h->mg->levels[0];
-  HDD_CUDA(cudaMemcpyAsync(host, a.result, size_t(h->mg->n_hier) * a.nv * sizeof(double), cudaMemcpyDeviceToHost,
+  HDD_CUDA(cudaMemcpyAsync(host, a.result, size_t(h->mg->n_hier()) * a.nv * sizeof(double), cudaMemcpyDeviceToHost,
                            h->mesh->stream));
 }
 
@@ -1712,8 +1668,8 @@ extern "C" int hdd_mg_level_operator(const hdd_swipdg* h, int level, int hier, i
     if (!st) HDD_THROW(HDD_ERR_USING_THIS_WRONG, "no multigrid hierarchy: solve with 'cg.mg', 'cg.mg2' or 'cg.mg2.simplex' first");
     if (level < 0 || level >= int(st->levels.size()))
       HDD_THROW(HDD_ERR_WRONG_INPUT, "level " << level << " of " << st->levels.size());
-    if (hier < 0 || hier >= st->n_hier) HDD_THROW(HDD_ERR_WRONG_INPUT, "hierarchy " << hier << " of " << st->n_hier);
-    if (level == 0 && hier == 1 && !st->q2())
+    if (hier < 0 || hier >= st->n_hier()) HDD_THROW(HDD_ERR_WRONG_INPUT, "hierarchy " << hier << " of " << st->n_hier());
+    if (level == 0 && hier == 1 && st->twisted0())
       HDD_THROW(HDD_ERR_WRONG_INPUT, "level 0 of the twisted hierarchy is C A_c C, read from the plain one's arrays");
     const hdd::MgLevel& L = *st->levels[size_t(level)];
     if (nx) *nx = L.nx;

@@ -363,15 +363,28 @@ bool setup_p2p(hdd_swipdg* h) {
   return true;
 }
 
-int parse_solver_type(const char* type) {
+// the solver types in the order hdd_solver_types lists their canonical names, with the other spellings hdd_solve accepts
+struct SolverTypeName {
+  SolverType type;
+  const char* name;
+  const char* aliases[5];  // unused entries nullptr
+};
+const SolverTypeName kSolverTypes[] = {
+    {SolverType::diagonal, "cg.diagonal", {"", "cg", "cg.jacobi", "cg.diagonal.lower", "cg.diagonal.upper"}},
+    {SolverType::blockdiagonal, "cg.blockdiagonal", {"cg.blockjacobi"}},
+    {SolverType::identity, "cg.identity", {"cg.identity.lower", "cg.identity.upper"}},
+    {SolverType::mg, "cg.mg", {"cg.multigrid"}},
+    {SolverType::mg2, "cg.mg2", {"cg.multigrid2"}},
+    {SolverType::mg2_simplex, "cg.mg2.simplex", {"cg.multigrid2.simplex"}},
+};
+
+SolverType parse_solver_type(const char* type) {
   const std::string t = type ? type : "";
-  if (t.empty() || t == "cg.diagonal" || t == "cg.jacobi" || t == "cg" || t == "cg.diagonal.lower" || t == "cg.diagonal.upper")
-    return 1;
-  if (t == "cg.identity" || t == "cg.identity.lower" || t == "cg.identity.upper") return 0;
-  if (t == "cg.blockdiagonal" || t == "cg.blockjacobi") return 2;
-  if (t == "cg.mg" || t == "cg.multigrid") return 3;
-  if (t == "cg.mg2" || t == "cg.multigrid2") return 4;
-  if (t == "cg.mg2.simplex" || t == "cg.multigrid2.simplex") return 5;
+  for (const SolverTypeName& e : kSolverTypes) {
+    if (t == e.name) return e.type;
+    for (const char* a : e.aliases)
+      if (a && t == a) return e.type;
+  }
   HDD_THROW(HDD_ERR_WRONG_INPUT, "solver type '" << t << "' is not one of solver_types()");
 }
 
@@ -496,7 +509,6 @@ double total(const std::vector<double>& v) {
 const char* const kEstimatorTypes[] = {"eta_NC_ESV2007", "eta_R_ESV2007",  "eta_R_ESV2007_*", "eta_DF_ESV2007", "eta_ESV2007",
                                        "eta_ESV2007_alt", "eta_NC_OS2014", "eta_R_OS2014",    "eta_R_OS2014_*", "eta_DF_OS2014",
                                        "eta_DF_OS2014_*", "eta_OS2014",    "eta_OS2014_*"};
-const char* const kSolverTypes[] = {"cg.diagonal", "cg.blockdiagonal", "cg.identity", "cg.mg", "cg.mg2", "cg.mg2.simplex"};
 
 }  // namespace
 
@@ -838,8 +850,13 @@ int hdd_residual(hdd_swipdg* h, const double* mu, int mu_size, double* relative_
 
 int hdd_solver_types(const char* const** types, int* n_types) {
   return guarded([&] {
-    if (types) *types = kSolverTypes;
-    if (n_types) *n_types = int(sizeof(kSolverTypes) / sizeof(kSolverTypes[0]));
+    static const std::vector<const char*> names = [] {
+      std::vector<const char*> v;
+      for (const SolverTypeName& e : kSolverTypes) v.push_back(e.name);
+      return v;
+    }();
+    if (types) *types = names.data();
+    if (n_types) *n_types = int(names.size());
   });
 }
 
@@ -854,7 +871,7 @@ struct CgStart {
 // The start of a CG solve, shared by hdd_solve and hdd_precondition: A(mu) frozen (and b(mu) into c.b if freeze_b), the
 // pure-Neumann fix, the preconditioner's set-up, the peer-memory decision, then x = 0, r = b, p = z = M^-1 b and
 // rz[0] = r.z.  The caller provides c.b, c.x, c.r, c.z (block Jacobi and multigrid), c.p, c.q, c.partial and c.sc.
-CgStart start_cg(hdd_swipdg* h, int use_diag, const double* mu, int mu_size, bool freeze_b, double precision, int max_iter,
+CgStart start_cg(hdd_swipdg* h, SolverType type, const double* mu, int mu_size, bool freeze_b, double precision, int max_iter,
                  CgBuffers& c) {
   hdd_mesh* m = h->mesh;
   cudaStream_t s = m->stream;
@@ -875,21 +892,21 @@ CgStart start_cg(hdd_swipdg* h, int use_diag, const double* mu, int mu_size, boo
   }
   c.values = vals;
   c.dinv = h->dinv.p;
-  if (use_diag >= 2) {
+  if (uses_block_inverses(type)) {
     if (!h->dinv_block.p) h->dinv_block.alloc(size_t(m->n_own) * h->nl * h->nl);
     launch_invert_diag_blocks(v, vals, h->dinv_block.p, s);
     pt.mark("setup: block inverses", s);
     c.dinv_block = h->dinv_block.p;
-    if (use_diag >= 3) mg_setup(h, vals, use_diag == 5 ? MgKind::mg2_simplex : use_diag == 4 ? MgKind::mg2 : MgKind::mg);
+    if (is_multigrid(type)) mg_setup(h, vals, type);
   } else {
     c.z = nullptr;
-    launch_extract_dinv(v, vals, use_diag, h->dinv.p, s);
+    launch_extract_dinv(v, vals, type == SolverType::diagonal, h->dinv.p, s);
   }
   Nccl& nc = Nccl::get();
   const bool multi = m->world > 1;
   // multi GPU, Q1, Jacobi / identity: fused SpMV + halo read over peer memory instead of pack + send/recv
-  bool p2p = multi && p2p_wanted() && use_diag < 2 && cg_spmv_uses_tma(v);
-  if (multi && use_diag < 2) {  // the decision must be collective: a rank without owned cells large enough would disagree
+  bool p2p = multi && p2p_wanted() && !uses_block_inverses(type) && cg_spmv_uses_tma(v);
+  if (multi && !uses_block_inverses(type)) {  // the decision must be collective: a rank without owned cells large enough would disagree
     DevBuf<double> vote;
     double want = p2p ? 0.0 : 1.0;
     vote.upload(&want, 1, s);
@@ -909,7 +926,7 @@ CgStart start_cg(hdd_swipdg* h, int use_diag, const double* mu, int mu_size, boo
     st.peer = &h->peer_view;
   }
   launch_cg_init(v, c, precision, max_iter, s);
-  if (use_diag >= 3) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
+  if (is_multigrid(type)) mg_apply(h, nullptr, c.r, c.z, c.p + size_t(m->own0) * h->nl, c.partial, c.sc);
   if (multi) nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s);
   launch_cg_init_finish(v, c, s);
   pt.mark("setup: cg init", s);
@@ -925,20 +942,20 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
   return guarded([&] {
     require_init(h);
     check_mu(h, mu, mu_size, "mu");
-    const int use_diag = parse_solver_type(type);
+    const SolverType solver = parse_solver_type(type);
     if (!(precision > 0.0)) HDD_THROW(HDD_ERR_WRONG_INPUT, "precision must be positive");
     hdd_mesh* m = h->mesh;
     m->set_device();
     cudaStream_t s = m->stream;
     ensure_solve_workspace(h);
-    if (use_diag >= 2 && !h->z.p) h->z.alloc(size_t(h->n_rows));
+    if (uses_block_inverses(solver) && !h->z.p) h->z.alloc(size_t(h->n_rows));
     cudaEvent_t e0, e1;
     HDD_CUDA(cudaEventCreate(&e0));
     HDD_CUDA(cudaEventCreate(&e1));
     HDD_CUDA(cudaEventRecord(e0, s));
     SolvePhases& pt = phase_timer();
     pt.begin(s);
-    h->last_precond = use_diag;
+    h->last_type = solver;
     CgBuffers c{};
     c.b = h->b.p;
     c.x = h->x.p;
@@ -952,7 +969,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       h->b.alloc(size_t(h->n_rows));
       c.b = h->b.p;
     }
-    const CgStart st = start_cg(h, use_diag, mu, mu_size, true, precision, max_iter, c);
+    const CgStart st = start_cg(h, solver, mu, mu_size, true, precision, max_iter, c);
     const double* vals = st.vals;
     const bool p2p = st.p2p;
     const PeerView* peer = st.peer;
@@ -970,7 +987,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       if (multi) { nc.all_reduce_sum(&c.sc->red[0], 1, m->comm, s); pt.mark("all-reduce p.q", s); }
       launch_cg_update(v, c, parity, s);
       pt.mark("update", s);
-      if (use_diag >= 3) mg_apply(h, &c.sc->done[parity], c.r, c.z, nullptr, c.partial, c.sc);
+      if (is_multigrid(solver)) mg_apply(h, &c.sc->done[parity], c.r, c.z, nullptr, c.partial, c.sc);
       if (multi) { nc.all_reduce_sum(&c.sc->red[1], 2, m->comm, s); pt.mark("all-reduce r.z", s); }
       launch_cg_direction(v, c, parity, s);
       pt.mark("direction", s);
@@ -979,7 +996,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       const char* e = std::getenv("HDD_CG_GRAPH");
       return !(e && e[0] == '0') && !phase_timer().on;
     }();
-    hdd_swipdg::CgGraph& cached = h->cg_graph[use_diag];
+    hdd_swipdg::CgGraph& cached = h->cg_graph[int(solver)];
     const void* key[5] = {vals, c.p_alt, peer, c.dinv_block, m->send_buf.p};
     if (cached.exec && std::memcmp(cached.key, key, sizeof(key)) != 0) {
       cudaGraphExecDestroy(cached.exec);
@@ -987,7 +1004,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     }
     bool capture_failed = false;
     double rr_prev = 1e300;
-    int par = 0, launched = 0, batch = use_diag >= 3 ? 8 : 16;
+    int par = 0, launched = 0, batch = is_multigrid(solver) ? 8 : 16;
     bool first_batch = !cached.exec;  // a cached graph means every one-time set-up has already happened
     for (;;) {
       if (!first_batch && graphs_wanted && !cached.exec && !capture_failed) {
@@ -1081,9 +1098,9 @@ int hdd_precondition(hdd_swipdg* h, const char* type, const double* mu, int mu_s
   return guarded([&] {
     require_init(h);
     check_mu(h, mu, mu_size, "mu");
-    const int use_diag = parse_solver_type(type);
+    const SolverType solver = parse_solver_type(type);
     if (!r_host || !z_host) HDD_THROW(HDD_ERR_WRONG_INPUT, "r_host and z_host must not be NULL");
-    if (vertex_host && use_diag < 3) HDD_THROW(HDD_ERR_WRONG_INPUT, "vertex_host needs a multigrid solver type");
+    if (vertex_host && !is_multigrid(solver)) HDD_THROW(HDD_ERR_WRONG_INPUT, "vertex_host needs a multigrid solver type");
     hdd_mesh* m = h->mesh;
     if (m->world > 1) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "hdd_precondition on more than one GPU");
     if (m->purely_neumann) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "hdd_precondition for the modified pure-Neumann system");
@@ -1112,7 +1129,7 @@ int hdd_precondition(hdd_swipdg* h, const char* type, const double* mu, int mu_s
     c.q = q.p;
     c.partial = partial.p;
     c.sc = sc.p;
-    start_cg(h, use_diag, mu, mu_size, false, 1.0, 1, c);
+    start_cg(h, solver, mu, mu_size, false, 1.0, 1, c);
     HDD_CUDA(cudaMemcpyAsync(z_host, p.p + size_t(m->own0) * h->nl, rows * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (rz) HDD_CUDA(cudaMemcpyAsync(rz, &sc.p->rz[0], sizeof(double), cudaMemcpyDeviceToHost, s));
     if (vertex_host) mg_vertex_result(h, vertex_host);
@@ -1387,10 +1404,10 @@ int hdd_kernel_bytes(hdd_swipdg* h, int which, double* bytes) {
     switch (which) {
       case 0: b = 8.0 * nnz + rec * cells + 8.0 * rows /* read p */ + 8.0 * rows /* write q */; break;
       case 1:  // diagonal: read x,p,q,r,dinv, write x,r; block: read x,p,q,r + n_loc^2 block per cell, write x,r,z
-        b = h->last_precond >= 2 ? 7.0 * 8.0 * rows + 8.0 * nl * rows : 7.0 * 8.0 * rows;
+        b = uses_block_inverses(h->last_type) ? 7.0 * 8.0 * rows + 8.0 * nl * rows : 7.0 * 8.0 * rows;
         break;
       case 2:  // diagonal: read r,dinv,p, write p; block: read z,p, write p
-        b = h->last_precond >= 2 ? 3.0 * 8.0 * rows : 4.0 * 8.0 * rows;
+        b = uses_block_inverses(h->last_type) ? 3.0 * 8.0 * rows : 4.0 * 8.0 * rows;
         break;
       case 3:  // the tensor-grid Q1 kernel reads the neighbour record, the block offset and vertex 0 (28 B), no geometry
         b = 8.0 * nnz + ((m->kind == HDD_CUBE2D && h->polorder == 1 && m->sx > 0) ? 28.0 : geo + rec) * cells;
@@ -1428,7 +1445,7 @@ int hdd_profile_kernel(hdd_swipdg* h, int which, int reps, double* avg_seconds) 
     c.values = h->lhs_comps.empty() ? h->lhs_affine->values.p : h->frozen.p;
     c.dinv = h->dinv.p; c.b = h->b.p; c.x = h->x.p; c.r = h->r.p; c.p = h->p.p; c.q = h->q.p;
     c.partial = h->partial.p; c.sc = h->sc.p;
-    if (h->last_precond >= 2) { c.dinv_block = h->dinv_block.p; c.z = h->z.p; }
+    if (uses_block_inverses(h->last_type)) { c.dinv_block = h->dinv_block.p; c.z = h->z.p; }
     if (which < 3) {
       // un-latch the convergence flag of parity 0 so that the kernels do their work; the vectors are scratch now
       CgScalars sc = *h->sc_host;

@@ -243,7 +243,7 @@ def test_mg2_simplex_gauss_jordan_coarsest_inverse(gpu):
 
 
 def test_mg2_simplex_preconditioner_on_a_large_grid(gpu):
-    """simplex(208): 346 112 owned triangles (the grid-stride loop of k_dg_prolong_dot_p2 runs more than once), 417^2
+    """simplex(208): 346 112 owned triangles (the grid-stride loop of k_dg_prolong_dot_lattice<2> runs more than once), 417^2
     vertices, six levels down to 14^2; the level-0 operator comes from the device"""
     s, nx = 208, 416
     g = grids.simplex(s)
