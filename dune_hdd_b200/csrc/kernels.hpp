@@ -2,9 +2,36 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "device.cuh"
 
 namespace hdd {
+
+// compile-time dispatch of the launchers: f(ic<NF>, ic<NL>) for the block shape (faces, local DoFs) of a mesh, f(ic<NL>)
+// for the local DoFs alone
+template <int V>
+using ic = std::integral_constant<int, V>;
+
+template <class F>
+void dispatch_block(const MeshView& m, F&& f) {
+  if (m.nf == 3 && m.nl == 3) f(ic<3>{}, ic<3>{});
+  else if (m.nf == 3 && m.nl == 6) f(ic<3>{}, ic<6>{});
+  else if (m.nf == 4 && m.nl == 4) f(ic<4>{}, ic<4>{});
+  else if (m.nf == 4 && m.nl == 9) f(ic<4>{}, ic<9>{});
+  else HDD_THROW(HDD_ERR_INTERNAL, "unsupported block shape nf = " << m.nf << ", nl = " << m.nl);
+}
+
+template <class F>
+void dispatch_nl(int nl, F&& f) {
+  switch (nl) {
+    case 3: f(ic<3>{}); break;
+    case 4: f(ic<4>{}); break;
+    case 6: f(ic<6>{}); break;
+    case 9: f(ic<9>{}); break;
+    default: HDD_THROW(HDD_ERR_INTERNAL, "unsupported n_loc " << nl);
+  }
+}
 
 // ---- K0: device-side localisation of the host grid -------------------------------------------------------------------
 // cgeo[c] from (xy, cell_verts); xy is addressed by global vertex id and valid in [v_begin, v_end); flag |= 1 if a cube

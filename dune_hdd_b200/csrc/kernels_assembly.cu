@@ -9,9 +9,7 @@
 // value array, written with 256-bit stores for Q1 (one full 32-byte sector per block row).
 #include <cub/device/device_scan.cuh>
 
-#include <cstdlib>
 #include <cstring>
-#include <type_traits>
 
 #include "kernels.hpp"
 
@@ -236,20 +234,10 @@ __device__ __forceinline__ void store_block(double* __restrict__ row0, int row_s
 // (cp.async.bulk.global.shared::cta, SASS UBLKCP) instead of every thread looping over LDS + STG; the staging buffer is laid
 // out so that shared and global addresses agree modulo 16 (the caller offsets its rows by `stage_pad(dst)` doubles).
 // Must be called by every thread of the CTA after the rows have been written; returns when the shared memory may be reused.
-// HDD_ASM_BULK_STORE=0: staged rows are written out by a store loop of all threads instead of one bulk copy (A/B switch)
-static int bulk_store_on() {
-  static const int on = [] { const char* e = std::getenv("HDD_ASM_BULK_STORE"); return (e && e[0] == '0') ? 0 : 1; }();
-  return on;
-}
 __device__ __forceinline__ int stage_pad(const double* dst) { return int((reinterpret_cast<uintptr_t>(dst) >> 3) & 1); }
 
 __device__ __forceinline__ void bulk_write_out(double* __restrict__ dst, const double* stage /* = stage0 + stage_pad(dst) */,
-                                               int64_t total, bool bulk) {
-  if (!bulk) {
-    __syncthreads();
-    for (int64_t t = threadIdx.x; t < total; t += blockDim.x) dst[t] = stage[t];
-    return;
-  }
+                                               int64_t total) {
   // make the generic-proxy writes to shared memory visible to the async proxy, then meet
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   __syncthreads();
@@ -271,30 +259,30 @@ __device__ __forceinline__ void bulk_write_out(double* __restrict__ dst, const d
 // FK = kind of the diffusion-factor part (HDD_FN_*), resolved at compile time so that constant and cell-wise data
 // cost no function evaluation per quadrature point.  An Expression is one global function: both sides of a face
 // see the same value at the same point, so it is evaluated once per point.
-template <int FK>
-__device__ __forceinline__ double factor_at(const DevFn& fn, double a_cell, double x, double y) {
-  if constexpr (FK == HDD_FN_EXPRESSION) {
-    const double v[2] = {x, y};
-    return eval_program(fn.prog, v);
-  } else {
-    return a_cell;
-  }
+__device__ __forceinline__ double expression_at(const DevFn& fn, double x, double y) {
+  const double v[2] = {x, y};
+  return eval_program(fn.prog, v);
 }
 
-template <int KIND, int FK, int OCC = 1>
-__global__ void __launch_bounds__(kThreads, OCC)
+template <int FK>
+__device__ __forceinline__ double factor_at(const DevFn& fn, double a_cell, double x, double y) {
+  if constexpr (FK == HDD_FN_EXPRESSION) return expression_at(fn, x, y);
+  else return a_cell;
+}
+
+// P1 on triangles with an Expression factor.  Bounded for one resident CTA per SM it compiles without spills; bounded for 4
+// it is squeezed to 128 registers with spilled values and measured slower (1.99 vs 1.92 ms on 16.8 M triangles).
+__global__ void __launch_bounds__(kThreads, 1)
     k_assemble_lhs(MeshView m, const __grid_constant__ DevFn fn, ElemRule vol, LineRule fr, double s_in, double s_bnd,
-                   double* __restrict__ vals, int bulk) {
-  using G = Geo<KIND>;
+                   double* __restrict__ vals) {
+  using G = Geo<HDD_SIMPLEX2D>;
   constexpr int NL = G::NL, NF = G::NF;
   // P1 row blocks are 3 doubles wide: written straight from the registers every store instruction would touch 32
   // different sectors for 24 bytes each.  The row blocks of the CTA's cells are one contiguous range of the value array,
   // so they are staged in shared memory and written out as one bulk copy (see bulk_write_out).
-  constexpr bool kStaged = (NL == 3);
-  __shared__ __align__(16) double stage0[kStaged ? kThreads * (NF + 1) * NL * NL + 2 : 2];
+  __shared__ __align__(16) double stage0[kThreads * (NF + 1) * NL * NL + 2];
   const int k_first = blockIdx.x * blockDim.x;
   const bool live = k_first + int(threadIdx.x) < m.n_own;
-  if (!kStaged && !live) return;
   const int k = live ? k_first + threadIdx.x : m.n_own - 1;  // idle threads of the last CTA recompute its last cell
   const int c = m.own0 + k;
   G g;
@@ -305,12 +293,9 @@ __global__ void __launch_bounds__(kThreads, OCC)
   load_neigh<NF>(m.neigh, k, nb);
   const int nblk = block_count<NF>(nb);
   const int rs = nblk * NL;
-  const int64_t base_blk = kStaged ? __ldg(m.blk_start + k_first) : 0;
-  double* stage = stage0 + (kStaged ? stage_pad(vals + base_blk * (NL * NL)) : 0);
-  double* row0 = kStaged ? stage + (m.blk_start[k] - base_blk) * (NL * NL) : vals + m.blk_start[k] * (NL * NL);
-  double a_self = 0.0;
-  if constexpr (FK == HDD_FN_CONSTANT) a_self = fn.value;
-  if constexpr (FK == HDD_FN_CELLWISE) a_self = __ldg(fn.cell + c);
+  const int64_t base_blk = __ldg(m.blk_start + k_first);
+  double* stage = stage0 + stage_pad(vals + base_blk * (NL * NL));
+  double* row0 = stage + (m.blk_start[k] - base_blk) * (NL * NL);
 
   double D[NL * NL];
 #pragma unroll
@@ -321,7 +306,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
     double phi[NL], gx[NL], gy[NL], x, y;
     g.basis(vol.x[q], vol.y[q], phi, gx, gy);
     g.to_global(vol.x[q], vol.y[q], x, y);
-    const double wa = vol.w[q] * g.detj * factor_at<FK>(fn, a_self, x, y);
+    const double wa = vol.w[q] * g.detj * expression_at(fn, x, y);
 #pragma unroll
     for (int j = 0; j < NL; ++j) {
       const double fx = wa * (K[0] * gx[j] + K[1] * gy[j]);
@@ -347,7 +332,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
         double xi, eta, phi[NL], gx[NL], gy[NL], A[NL], B[NL];
         g.to_local(x, y, xi, eta);
         g.basis(xi, eta, phi, gx, gy);
-        const double a = factor_at<FK>(fn, a_self, x, y);
+        const double a = expression_at(fn, x, y);
         const double w = fr.w[q] * e.h;
         const double wpen = w * pen0 * a, wa = w * a;
 #pragma unroll
@@ -371,19 +356,16 @@ __global__ void __launch_bounds__(kThreads, OCC)
       const double gamma = dp * dm * isum;
       const double wm = dp * isum, wp = dm * isum;
       const double pen0 = s_in * gamma * 0.5 * e.ih;
-      double a_nb = a_self;
-      if constexpr (FK == HDD_FN_CELLWISE) a_nb = __ldg(fn.cell + n);
       double E[NL * NL];
 #pragma unroll
       for (int t = 0; t < NL * NL; ++t) E[t] = 0.0;
       for (int q = 0; q < fr.n; ++q) {
         const double x = e.ax + fr.x[q] * (e.bx - e.ax), y = e.ay + fr.x[q] * (e.by - e.ay);
         double xi, eta, phm[NL], php[NL], gx[NL], gy[NL], A[NL], B[NL], Cc[NL];
-        const double am = factor_at<FK>(fn, a_self, x, y);
-        const double ap = (FK == HDD_FN_EXPRESSION) ? am : a_nb;
+        const double a = expression_at(fn, x, y);  // the same value on both sides of the face
         const double w = fr.w[q] * e.h;
-        const double wpen = w * pen0 * (am + ap);
-        const double wwm = w * wm * am, wwp = w * wp * ap;
+        const double wpen = w * pen0 * (a + a);
+        const double wwm = w * wm * a, wwp = w * wp * a;
         g.to_local(x, y, xi, eta);
         g.basis(xi, eta, phm, gx, gy);
 #pragma unroll
@@ -408,10 +390,8 @@ __global__ void __launch_bounds__(kThreads, OCC)
     }
   }
   if (live) store_block<NL>(row0, rs, block_slot<NF>(c, nb, c), D);
-  if constexpr (kStaged) {
-    const int k_end = min(k_first + int(blockDim.x), m.n_own);
-    bulk_write_out(vals + base_blk * (NL * NL), stage, (__ldg(m.blk_start + k_end) - base_blk) * (NL * NL), bulk != 0);
-  }
+  const int k_end = min(k_first + int(blockDim.x), m.n_own);
+  bulk_write_out(vals + base_blk * (NL * NL), stage, (__ldg(m.blk_start + k_end) - base_blk) * (NL * NL));
 }
 
 // K2 for P1 on triangles with a diffusion factor that is constant per cell (Constant / per-cell data: ESV2007, SPE10,
@@ -497,10 +477,10 @@ __device__ __forceinline__ void p1_face(const MeshView& m, const DevFn& fn, cons
   if (live) store_block<3>(row0, rs, block_slot<3>(c, nb, n), E);
 }
 
-template <int FK, int OCC>
-__global__ void __launch_bounds__(kThreads, OCC)
-    k_assemble_p1_closed(MeshView m, const __grid_constant__ DevFn fn, double s_in, double s_bnd, double* __restrict__ vals,
-                         int bulk) {
+// 4 resident CTAs per SM: at most 128 registers and no spills; bounded for 5 it is squeezed to 96 registers and spills
+template <int FK>
+__global__ void __launch_bounds__(kThreads, 4)
+    k_assemble_p1_closed(MeshView m, const __grid_constant__ DevFn fn, double s_in, double s_bnd, double* __restrict__ vals) {
   using G = Geo<HDD_SIMPLEX2D>;
   // row blocks are 3 doubles wide: staged in shared memory and written out as one bulk copy (see bulk_write_out)
   __shared__ __align__(16) double stage0[kThreads * 4 * 9 + 2];
@@ -535,7 +515,7 @@ __global__ void __launch_bounds__(kThreads, OCC)
   p1_face<FK, 1, 2, 0>(m, fn, g, gx, gy, K, area, a_self, k, c, nb[2], 2, s_in, s_bnd, D, row0, rs, nb, live);
   if (live) store_block<3>(row0, rs, block_slot<3>(c, nb, c), D);
   const int k_end = min(k_first + int(blockDim.x), m.n_own);
-  bulk_write_out(dst, stage, (__ldg(m.blk_start + k_end) - base_blk) * 9, bulk != 0);
+  bulk_write_out(dst, stage, (__ldg(m.blk_start + k_end) - base_blk) * 9);
 }
 
 // K2 for Q1 on axis-parallel rectangles.  Same integrals as k_assemble_lhs, with two structural facts used at compile
@@ -759,7 +739,7 @@ __device__ __forceinline__ double pick(const double* v, int i) {
 template <int KIND, int P, int FK, int MODE, int MINB = 2>
 __global__ void __launch_bounds__(kThreads, MINB)
     k_assemble_rows(MeshView m, const __grid_constant__ DevFn fn, ElemRule vol, LineRule fr, double s_in, double s_bnd,
-                    double* __restrict__ vals, int bulk) {
+                    double* __restrict__ vals) {
   using G = Elem<KIND, P>;
   constexpr int NL = G::NL, NF = G::NF;
   // The rows of the CTA are one contiguous range of the value array.  Written straight from the registers every store
@@ -911,7 +891,7 @@ __global__ void __launch_bounds__(kThreads, MINB)
   load_neigh<NF>(m.neigh, kl, nbl);
   const int nblkl = block_count<NF>(nbl);
   const int64_t total = __ldg(m.blk_start + kl) * (NL * NL) + int64_t(il + 1) * nblkl * NL - base;
-  bulk_write_out(vals + base, stage, total, bulk != 0);
+  bulk_write_out(vals + base, stage, total);
 }
 
 // K2 for Q2 on axis-parallel rectangles (BASELINE config 5 at p = 2).  One thread per matrix row, 32 cells per CTA.
@@ -939,9 +919,9 @@ __host__ __device__ __forceinline__ void lagrange2(double t, double* l, double* 
   d[0] = 4.0 * t - 3.0;               d[1] = 4.0 - 8.0 * t;       d[2] = 4.0 * t - 1.0;
 }
 
-template <int F, int FK>
+template <int F>
 __device__ __forceinline__ void q2_face(const MeshView& m, const DevFn& fn, const Geo<HDD_CUBE2D>& g, const double* K, int k,
-                                        int c, int n, int i, double a_self, const LineRule& fr, double s_in, double s_bnd,
+                                        int c, int n, int i, const LineRule& fr, double s_in, double s_bnd,
                                         double* tab /* this cell's [q][2][9] */, double* D, double* row, const int* nb, bool live) {
   constexpr bool vertical = F < 2;                      // faces 0,1: x = const; faces 2,3: y = const
   constexpr double sgn = (F == 0 || F == 2) ? -1.0 : 1.0;
@@ -960,7 +940,7 @@ __device__ __forceinline__ void q2_face(const MeshView& m, const DevFn& fn, cons
   const double dm = vertical ? K[0] : K[3];
   const bool inner = n >= 0;
   const bool dirichlet = !inner && !(m.btype && __ldg(m.btype + size_t(4) * k + F) != 1);
-  double wm = 1.0, wp = 0.0, pen0 = s_bnd * dm * ih, a_nb = a_self, kn_ac_p = 0.0, kn_al_p = 0.0, i_across_p = 0.0;
+  double wm = 1.0, wp = 0.0, pen0 = s_bnd * dm * ih, kn_ac_p = 0.0, kn_al_p = 0.0, i_across_p = 0.0;
   if (inner) {
     double Kn[4];
     load_tensor(m.tensor, n, Kn);
@@ -971,7 +951,6 @@ __device__ __forceinline__ void q2_face(const MeshView& m, const DevFn& fn, cons
     pen0 = s_in * dp * dm * isum * 0.5 * ih;
     kn_ac_p = sgn * (vertical ? Kn[0] : Kn[3]);
     kn_al_p = sgn * (vertical ? Kn[1] : Kn[2]);
-    if constexpr (FK == HDD_FN_CELLWISE) a_nb = __ldg(fn.cell + n);
     Geo<HDD_CUBE2D> gn;
     gn.load(m.cgeo, n);
     i_across_p = vertical ? gn.ihx : gn.ihy;
@@ -981,15 +960,11 @@ __device__ __forceinline__ void q2_face(const MeshView& m, const DevFn& fn, cons
   for (int q = 0; q < fr.n; ++q) {
     double lt[3], dt[3];
     lagrange2(fr.x[q], lt, dt);
-    double am = a_self;
-    if constexpr (FK == HDD_FN_EXPRESSION) {
-      const double xi = vertical ? (side == 0 ? 0.0 : 1.0) : fr.x[q], eta = vertical ? fr.x[q] : (side == 0 ? 0.0 : 1.0);
-      am = factor_at<FK>(fn, a_self, g.x0 + g.hx * xi, g.y0 + g.hy * eta);
-    }
-    const double ap = (FK == HDD_FN_EXPRESSION) ? am : a_nb;
+    const double xi = vertical ? (side == 0 ? 0.0 : 1.0) : fr.x[q], eta = vertical ? fr.x[q] : (side == 0 ? 0.0 : 1.0);
+    const double a = expression_at(fn, g.x0 + g.hx * xi, g.y0 + g.hy * eta);  // the same on both sides
     const double w = fr.w[q] * h;
-    const double wpen = inner ? w * pen0 * (am + ap) : w * pen0 * am;
-    const double wwm = w * wm * am, wwp = w * wp * ap;
+    const double wpen = inner ? w * pen0 * (a + a) : w * pen0 * a;
+    const double wwm = w * wm * a, wwp = w * wp * a;
     const double la = pick<3>(lt, along), da = pick<3>(dt, along);
     const double phi = l_own * la;
     // grad phi . K^T n = d/d(across) * kn_ac + d/d(along) * kn_al
@@ -1037,10 +1012,9 @@ __device__ __forceinline__ void q2_face(const MeshView& m, const DevFn& fn, cons
   }
 }
 
-template <int FK>
 __global__ void __launch_bounds__(kQ2Threads, 3)
     k_assemble_q2_cube(MeshView m, const __grid_constant__ DevFn fn, ElemRule vol, LineRule fr, double s_in, double s_bnd,
-                       double* __restrict__ vals, int bulk) {
+                       double* __restrict__ vals) {
   // A_j, C_j of the current face: [parity][cell][q][2][9]; two buffers, so that one barrier per face is enough
   extern __shared__ __align__(16) double q2_smem[];
   double (*tabs)[kQ2Cells][kQ2MaxFacePts * 2 * 9] = reinterpret_cast<double (*)[kQ2Cells][kQ2MaxFacePts * 2 * 9]>(q2_smem);
@@ -1062,9 +1036,6 @@ __global__ void __launch_bounds__(kQ2Threads, 3)
   double* out = vals + base_blk * 81;
   double* stage = stage0 + stage_pad(out);
   double* row = stage + (__ldg(m.blk_start + k) - base_blk) * 81 + int64_t(i) * nblk * 9;
-  double a_self = 0.0;
-  if constexpr (FK == HDD_FN_CONSTANT) a_self = fn.value;
-  if constexpr (FK == HDD_FN_CELLWISE) a_self = __ldg(fn.cell + c);
   const int ai = i % 3, bi = i / 3;
   double D[9];
 #pragma unroll
@@ -1074,8 +1045,7 @@ __global__ void __launch_bounds__(kQ2Threads, 3)
     double lx[3], dx[3], ly[3], dy[3];
     lagrange2(vol.x[q], lx, dx);
     lagrange2(vol.y[q], ly, dy);
-    double a = a_self;
-    if constexpr (FK == HDD_FN_EXPRESSION) a = factor_at<FK>(fn, a_self, g.x0 + g.hx * vol.x[q], g.y0 + g.hy * vol.y[q]);
+    const double a = expression_at(fn, g.x0 + g.hx * vol.x[q], g.y0 + g.hy * vol.y[q]);
     const double wa = vol.w[q] * g.detj * a;
     const double gxi = wa * pick<3>(dx, ai) * pick<3>(ly, bi) * g.ihx, gyi = wa * pick<3>(lx, ai) * pick<3>(dy, bi) * g.ihy;
     const double cx = K[0] * gxi + K[2] * gyi, cy = K[1] * gxi + K[3] * gyi;  // (K grad phi_j) . grad phi_i = grad phi_j . K^T grad phi_i
@@ -1085,17 +1055,17 @@ __global__ void __launch_bounds__(kQ2Threads, 3)
       for (int a2 = 0; a2 < 3; ++a2)
         D[a2 + 3 * b] = fma(dx[a2] * ly[b] * g.ihx, cx, fma(lx[a2] * dy[b] * g.ihy, cy, D[a2 + 3 * b]));
   }
-  q2_face<0, FK>(m, fn, g, K, k, c, nb[0], i, a_self, fr, s_in, s_bnd, tabs[0][cs], D, row, nb, live);
-  q2_face<1, FK>(m, fn, g, K, k, c, nb[1], i, a_self, fr, s_in, s_bnd, tabs[1][cs], D, row, nb, live);
-  q2_face<2, FK>(m, fn, g, K, k, c, nb[2], i, a_self, fr, s_in, s_bnd, tabs[0][cs], D, row, nb, live);
-  q2_face<3, FK>(m, fn, g, K, k, c, nb[3], i, a_self, fr, s_in, s_bnd, tabs[1][cs], D, row, nb, live);
+  q2_face<0>(m, fn, g, K, k, c, nb[0], i, fr, s_in, s_bnd, tabs[0][cs], D, row, nb, live);
+  q2_face<1>(m, fn, g, K, k, c, nb[1], i, fr, s_in, s_bnd, tabs[1][cs], D, row, nb, live);
+  q2_face<2>(m, fn, g, K, k, c, nb[2], i, fr, s_in, s_bnd, tabs[0][cs], D, row, nb, live);
+  q2_face<3>(m, fn, g, K, k, c, nb[3], i, fr, s_in, s_bnd, tabs[1][cs], D, row, nb, live);
   if (live) {
     double* dst = row + block_slot<4>(c, nb, c) * 9;
 #pragma unroll
     for (int j = 0; j < 9; ++j) dst[j] = D[j];
   }
   const int k_end = min(k_first + kQ2Cells, m.n_own);
-  bulk_write_out(out, stage, (__ldg(m.blk_start + k_end) - base_blk) * 81, bulk != 0);
+  bulk_write_out(out, stage, (__ldg(m.blk_start + k_end) - base_blk) * 81);
 }
 
 // K2 for Q2 on axis-parallel rectangles with a constant or cellwise factor: no quadrature loop at all.  On such a cell every
@@ -1216,7 +1186,7 @@ constexpr int kQ2ClosedSmemBytes = (kQ2StageDoubles + 2) * 8;
 template <int FK>
 __global__ void __launch_bounds__(kQ2Threads, 4)
     k_assemble_q2_closed(MeshView m, const __grid_constant__ DevFn fn, const __grid_constant__ Q2Tables T, double s_in, double s_bnd,
-                         double* __restrict__ vals, int bulk) {
+                         double* __restrict__ vals) {
   extern __shared__ __align__(16) double q2_smem[];
   const int cs = threadIdx.x / 9, i = threadIdx.x % 9;
   const int k_raw = blockIdx.x * kQ2Cells + cs;
@@ -1271,7 +1241,7 @@ __global__ void __launch_bounds__(kQ2Threads, 4)
     for (int j = 0; j < 9; ++j) dst[j] = D[j];
   }
   const int k_end = min(k_first + kQ2Cells, m.n_own);
-  bulk_write_out(out, stage, (__ldg(m.blk_start + k_end) - base_blk) * 81, bulk != 0);
+  bulk_write_out(out, stage, (__ldg(m.blk_start + k_end) - base_blk) * 81);
 }
 
 // Volume-pattern products (discretizations/swipdg.hh:359-443): one dense n_loc x n_loc block per cell, one thread per
@@ -1678,10 +1648,7 @@ void exclusive_scan_i64(const int64_t* in, int64_t* out, int64_t n, cudaStream_t
   count_launch(2);
 }
 
-// compile-time dispatch helpers: (element kind, polynomial order) and (faces, local DoFs)
-template <int V>
-using ic = std::integral_constant<int, V>;
-
+// compile-time dispatch helpers: (element kind, polynomial order) and factor kind
 template <class F>
 static void dispatch_elem(int kind, int polorder, F&& f) {
   if (polorder != 1 && polorder != 2) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "polorder " << polorder);
@@ -1690,15 +1657,6 @@ static void dispatch_elem(int kind, int polorder, F&& f) {
   } else {
     if (polorder == 1) f(ic<HDD_CUBE2D>{}, ic<1>{}); else f(ic<HDD_CUBE2D>{}, ic<2>{});
   }
-}
-
-template <class F>
-static void dispatch_block(const MeshView& m, F&& f) {
-  if (m.nf == 3 && m.nl == 3) f(ic<3>{}, ic<3>{});
-  else if (m.nf == 3 && m.nl == 6) f(ic<3>{}, ic<6>{});
-  else if (m.nf == 4 && m.nl == 4) f(ic<4>{}, ic<4>{});
-  else if (m.nf == 4 && m.nl == 9) f(ic<4>{}, ic<9>{});
-  else HDD_THROW(HDD_ERR_INTERNAL, "unsupported block shape nf = " << m.nf << ", nl = " << m.nl);
 }
 
 template <class F>
@@ -1718,75 +1676,30 @@ void launch_fill_csr(const MeshView& m, int64_t* rowptr, int32_t* col, cudaStrea
   HDD_CUDA(cudaGetLastError());
 }
 
-template <int KIND>
-static void assemble_dispatch(int fk, int blocks, cudaStream_t s, const MeshView& m, const DevFn& fn, const ElemRule& vol,
-                              const LineRule& fr, double si, double sb, double* values) {
-  // P1 quadrature kernel (Expression factors): 3 resident CTAs per SM (144-148 registers); HDD_ASM_P1_OCC=4 squeezes it to
-  // 128 registers with a few spilled values (measured slower: 1.99 vs 1.92 ms on 16.8 M triangles)
-  static const bool occ4 = [] { const char* e = std::getenv("HDD_ASM_P1_OCC"); return e && e[0] == '4'; }();
-  dispatch_fk(fk, [&](auto k) {
-    if (KIND == HDD_SIMPLEX2D && occ4)
-      k_assemble_lhs<KIND, decltype(k)::value, 4><<<blocks, kThreads, 0, s>>>(m, fn, vol, fr, si, sb, values, bulk_store_on());
-    else
-      k_assemble_lhs<KIND, decltype(k)::value><<<blocks, kThreads, 0, s>>>(m, fn, vol, fr, si, sb, values, bulk_store_on());
-  });
-}
-
+// The left-hand-side kernel for (grid, polOrder, factor kind); "closed" = a factor constant per cell (constant or cell-wise):
+//   P1 triangles   closed: k_assemble_p1_closed<FK>   Expression: k_assemble_lhs
+//   Q1 rectangles  k_assemble_lhs_cube<FK, 4, true> with the tensor-grid tables (m.tgeo), else <FK, 3, false>
+//   Q2 rectangles  closed: k_assemble_q2_closed<FK>   Expression: k_assemble_q2_cube for up to kQ2MaxFacePts face points,
+//                  else k_assemble_rows
+//   P2 triangles   k_assemble_rows<FK>
 void launch_assemble_lhs(const MeshView& m, const DevFn& factor_dev, int factor_kind, int factor_order, int polorder,
                          double* values, cudaStream_t s) {
   if (m.n_own == 0) return;
+  if (polorder != 1 && polorder != 2) HDD_THROW(HDD_ERR_NOT_IMPLEMENTED, "polorder " << polorder);
   const ElemRule vol = element_rule(m.kind, factor_order + 2 * (polorder - 1));
   const LineRule fr = line_rule(factor_order + 2 * polorder);
   const double si = sigma_inner(polorder), sb = sigma_boundary(polorder);
   const int blocks = grid_for(m.n_own, kThreads);
-  // HDD_ASSEMBLY_GENERIC=1 / HDD_ASM_TENSOR=0: run a cube grid through the generic kernel / without the tensor-grid
-  // tables (kept for A/B measurements and as cross-checks of the specialised variants)
-  static const bool generic_cube = [] { const char* e = std::getenv("HDD_ASSEMBLY_GENERIC"); return e && e[0] == '1'; }();
-  static const bool tensor_ok = [] { const char* e = std::getenv("HDD_ASM_TENSOR"); return !(e && e[0] == '0'); }();
-  static const bool q2_fast = [] { const char* e = std::getenv("HDD_ASM_Q2_CUBE"); return !(e && e[0] == '0'); }();
-  // HDD_ASM_Q2_CLOSED=0: Q2 with a constant / cellwise factor through the quadrature kernel (A/B switch, cross-check)
-  static const bool q2_closed = [] { const char* e = std::getenv("HDD_ASM_Q2_CLOSED"); return !(e && e[0] == '0'); }();
-  if (polorder == 2 && m.kind == HDD_CUBE2D && q2_fast && q2_closed && factor_kind != HDD_FN_EXPRESSION) {
-    const Q2Tables T = make_q2_tables(line_rule(factor_order + 2 * (polorder - 1)), fr);
-    auto launch = [&](auto kern) {
-      HDD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kQ2ClosedSmemBytes));
-      kern<<<(m.n_own + kQ2Cells - 1) / kQ2Cells, kQ2Threads, kQ2ClosedSmemBytes, s>>>(m, factor_dev, T, si, sb, values, bulk_store_on());
-    };
-    if (factor_kind == HDD_FN_CONSTANT) launch(k_assemble_q2_closed<HDD_FN_CONSTANT>);
-    else launch(k_assemble_q2_closed<HDD_FN_CELLWISE>);
-  } else if (polorder == 2 && m.kind == HDD_CUBE2D && q2_fast && fr.n <= kQ2MaxFacePts) {
-    // Q2 on axis-parallel rectangles: tensor-product basis, per-cell flux vectors shared through shared memory
-    dispatch_fk(factor_kind, [&](auto k) {
-      auto kern = k_assemble_q2_cube<decltype(k)::value>;
-      HDD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kQ2SmemBytes));
-      kern<<<(m.n_own + kQ2Cells - 1) / kQ2Cells, kQ2Threads, kQ2SmemBytes, s>>>(m, factor_dev, vol, fr, si, sb, values, bulk_store_on());
-    });
-  } else if (polorder != 1) {
-    // p = 2: one thread per row, 3 CTAs per SM (168 registers; 2.85 ms vs 3.48 ms with 2 at 1024^2 Q2)
-    const int64_t rows = int64_t(m.n_own) * m.nl;
-    dispatch_elem(m.kind, polorder, [&](auto kind, auto p) {
-      if constexpr (decltype(p)::value == 2)
-        dispatch_fk(factor_kind, [&](auto k) {
-          k_assemble_rows<decltype(kind)::value, 2, decltype(k)::value, 0, 3>
-              <<<grid_for(rows, kThreads), kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values, bulk_store_on());
-        });
-    });
-  } else if (m.kind == HDD_SIMPLEX2D) {
-    // HDD_ASM_P1_CLOSED=0: quadrature kernel; HDD_ASM_P1_OCC=5: 5 resident CTAs per SM (96 registers, a few spills) instead of
-    // 4 (126 registers, none) - kept for A/B measurements
-    static const bool closed = [] { const char* e = std::getenv("HDD_ASM_P1_CLOSED"); return !(e && e[0] == '0'); }();
-    static const bool occ5 = [] { const char* e = std::getenv("HDD_ASM_P1_OCC"); return e && e[0] == '5'; }();
-    if (closed && factor_kind == HDD_FN_CONSTANT && occ5)
-      k_assemble_p1_closed<HDD_FN_CONSTANT, 5><<<blocks, kThreads, 0, s>>>(m, factor_dev, si, sb, values, bulk_store_on());
-    else if (closed && factor_kind == HDD_FN_CONSTANT)
-      k_assemble_p1_closed<HDD_FN_CONSTANT, 4><<<blocks, kThreads, 0, s>>>(m, factor_dev, si, sb, values, bulk_store_on());
-    else if (closed && factor_kind == HDD_FN_CELLWISE)
-      k_assemble_p1_closed<HDD_FN_CELLWISE, 4><<<blocks, kThreads, 0, s>>>(m, factor_dev, si, sb, values, bulk_store_on());
+  // p = 2 row kernel: one thread per row, 3 CTAs per SM (168 registers; 2.85 ms vs 3.48 ms with 2 at 1024^2 Q2)
+  const int row_blocks = grid_for(int64_t(m.n_own) * m.nl, kThreads);
+  if (m.kind == HDD_SIMPLEX2D && polorder == 1) {
+    if (factor_kind == HDD_FN_CONSTANT)
+      k_assemble_p1_closed<HDD_FN_CONSTANT><<<blocks, kThreads, 0, s>>>(m, factor_dev, si, sb, values);
+    else if (factor_kind == HDD_FN_CELLWISE)
+      k_assemble_p1_closed<HDD_FN_CELLWISE><<<blocks, kThreads, 0, s>>>(m, factor_dev, si, sb, values);
     else
-      assemble_dispatch<HDD_SIMPLEX2D>(factor_kind, blocks, s, m, factor_dev, vol, fr, si, sb, values);
-  } else if (generic_cube) {
-    assemble_dispatch<HDD_CUBE2D>(factor_kind, blocks, s, m, factor_dev, vol, fr, si, sb, values);
-  } else {
+      k_assemble_lhs<<<blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
+  } else if (polorder == 1) {
     // resident CTAs per SM the kernel is compiled for: 3 (160 registers) for the general kernel, 4 (128) for the tensor
     // grid variant, which keeps no neighbour geometry records alive (measured 2.15 -> 2.03 ms at 4096^2; 5 CTAs spill:
     // 2.81 ms)
@@ -1794,11 +1707,33 @@ void launch_assemble_lhs(const MeshView& m, const DevFn& factor_dev, int factor_
     // 5 resident CTAs: 2.07 ms against 2.05-2.09 ms, and 2.37 ms when a thread stores row after row instead of block after
     // block - this kernel is limited by its scattered 32-byte-sector store stream, not by instruction issue; DESIGN.md 4)
     dispatch_fk(factor_kind, [&](auto k) {
-      constexpr int FKV = decltype(k)::value;
-      if (m.tgeo && tensor_ok)
-        k_assemble_lhs_cube<FKV, 4, true><<<blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
+      constexpr int FK = decltype(k)::value;
+      if (m.tgeo)
+        k_assemble_lhs_cube<FK, 4, true><<<blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
       else
-        k_assemble_lhs_cube<FKV, 3, false><<<blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
+        k_assemble_lhs_cube<FK, 3, false><<<blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
+    });
+  } else if (m.kind == HDD_CUBE2D) {
+    const int q2_blocks = (m.n_own + kQ2Cells - 1) / kQ2Cells;
+    if (factor_kind != HDD_FN_EXPRESSION) {
+      const Q2Tables T = make_q2_tables(line_rule(factor_order + 2 * (polorder - 1)), fr);
+      auto launch = [&](auto kern) {
+        HDD_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kQ2ClosedSmemBytes));
+        kern<<<q2_blocks, kQ2Threads, kQ2ClosedSmemBytes, s>>>(m, factor_dev, T, si, sb, values);
+      };
+      if (factor_kind == HDD_FN_CONSTANT) launch(k_assemble_q2_closed<HDD_FN_CONSTANT>);
+      else launch(k_assemble_q2_closed<HDD_FN_CELLWISE>);
+    } else if (fr.n <= kQ2MaxFacePts) {
+      HDD_CUDA(cudaFuncSetAttribute(k_assemble_q2_cube, cudaFuncAttributeMaxDynamicSharedMemorySize, kQ2SmemBytes));
+      k_assemble_q2_cube<<<q2_blocks, kQ2Threads, kQ2SmemBytes, s>>>(m, factor_dev, vol, fr, si, sb, values);
+    } else {
+      k_assemble_rows<HDD_CUBE2D, 2, HDD_FN_EXPRESSION, 0, 3>
+          <<<row_blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
+    }
+  } else {
+    dispatch_fk(factor_kind, [&](auto k) {
+      k_assemble_rows<HDD_SIMPLEX2D, 2, decltype(k)::value, 0, 3>
+          <<<row_blocks, kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
     });
   }
   count_launch();
@@ -1818,7 +1753,7 @@ void launch_assemble_penalty(const MeshView& m, const DevFn& factor_dev, int fac
   dispatch_elem(m.kind, polorder, [&](auto kind, auto p) {
     dispatch_fk(factor_kind, [&](auto k) {
       k_assemble_rows<decltype(kind)::value, decltype(p)::value, decltype(k)::value, 1>
-          <<<grid_for(rows, kThreads), kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values, bulk_store_on());
+          <<<grid_for(rows, kThreads), kThreads, 0, s>>>(m, factor_dev, vol, fr, si, sb, values);
     });
   });
   count_launch();
@@ -1878,10 +1813,8 @@ void launch_rhs_volume(const MeshView& m, const DevFn& force_dev, int force_orde
     return;
   }
   const ElemRule vol = element_rule(m.kind, force_order + polorder);
-  // HDD_EST_TRIG=0 also switches this kernel back to the general function evaluation
-  static const bool trig_on = [] { const char* e = std::getenv("HDD_EST_TRIG"); return !(e && e[0] == '0'); }();
   TrigProduct tp{};
-  if (trig_on && force_dev.kind == HDD_FN_EXPRESSION && force_dev.fast.n_terms > 0) tp = as_trig_product(force_dev.fast);
+  if (force_dev.kind == HDD_FN_EXPRESSION && force_dev.fast.n_terms > 0) tp = as_trig_product(force_dev.fast);
   dispatch_elem(m.kind, polorder, [&](auto kind, auto p) {
     if (tp.valid)
       k_rhs_volume<decltype(kind)::value, decltype(p)::value, true><<<grid_for(m.n_own, kThreads), kThreads, 0, s>>>(m, force_dev, tp, vol, acc, b);

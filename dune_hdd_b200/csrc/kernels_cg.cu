@@ -20,7 +20,6 @@
 // launched after convergence are no-ops.  Preconditioners: identity, diagonal (Jacobi), and the cell-block diagonal
 // (block Jacobi with the n_loc x n_loc diagonal blocks, the natural choice for DG).
 #include <cstdlib>
-#include <type_traits>
 
 #include "kernels.hpp"
 #include "reduce.cuh"
@@ -721,46 +720,15 @@ __global__ void k_pack(const double* __restrict__ v, const int32_t* __restrict__
   }
 }
 
-template <int V>
-using ic = std::integral_constant<int, V>;
-
-template <class F>
-void dispatch_block(const MeshView& m, F&& f) {
-  if (m.nf == 3 && m.nl == 3) f(ic<3>{}, ic<3>{});
-  else if (m.nf == 3 && m.nl == 6) f(ic<3>{}, ic<6>{});
-  else if (m.nf == 4 && m.nl == 4) f(ic<4>{}, ic<4>{});
-  else if (m.nf == 4 && m.nl == 9) f(ic<4>{}, ic<9>{});
-  else HDD_THROW(HDD_ERR_INTERNAL, "unsupported block shape nf = " << m.nf << ", nl = " << m.nl);
-}
-
-template <class F>
-void dispatch_nl(int nl, F&& f) {
-  switch (nl) {
-    case 3: f(ic<3>{}); break;
-    case 4: f(ic<4>{}); break;
-    case 6: f(ic<6>{}); break;
-    case 9: f(ic<9>{}); break;
-    default: HDD_THROW(HDD_ERR_INTERNAL, "unsupported n_loc " << nl);
-  }
-}
-
 inline int cg_grid(int64_t items) {
   const int64_t need = (items + kCgThreads - 1) / kCgThreads;
   return int(std::max<int64_t>(1, std::min<int64_t>(need, kMaxBlocks)));
 }
 
-bool use_tma_impl() {
-  static const bool on = [] {
-    const char* e = std::getenv("HDD_SPMV_TMA");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 }  // namespace
 
 bool cg_spmv_uses_tma(const MeshView& m) {
-  return m.kind == HDD_CUBE2D && m.nl == 4 && use_tma_impl() && m.n_own >= 148 * kTmaTileCells;
+  return m.kind == HDD_CUBE2D && m.nl == 4 && m.n_own >= 148 * kTmaTileCells;
 }
 
 int cg_partial_capacity() { return 3 * kMaxBlocks; }
@@ -825,7 +793,7 @@ void launch_cg_spmv(const MeshView& m, const CgBuffers& c, int parity, cudaStrea
     PeerView pv{};
     if (peer) pv = *peer;
     k_cg_spmv_tma<<<grid, kTmaThreads, kTmaSmemBytes, s>>>(m, c, parity, cells_per_cta, pv);
-  } else if (use_tma_impl() && !peer && m.n_own >= 1024 && !(m.nf == 4 && m.nl == 4)) {
+  } else if (!peer && m.n_own >= 1024 && !(m.nf == 4 && m.nl == 4)) {
     if (m.nf == 3 && m.nl == 3) launch_cg_spmv_tma_g<3, 3, 10>(m, c, parity, s);
     else if (m.nf == 3 && m.nl == 6) launch_cg_spmv_tma_g<3, 6, 5>(m, c, parity, s);
     else if (m.nf == 4 && m.nl == 9) launch_cg_spmv_tma_g<4, 9, 3>(m, c, parity, s);

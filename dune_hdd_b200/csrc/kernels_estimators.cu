@@ -348,11 +348,9 @@ void launch_indicators(const MeshView& m, const IndicatorArgs& a, const DevFn* f
                       combo_is_cellwise(a.a_bar, fn_table_host) && combo_is_cellwise(a.a_cut, fn_table_host) &&
                       combo_is_cellwise(a.a_min, fn_table_host) && combo_is_cellwise(a.a_max, fn_table_host));
   const int grid = (m.n_own + 127) / 128;
-  // HDD_EST_TRIG=0: the force always through the general function evaluation (A/B switch, cross-check)
-  static const bool trig_on = [] { const char* e = std::getenv("HDD_EST_TRIG"); return !(e && e[0] == '0'); }();
   const DevFn& force = fn_table_host[a.force_idx];
   TrigProduct tp{};
-  if (trig_on && force.kind == HDD_FN_EXPRESSION && force.fast.n_terms > 0) tp = as_trig_product(force.fast);
+  if (force.kind == HDD_FN_EXPRESSION && force.fast.n_terms > 0) tp = as_trig_product(force.fast);
   const double si = sigma_inner(p), sb = sigma_boundary(p);
   if (expr && tp.valid)
     k_indicators<true, true><<<grid, 128, fn_bytes, s>>>(m, a, R, tp, si, sb);

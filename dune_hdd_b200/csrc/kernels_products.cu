@@ -1,8 +1,6 @@
 // K12/K13 for sm_100a: what the reference's product matrices are used for - bilinear forms u^T P v and the induced
 // norms (discretizations/base.hh:272-291; test/linearelliptic-swipdg.hh:267-290) - plus the per-cell error norms of
 // u_h against an analytic solution (SURVEY 8f rank 3).  All HBM-bound streaming work.
-#include <type_traits>
-
 #include "kernels.hpp"
 
 namespace hdd {
@@ -10,20 +8,6 @@ namespace hdd {
 namespace {
 
 constexpr int kThreads = 256;
-
-template <int V>
-using ic = std::integral_constant<int, V>;
-
-template <class F>
-void dispatch_nl(int nl, F&& f) {
-  switch (nl) {
-    case 3: f(ic<3>{}); break;
-    case 4: f(ic<4>{}); break;
-    case 6: f(ic<6>{}); break;
-    case 9: f(ic<9>{}); break;
-    default: HDD_THROW(HDD_ERR_INTERNAL, "unsupported n_loc " << nl);
-  }
-}
 
 // volume pattern: one dense NL x NL block per owned cell, global column indices
 template <int NL>

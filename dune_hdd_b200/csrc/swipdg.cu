@@ -120,10 +120,7 @@ FnRef add_function(hdd_swipdg* h, const hdd_function& f, const char* what) {
       if (!f.expression) HDD_THROW(HDD_ERR_WRONG_INPUT, what << ": expression is NULL");
       d.prog = compile_expression(f.expression, "x");
       d.separable = compile_separable(f.expression, "x", d.px, d.py) ? 1 : 0;
-      {
-        static const bool fast_on = [] { const char* e = std::getenv("HDD_EXPR_FAST"); return !(e && e[0] == '0'); }();
-        if (fast_on) compile_fast(f.expression, "x", d.fast);
-      }
+      compile_fast(f.expression, "x", d.fast);
       break;
     default:
       HDD_THROW(HDD_ERR_WRONG_INPUT, what << ": unknown function kind " << f.kind);
@@ -979,7 +976,8 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
     // One CG iteration = 3 kernels (+ 2 all-reduces, + ~100 small multigrid kernels for cg.mg / cg.mg2 / cg.mg2.simplex).  The first batch is
     // launched directly (one-time attribute / buffer set-up happens there); after that two iterations (parity 0 and 1)
     // are captured into a CUDA graph and replayed, so a launch-bound iteration costs one graph launch instead of up to
-    // a hundred kernel launches and does not stall the GPU when the host thread is delayed.  HDD_CG_GRAPH=0 disables it.
+    // a hundred kernel launches and does not stall the GPU when the host thread is delayed.  The phase timer
+    // (HDD_CG_PHASES=1) records events between the kernels of every iteration, so it launches them one by one.
     auto iteration = [&](int parity) {
       if (multi && !p2p) { m->halo_exchange(c.p, h->nl); pt.mark("halo exchange (p)", s); }
       launch_cg_spmv(v, c, parity, s, peer);
@@ -992,10 +990,7 @@ int hdd_solve(hdd_swipdg* h, const char* type, double precision, int max_iter, c
       launch_cg_direction(v, c, parity, s);
       pt.mark("direction", s);
     };
-    static const bool graphs_wanted = [] {
-      const char* e = std::getenv("HDD_CG_GRAPH");
-      return !(e && e[0] == '0') && !phase_timer().on;
-    }();
+    const bool graphs_wanted = !phase_timer().on;
     hdd_swipdg::CgGraph& cached = h->cg_graph[int(solver)];
     const void* key[5] = {vals, c.p_alt, peer, c.dinv_block, m->send_buf.p};
     if (cached.exec && std::memcmp(cached.key, key, sizeof(key)) != 0) {

@@ -439,9 +439,8 @@ def test_p2_parametric_cellwise_and_block_views(gpu):
 
 # ---- a9: non-zero Neumann data (Functionals::L2Face, discretizations/swipdg.hh:335-356) --------------------------
 def test_q2_closed_form_kernel_full_tensor_cellwise_factor_rectangles(gpu, monkeypatch):
-    """the closed-form Q2 kernel (1-d quadrature matrices instead of quadrature loops) against the oracle where its formulas
-    have the most terms: cells with hx != hy, a full symmetric cell-wise tensor, a cell-wise factor - and against the
-    quadrature kernel it replaces (HDD_ASM_Q2_CLOSED is read once per process, so that comparison goes through the oracle)"""
+    """the closed-form Q2 kernel (1-d quadrature matrices instead of quadrature loops) against the oracle's quadrature loops
+    where its formulas have the most terms: cells with hx != hy, a full symmetric cell-wise tensor, a cell-wise factor"""
     g = grids.cube(7, 5, lower_left=(-1.0, 0.0), upper_right=(2.5, 1.0))
     rng = np.random.default_rng(11)
     k = rng.uniform(0.5, 4.0, (g.n_cells, 2))
@@ -645,7 +644,7 @@ def test_cg_mg_spe10_shape_parametric_and_requirements(gpu):
 @pytest.mark.parametrize("kind,n,polorder", [("alu", 16, 1), ("alu", 32, 1), ("alu", 16, 2), ("sgrid", 32, 2), ("sgrid", 40, 1)])
 def test_bulk_copy_spmv_paths(gpu, kind, n, polorder):
     """grids large enough (>= 1024 cells) for the TMA-staged CG SpMV kernels of every block size, against the direct
-    solve and against the generic kernels (HDD_SPMV_TMA=0 is read once per process, so compare through the oracle)"""
+    solve and, iterate by iterate, against the oracle's CG"""
     g = _grid(kind, n)
     assert g.n_cells >= 1024
     os.environ["HDD_SPMV_CTAS"] = "3"  # few CTAs: every CTA walks its shared-memory ring several times

@@ -1,4 +1,4 @@
-"""assembly kernel timing for the current HDD_ASM_* environment: python tools/quick_asm_variants.py n polorder kind"""
+"""matrix-assembly kernel time (ESV2007 data): python tools/quick_asm_variants.py n polorder [cube|simplex]"""
 import sys, json, ctypes as C
 sys.path.insert(0, '.')
 import dune_hdd_b200 as hdd
@@ -12,6 +12,4 @@ L = capi.lib()
 sec, byt = C.c_double(), C.c_double()
 capi.check(L.hdd_profile_kernel(d._h, 3, 10, C.byref(sec)))
 capi.check(L.hdd_kernel_bytes(d._h, 3, C.byref(byt)))
-import os
-print(json.dumps({"n": n, "p": p, "kind": kind, "env": {k: v for k, v in os.environ.items() if k.startswith("HDD_")},
-                  "ms": sec.value * 1e3, "GBs": byt.value / sec.value / 1e9}))
+print(json.dumps({"n": n, "p": p, "kind": kind, "ms": sec.value * 1e3, "GBs": byt.value / sec.value / 1e9}))
